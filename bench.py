@@ -70,7 +70,18 @@ def parse():
     ap.add_argument("--exchange", default="p2p", choices=["p2p", "nccl"],
                     help="mosaic halo / range exchange: this library's kernels over NVLink peer memory, or NCCL send/recv + all-reduce")
     ap.add_argument("--zstack", default="1024x1024x64", help="X x Y x Z of the --workload zstack volume (BASELINE config 4)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="--workload fov only: after the timed steps, write what the last timed step returned on rank 0 "
+                         "(other ranks write nothing) to DIR: score.npy (2048x2048 float32 score map) and, except for "
+                         "--path fused, channel_sum.npy (2048x2048 float64 channel sums) and channel_sum_max_min.npy "
+                         "(their global max and min), so that two builds can be compared output for output (the "
+                         "inputs are seeded: the same arguments give the same inputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "fov"):
+        ap.error("--dump-outputs writes the headline workload's outputs: it needs --impl b200 --workload fov")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -436,25 +447,27 @@ def run_b200(args):
     streams = [torch.cuda.Stream(device=dev) for _ in range(args.streams)] if args.streams > 1 else None
 
     def step(i, ev=None):
+        """One FOV through the timed path: (score, float64 channel sums, MaxKey of the sums); the fused path returns
+        the score alone, (score, None, None)."""
         cube = cubes[i % len(cubes)]
         st = streams[i % len(streams)] if streams else torch.cuda.current_stream()
         with torch.cuda.stream(st):
             if args.path == "pipeline":
-                return ops.neighbor2d_pipeline(cube, "F1", bands=args.bands)[0]
+                return ops.neighbor2d_pipeline(cube, "F1", bands=args.bands)
             if args.path == "fused":
                 if ev:
                     ev[0].record(st)
                 out = ops.neighbor2d_fused(cube, "F1")
                 if ev:
                     ev[1].record(st)
-                return out
+                return out, None, None
             if ev:
                 ev[0].record(st)
             s, mk = ops.channel_sum(cube, None, normalize=False, dtype=torch.float64, return_max=True)
             if ev:
                 ev[1].record(st)
             out = ops.lne2d_fixed(s, "F1", 11, 9, padded=False, range_keys=mk)
-        return out
+        return out, s, mk
 
     def fork():
         if streams:
@@ -504,13 +517,22 @@ def run_b200(args):
     e0.record()
     fork()
     for i in range(args.steps):
-        step(i, k1_events[i])
+        last = step(i, k1_events[i])
     join()
     e1.record()
     barrier()
     clocks = sampler.stop()
     launches = lib.hipr_launch_count() - launches0
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        score, s, mk = last
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "score.npy"), score.cpu().numpy().astype(np.float32))
+        if s is not None:
+            np.save(os.path.join(args.dump_outputs, "channel_sum.npy"), s.cpu().numpy().astype(np.float64))
+            np.save(os.path.join(args.dump_outputs, "channel_sum_max_min.npy"),
+                    torch.cat(mk.values()).cpu().numpy().astype(np.float64))
+    del last
 
     # ---- roofline region: the dominant kernel (channel sum) launched alone, K times ---------------
     # (inside the headline region its launches share the SMs with the other stream's stencil, so a

@@ -1,4 +1,7 @@
 """GPU parity, 3-D path (bio/neighbor.pyx) against the oracle."""
+import hashlib
+import os
+
 import numpy as np
 import pytest
 
@@ -6,10 +9,17 @@ from conftest import smooth_image
 
 pytestmark = pytest.mark.gpu
 RTOL, ATOL_F32, ATOL_F64 = 1e-5, 2e-6, 1e-12
+GOLD = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_vectors.npz"))
 
 
 def _cuda(torch, a):
     return torch.from_numpy(np.ascontiguousarray(a)).cuda()
+
+
+def _golden_padded_volume():
+    """The padded input the reference stencils were run on for tests/golden/reference_vectors.npz."""
+    vol = GOLD["vol3d"]
+    return np.pad(vol / vol.max(), 5, mode="edge")
 
 
 @pytest.mark.parametrize("shape,params", [((3, 4, 5), (11, 9, 9)), ((9, 8, 33), (11, 9, 9)), ((6, 5, 7), (7, 5, 4)),
@@ -24,10 +34,11 @@ def test_line_profile_v2_bit_exact(torch_cuda, oracle, shape, params):
     assert np.array_equal(got, want)
 
 
-def test_line_profile_v2_vs_compiled_reference(torch_cuda, ref3d):
+def test_line_profile_v2_vs_compiled_reference(torch_cuda):
+    """Against the output of the unmodified reference stencil, stored in tests/golden/reference_vectors.npz."""
     import neighbor
-    a = np.random.default_rng(2).random((17, 19, 21))
-    assert np.array_equal(neighbor.line_profile_v2(a, 11, 9, 9), ref3d.line_profile_v2(a, 11, 9, 9))
+    lp = neighbor.line_profile_v2(_golden_padded_volume(), 11, 9, 9)
+    assert hashlib.sha256(lp.tobytes()).digest() == GOLD["lp3d_sha256"].tobytes()
 
 
 @pytest.mark.parametrize("shape,params", [((9, 10, 40), (11, 9, 9)), ((4, 3, 5), (11, 9, 9)), ((6, 5, 7), (7, 5, 4)),
@@ -42,11 +53,10 @@ def test_memory_efficient_v2(torch_cuda, oracle, shape, params):
     np.testing.assert_allclose(got, want, rtol=1e-12, atol=1e-15)
 
 
-def test_memory_efficient_v2_vs_compiled_reference(torch_cuda, ref3d):
+def test_memory_efficient_v2_vs_compiled_reference(torch_cuda):
     import neighbor
-    a = smooth_image((14, 15, 16), 4).astype(np.float64)      # 4x5x6 voxels: the reference is slow
-    got = neighbor.line_profile_memory_efficient_v2(a, 11, 9, 9)
-    np.testing.assert_allclose(got, ref3d.line_profile_memory_efficient_v2(a, 11, 9, 9), rtol=1e-12, atol=1e-15)
+    got = neighbor.line_profile_memory_efficient_v2(_golden_padded_volume(), 11, 9, 9)
+    np.testing.assert_allclose(got, GOLD["me2_3d"], rtol=1e-12, atol=1e-15)
 
 
 def test_memory_efficient_v2_host_bands(torch_cuda):
@@ -104,19 +114,20 @@ def test_lne3d_generic_parameters(torch_cuda, oracle, flavour):
     np.testing.assert_allclose(got, want, rtol=RTOL, atol=ATOL_F64)
 
 
-def test_memory_efficient_v3(torch_cuda, oracle, ref3d):
-    """v3 reads outside its patch (flat addressing): equal to the oracle everywhere, NaN exactly
-    where the reference's read leaves the buffer, and equal to the compiled reference elsewhere."""
+def test_memory_efficient_v3(torch_cuda, oracle):
+    """v3 reads outside its patch (flat addressing).  On a smooth volume: equal to the oracle, NaN exactly where
+    the reference's read leaves the buffer.  On the input of tests/golden/reference_vectors.npz: equal to the
+    compiled reference's stored output on the first 6 rows, whose reads stay in the buffer."""
     import neighbor
     a = smooth_image((24, 15, 14), 7).astype(np.float64)
     got = neighbor.line_profile_memory_efficient_v3(a, 11, 9, 9)
     want = oracle.line_profile_memory_efficient_v3(a, 11, 9, 9)
     assert np.array_equal(np.isnan(got), np.isnan(want))
     np.testing.assert_allclose(got, want, rtol=1e-9, atol=1e-12, equal_nan=True)
-    ok = ~np.isnan(got)
-    assert ok.any()
-    ref = ref3d.line_profile_memory_efficient_v3(a, 11, 9, 9)
-    np.testing.assert_allclose(got[ok], ref[ok], rtol=1e-9, atol=1e-12)
+    assert (~np.isnan(got)).any()          # the comparison above is not over NaN alone
+    got = neighbor.line_profile_memory_efficient_v3(GOLD["v3_in"], 11, 9, 9)[:6]
+    assert not np.isnan(got).any()
+    np.testing.assert_allclose(got, GOLD["v3_out"], rtol=1e-9, atol=1e-12)
 
 
 def test_neighbor3d_score_pipeline(torch_cuda, oracle):

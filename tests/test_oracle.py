@@ -83,6 +83,38 @@ def test_3d_vs_compiled_reference(oracle, ref3d, params):
     assert np.array_equal(ref3d.line_profile_memory_efficient_v3(a, *params)[ok], got[ok])
 
 
+PARAMS = np.load(os.path.join(os.path.dirname(__file__), "golden", "oracle_params_vectors.npz"))
+
+
+def _sha(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).digest()
+
+
+@pytest.mark.parametrize("params", [(11, 9), (7, 5), (11, 4), (15, 9), (11, 12), (5, 3), (13, 16)])
+def test_line_profile_2d_frozen_at_other_parameters(oracle, params):
+    """The inputs of test_line_profile_2d_vs_compiled_reference against the oracle's frozen output
+    (tests/golden/make_golden_params.py): runs without oracle/_ref, so a change of the oracle at
+    non-default parameters is caught in a clean checkout too."""
+    P, R = params
+    a = np.random.default_rng(P * 100 + R).random((P + 12, P + 16))
+    assert _sha(oracle.line_profile_2d_v2(a, P, R)) == PARAMS["lp2d_sha256_%d_%d" % params].tobytes()
+
+
+@pytest.mark.parametrize("params", [(11, 9, 9), (7, 5, 4), (9, 6, 7), (5, 3, 3)])
+def test_3d_frozen_at_other_parameters(oracle, params):
+    """The inputs of test_3d_vs_compiled_reference against the oracle's frozen outputs
+    (tests/golden/make_golden_params.py)."""
+    P = params[0]
+    k = "%d_%d_%d" % params
+    a = np.random.default_rng(sum(params)).random((P + 10, P + 4, P + 3))
+    assert _sha(oracle.line_profile_v2(a, *params)) == PARAMS["lp3d_sha256_" + k].tobytes()
+    small = a[:P + 2, :P + 2, :P + 1]
+    assert np.array_equal(oracle.line_profile_memory_efficient_v2(small, *params), PARAMS["me2_3d_" + k])
+    got = oracle.line_profile_memory_efficient_v3(a, *params)
+    assert (~np.isnan(got)).any()
+    assert np.array_equal(got, PARAMS["v3_" + k], equal_nan=True)
+
+
 def test_identities_from_the_survey(oracle):
     """me_v2 == (v2[..., 5] - min) / max(max - min, 1e-8); percentiles of 9 values are order
     statistics 2 and 6; of 72 values they are lerps at 17.75 / 53.25."""
