@@ -18,6 +18,9 @@ _SIGNATURES = {
     "hipr_chansum": (_i, [_vp, _vp, _i64, _i, _vp, _i, _vp, _vp]),
     "hipr_chansum_raw": (_i, [_vp, _i, C.c_double, _i64, _i, _vp, _vp, _vp]),
     "hipr_register_stacks": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
+    "hipr_xcorr2d_workspace_bytes": (_i64, [_i, _i, _i]),
+    "hipr_register_translation_2d": (_i, [_vp, _vp, _i, _i, _i, _vp, _i64, _vp, _vp, _vp]),
+    "hipr_excitation_shifts": (_i, [_vp, _vp, _i, _i, _i, _i, C.c_double, _vp, _i64, _vp, _vp]),
     "hipr_image_range": (_i, [_vp, _i, _i64, _vp, _vp]),
     "hipr_normalize_cast": (_i, [_vp, _i64, _vp, _vp, _vp]),
     "hipr_normalize": (_i, [_vp, _i, _i64, _vp, _vp]),

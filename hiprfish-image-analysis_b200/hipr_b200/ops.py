@@ -4,6 +4,7 @@ runs here is one of libhipr_b200's.  No CPU fallback: CPU tensors are rejected.
 
 Reference blocks replaced (paths relative to the reference repository):
   register_stacks   syn/hiprfish_imaging_multispecies_spectral_image_measurement.py:86-105
+  excitation_shifts syn/hiprfish_imaging_multispecies_spectral_image_measurement.py:83-85 (register_translation)
   channel_sum       syn/hiprfish_imaging_multispecies_spectral_image_measurement.py:105-106
   lne2d             eco/neighbor2d.pyx:56-63 + syn/...measurement.py:109-124 (F1), bio F2 / F3
   neighbor2d_score  syn/...measurement.py:105-124 without the skimage denoise
@@ -129,8 +130,8 @@ def register_stacks(stacks, shifts=None, calibration=None, return_cube=True):
 
     stacks: list of (H, W, c_e) float32 CUDA tensors, one per excitation; shifts: per stack (row, col)
     integer shifts as the scripts derive them from register_translation (int(shift_vector)), None = no
-    shift; calibration: None or a (H, W, C) float32 divisor.  Returns (cube (H, W, C) float32 or None,
-    channel sums (H, W) float64, MaxKey)."""
+    shift, "estimate" = excitation_shifts(stacks) first (one synchronisation); calibration: None or a
+    (H, W, C) float32 divisor.  Returns (cube (H, W, C) float32 or None, channel sums (H, W) float64, MaxKey)."""
     stacks = [_dev(s, "stack %d" % i, (torch.float32,)) for i, s in enumerate(stacks)]
     if not stacks:
         raise ValueError("need at least one excitation stack")
@@ -141,6 +142,10 @@ def register_stacks(stacks, shifts=None, calibration=None, return_cube=True):
     n = len(stacks)
     if shifts is None:
         shifts = [(0, 0)] * n
+    elif isinstance(shifts, str):
+        if shifts != "estimate":
+            raise ValueError("shifts must be None, 'estimate' or one (row, col) per stack")
+        shifts = excitation_shifts(stacks)
     if len(shifts) != n:
         raise ValueError("one (row, col) shift per stack")
     chans = np.asarray([s.shape[2] for s in stacks], dtype=np.int32)
@@ -167,10 +172,84 @@ def register_stacks(stacks, shifts=None, calibration=None, return_cube=True):
 
 def neighbor2d_score_from_stacks(stacks, shifts=None, calibration=None, flavour="F1", return_cube=True):
     """syn/..._measurement.py:86-124 without the skimage calls: excitation stacks -> registered cube,
-    channel sums, score map (fixed-point stencil).  Returns (score, cube, sums, MaxKey)."""
+    channel sums, score map (fixed-point stencil); shifts as register_stacks ("estimate": estimated from the
+    stacks with excitation_shifts).  Returns (score, cube, sums, MaxKey)."""
     cube, s64, mk = register_stacks(stacks, shifts, calibration, return_cube)
     score = lne2d_fixed(s64, flavour, 11, 9, padded=False, range_keys=mk)
     return score, cube, s64, mk
+
+
+def _xcorr_workspace(H, W, n, device):
+    need = int(lib().hipr_xcorr2d_workspace_bytes(int(H), int(W), int(n)))
+    if need < 0:
+        if need == -9:
+            raise ValueError("image height and width must each be a power of two in [2, 8192], got (%d, %d)" % (H, W))
+        check(need, "xcorr2d_workspace_bytes")
+    return torch.empty(need, dtype=torch.uint8, device=device)
+
+
+def register_translation(src, target, return_correlation=False):
+    """skimage.feature.register_translation(src, target)[0] (upsample_factor=1, space="real") on the device, as
+    syn/...measurement.py:83-85 calls it: the peak of |ifftn(fftn(src) * conj(fftn(target)))| in float64 FFTs
+    (csrc/xcorr2d.cu), numpy's argmax order, indices above n // 2 wrapped to negative shifts.
+    src, target: (H, W) float32 / float64 CUDA tensors of the same shape and dtype, H and W powers of two in
+    [2, 8192].  Returns the (row, col) shift as a numpy (2,) float64 array (synchronises once); with
+    return_correlation also the (H, W) float64 |cc| tensor."""
+    src = _dev(src, "src")
+    target = _dev(target, "target")
+    if src.dim() != 2 or src.shape != target.shape:
+        raise ValueError("src and target must be 2-D images of the same shape")
+    if src.dtype != target.dtype:
+        raise TypeError("src and target must have the same dtype, got %s and %s" % (src.dtype, target.dtype))
+    if src.device != target.device:
+        raise ValueError("src and target must be on the same device")
+    H, W = src.shape
+    dev = src.device
+    work = _xcorr_workspace(H, W, 2, dev)
+    shift = torch.empty(2, dtype=torch.float64, device=dev)
+    corr = torch.empty((H, W), dtype=torch.float64, device=dev) if return_correlation else None
+    with torch.cuda.device(dev):
+        check(lib().hipr_register_translation_2d(C.c_void_p(src.data_ptr()), C.c_void_p(target.data_ptr()),
+                                                 _DT[src.dtype], H, W, C.c_void_p(work.data_ptr()), work.numel(),
+                                                 C.c_void_p(shift.data_ptr()),
+                                                 C.c_void_p(corr.data_ptr()) if corr is not None else None,
+                                                 _stream()), "register_translation")
+    out = shift.cpu().numpy()
+    return (out, corr) if return_correlation else out
+
+
+SHIFT_TRANSFORMS = {None: 0, "log": 1}
+
+
+def excitation_shifts(stacks, transform="log", eps=0.0):
+    """The scripts' registration shifts (syn/...measurement.py:83-85) on the device: per excitation stack the float64
+    channel sum, transformed (transform="log": ln(sum + eps); None: the sum itself), then
+    register_translation(T(sum_0), T(sum_e)) for every e >= 1; row 0 is (0, 0).  The default "log" is a reading of
+    the scripts that has not been confirmed against them.  stacks: list of (H, W, c_e) float32 CUDA tensors (the
+    register_stacks input), H and W powers of two in [2, 8192].  Returns a numpy (n, 2) float64 array (synchronises
+    once)."""
+    if transform not in SHIFT_TRANSFORMS:
+        raise ValueError("transform must be None or 'log'")
+    stacks = [_dev(s, "stack %d" % i, (torch.float32,)) for i, s in enumerate(stacks)]
+    if not stacks:
+        raise ValueError("need at least one excitation stack")
+    H, W = stacks[0].shape[:2]
+    for s in stacks:
+        if s.dim() != 3 or tuple(s.shape[:2]) != (H, W) or s.device != stacks[0].device:
+            raise ValueError("every stack must be (H, W, c_e) with the same H, W, on the same device")
+    n = len(stacks)
+    if n > 8:
+        raise ValueError("at most 8 excitation stacks")
+    dev = stacks[0].device
+    work = _xcorr_workspace(H, W, n, dev)
+    shifts = torch.empty((n, 2), dtype=torch.float64, device=dev)
+    chans = np.asarray([s.shape[2] for s in stacks], dtype=np.int32)
+    ptrs = (C.c_void_p * n)(*[s.data_ptr() for s in stacks])
+    with torch.cuda.device(dev):
+        check(lib().hipr_excitation_shifts(ptrs, chans.ctypes.data_as(C.c_void_p), n, H, W,
+                                           SHIFT_TRANSFORMS[transform], float(eps), C.c_void_p(work.data_ptr()),
+                                           work.numel(), C.c_void_p(shifts.data_ptr()), _stream()), "excitation_shifts")
+    return shifts.cpu().numpy()
 
 
 def denoise_nl_means(image, patch_size=7, patch_distance=11, h=0.1):

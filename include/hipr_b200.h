@@ -97,11 +97,33 @@ int hipr_chansum_raw(const void *cube_dev, int sample_bytes, double scale, int64
  *               `image_registered` the scripts save and run the per-cell reduction on
  *   sum_dev     (H, W) float64 channel sums of the registered, flat-fielded cube
  *   maxkey_dev  NULL or two keys (max, min of the sums), as hipr_chansum
- * The shifts themselves come from the caller (skimage.feature.register_translation is out of scope).
+ * The shifts can be estimated on the device from the same stacks with hipr_excitation_shifts (below).
  */
 int hipr_register_stacks(const float *const *stacks_dev, const int32_t *chans, const int32_t *shift_row,
                          const int32_t *shift_col, int n_stacks, int H, int W, const float *calib_dev,
                          float *cube_dev, double *sum_dev, uint64_t *maxkey_dev, void *stream);
+
+/* ---- registration shifts: float64 FFT cross-correlation (csrc/xcorr2d.cu) ---------------------------------------
+ * Replaces skimage.feature.register_translation(src, target)[0] with its defaults (upsample_factor 1, space "real"),
+ * syn/..._measurement.py:83-85: cc = ifftn(fftn(src) * conj(fftn(target))), the peak of |cc| by numpy's argmax
+ * (a NaN wins over any number, ties go to the lowest flat index), and an index i > n // 2 wrapped to i - n.
+ * Parity unpinned: scikit-image is not pinned by the reference (tests/shift_oracle.py::register_translation).
+ * H and W are each a power of two in [2, 8192] (HIPR_E_UNSUPPORTED otherwise).  All arithmetic is float64.
+ * hipr_xcorr2d_workspace_bytes: device scratch for n_images (2 for hipr_register_translation_2d, n_stacks for
+ *   hipr_excitation_shifts; at most 8); negative for an unsupported size.  A smaller workspace is HIPR_E_RANGE.
+ * hipr_register_translation_2d: src_dev, target_dev (H, W) of dtype; shift_dev receives (row, col) float64 with
+ *   integer values; corr_dev NULL or (H, W) float64 receives |cc|.
+ * hipr_excitation_shifts: the scripts' shifts for the excitation stacks of hipr_register_stacks (same stacks_dev,
+ *   chans): per stack the float64 channel sum (hipr_chansum), transformed (transform 0: none; 1: log(sum + eps)),
+ *   then register_translation(T(sum_0), T(sum_e)) for e >= 1; shifts_dev (n_stacks, 2) float64, row 0 = (0, 0).
+ * Both only enqueue work on `stream`. */
+int64_t hipr_xcorr2d_workspace_bytes(int H, int W, int n_images);
+int hipr_register_translation_2d(const void *src_dev, const void *target_dev, int dtype, int H, int W,
+                                 void *work_dev, int64_t work_bytes, double *shift_dev, double *corr_dev,
+                                 void *stream);
+int hipr_excitation_shifts(const float *const *stacks_dev, const int32_t *chans, int n_stacks, int H, int W,
+                           int transform, double eps, void *work_dev, int64_t work_bytes, double *shifts_dev,
+                           void *stream);
 
 /* global min / max of any image as keys: range_dev[0] = max key, range_dev[1] = min key */
 int hipr_image_range(const void *image_dev, int dtype, int64_t n, uint64_t *range_dev, void *stream);
