@@ -129,29 +129,39 @@ kmeans1d_kernel(KmCtx ctx, int64_t n, int k, int n_init, int max_iter, double to
     // after reduce_all(v, 1, ..) of a pass whose v[0] is a weight sum: finds, for each of `nt` targets r[m], the first
     // sample (raster order over the valid samples) whose inclusive prefix sum of weights reaches r[m], and stores its
     // centred value in out_global[m].  weight(i, value) is re-evaluated by the owning warp.  Uses the partials of the
-    // pass just reduced: slot index 0 of parity^1 (block sums) and s_warp[.][0] (warp sums).
+    // pass just reduced: slot index 0 of parity^1 (block sums) and s_warp[.][0] (warp sums).  Blocks and warps without
+    // a valid sample are skipped (their sums are exactly 0, so the prefixes do not change): a target r <= 0, which
+    // k-means++ draws once the seeds cover every distinct value, then picks the first valid sample, as searchsorted
+    // does.  Where rounding leaves r above every prefix of the blocks, or of the chosen block's warps, the last valid
+    // sample there is taken (numpy clips to the last index).  Exactly one warp writes out_global[m].
     auto locate = [&](const double *r, int nt, double mean, auto weight, double *out_global) {
         const int pp = parity ^ 1;
         for (int m = 0; m < nt; ++m) {
-            // block: first g with prefix_inclusive >= r (all CTAs agree); the last block takes what rounding leaves over
-            double before = 0.0;
-            int gb = G - 1;
+            // block: first g with prefix_inclusive >= r (all CTAs agree)
+            double target = r[m], before = 0.0;
+            int gb = -1, glast = -1;
             for (int g = 0; g < G; ++g) {
+                if (!(__ldcg(&work->blockcnt[g]) > 0.0)) continue;
+                glast = g;
                 const double s = __ldcg(&work->part[pp][g][0]);
-                if (before + s >= r[m]) { gb = g; break; }
+                if (before + s >= target) { gb = g; break; }
                 before += s;
             }
+            if (gb < 0) { gb = glast; target = INFINITY; }
             if (gb != b) continue;
             double wbefore = before;
-            int wb = KM_WARPS - 1;
+            int wb = -1, wlast = -1;
             for (int w = 0; w < KM_WARPS; ++w) {
-                if (wbefore + s_warp[w][0] >= r[m]) { wb = w; break; }
+                if (!(s_cnt_warp[w] > 0.0)) continue;
+                wlast = w;
+                if (wbefore + s_warp[w][0] >= target) { wb = w; break; }
                 wbefore += s_warp[w][0];
             }
+            if (wb < 0) { wb = wlast; target = INFINITY; }
             if (wb != warp) continue;
             // this warp: walk the piece 32 samples at a time with an inclusive warp scan
             double run = wbefore, found_val = 0.0, last_valid = 0.0;
-            bool found = false, any_valid = false;
+            bool found = false;
             for (int64_t i0 = w0; i0 < w1 && !found; i0 += 32) {
                 const int64_t i = i0 + lane;
                 double v = 0.0, raw, wgt = 0.0;
@@ -167,21 +177,17 @@ kmeans1d_kernel(KmCtx ctx, int64_t n, int k, int n_init, int max_iter, double to
                     const double t = __shfl_up_sync(0xffffffffu, inc, o);
                     if (lane >= o) inc += t;
                 }
-                const unsigned hit = __ballot_sync(0xffffffffu, ok && (run + inc >= r[m]));
+                const unsigned hit = __ballot_sync(0xffffffffu, ok && (run + inc >= target));
                 const unsigned okm = __ballot_sync(0xffffffffu, ok);
-                if (okm) {
-                    any_valid = true;
-                    last_valid = __shfl_sync(0xffffffffu, v, 31 - __clz(okm));
-                }
+                if (okm) last_valid = __shfl_sync(0xffffffffu, v, 31 - __clz(okm));
                 if (hit) {
                     found = true;
                     found_val = __shfl_sync(0xffffffffu, v, __ffs(hit) - 1);
                 }
                 run += __shfl_sync(0xffffffffu, inc, 31);
             }
-            // rounding can leave the target just above the last prefix: numpy clips to the last index
-            if (!found && any_valid) { found = true; found_val = last_valid; }
-            if (lane == 0 && found) out_global[m] = found_val;
+            // rounding can leave the target just above the warp's last prefix: the warp has a valid sample, take its last
+            if (lane == 0) out_global[m] = found ? found_val : last_valid;
         }
     };
 
@@ -389,7 +395,7 @@ kmeans1d_kernel(KmCtx ctx, int64_t n, int k, int n_init, int max_iter, double to
             }
             reduce_all(acc, k + 1, tot);
         }
-        // best of n_init: better inertia and a different clustering (in 1-D the sorted cluster sizes identify it)
+        // best of n_init: better inertia and a different clustering (in 1-D the cluster sizes in centre order identify it)
         bool take = (best_init < 0);
         if (!take && tot[k] < best_inertia) {
             double a[KM_MAXK], bb[KM_MAXK], ca[KM_MAXK], cb[KM_MAXK];

@@ -842,6 +842,9 @@ def kmeans_threshold(image, n_clusters=2, random_state=0, n_init=1, transform=No
     if not isinstance(random_state, (int, np.integer)):
         raise TypeError("random_state must be an integer seed (the reference passes 0)")
     nu = lib().hipr_kmeans1d_uniforms(k, int(n_init))
+    if nu == -7:                                     # HIPR_E_RANGE: KM_MAXU = 256 seeding draws in the kernel
+        raise ValueError("kmeans_threshold: n_init=%d is too large for k=%d: the kernel holds 256 seeding draws, %d per "
+                         "initialisation" % (int(n_init), k, lib().hipr_kmeans1d_uniforms(k, 1)))
     check(nu if nu < 0 else 0, "kmeans_threshold")
     # scikit-learn's draws, in its order: RandomState(seed).choice (one double) then uniform(size=trials) per seed
     u = np.ascontiguousarray(np.random.RandomState(int(random_state)).random_sample(nu), dtype=np.float64)

@@ -652,7 +652,8 @@ def _kmeans_finish(img, valid, labels_valid, k, fill_label=0):
     return labels, valid & (labels == bright), pm, bright
 
 
-def kmeans1d_sklearn(image, n_clusters=2, random_state=0, n_init=1, transform=None, eps=0.0, positive_only=False):
+def kmeans1d_sklearn(image, n_clusters=2, random_state=0, n_init=1, transform=None, eps=0.0, positive_only=False,
+                     max_iter=300, tol=1e-4):
     """THE pinned oracle of this row: scikit-learn itself (1.9.0 in this image), called as the scripts call it:
     KMeans(n_clusters = k, random_state = 0).fit_predict(x.reshape(-1, 1))  (syn/..._measurement.py:125, 141;
     bio/..._analysis.py:367, 384, 463, 819, 830; eco/..._measurement.py:73, 85).  n_init=1 is scikit-learn >= 1.4's
@@ -660,7 +661,8 @@ def kmeans1d_sklearn(image, n_clusters=2, random_state=0, n_init=1, transform=No
     Returns (cluster_centers_ (k,), labels (image shape, int32), foreground mask, n_iter, inertia)."""
     from sklearn.cluster import KMeans
     img, valid, x = _kmeans_samples(image, transform, eps, positive_only)
-    km = KMeans(n_clusters=n_clusters, random_state=random_state, n_init=n_init).fit(x.reshape(-1, 1))
+    km = KMeans(n_clusters=n_clusters, random_state=random_state, n_init=n_init, max_iter=max_iter,
+                tol=tol).fit(x.reshape(-1, 1))
     labels, mask, _, _ = _kmeans_finish(img, valid, km.labels_, n_clusters)
     return km.cluster_centers_.ravel().copy(), labels, mask, int(km.n_iter_), float(km.inertia_)
 
@@ -669,14 +671,17 @@ def kmeans1d(image, n_clusters=2, random_state=0, n_init=1, transform=None, eps=
              tol=1e-4):
     """numpy restatement of what scikit-learn 1.9.0's KMeans does on one feature (sklearn/cluster/_kmeans.py:
     fit -> _kmeans_plusplus -> _kmeans_single_lloyd), checked label for label against kmeans1d_sklearn in
-    tests/test_oracle.py.  It documents exactly what the CUDA kernel reproduces:
+    tests/test_kmeans.py and tests/test_kmeans_sweep.py.  It documents exactly what the CUDA kernel reproduces:
       * X is centred by its mean; tol_abs = tol * var(X);
       * seeding: first seed = sample floor(u0 * n) (RandomState.choice with uniform p); every further seed: `trials`
         = 2 + int(log(k)) candidates at searchsorted(cumsum(closest_dist_sq), u * current_pot), keep the one with the
-        smallest new potential;
+        smallest new potential (a target of 0, once the seeds cover every distinct value, picks the first sample);
       * Lloyd: label = argmin_j(c_j^2 - 2 x c_j) (first minimum), centres = cluster means; stop when the labels did not
         change (in 1-D: the cluster sizes) or sum((c_new - c_old)^2) <= tol_abs; labels are then those of the final centres;
-      * best of n_init by inertia (first wins ties).
+      * a Lloyd step that leaves a cluster empty raises RuntimeError (scikit-learn relocates the cluster and warns
+        that fewer distinct clusters than n_clusters were found; neither is reproduced);
+      * best of n_init by inertia (first wins ties), and only when the clustering differs from the best so far: in 1-D
+        a clustering is identified by its cluster sizes in centre order (scikit-learn's _is_same_clustering).
     Returns like kmeans1d_sklearn."""
     img, valid, x = _kmeans_samples(image, transform, eps, positive_only)
     k, n = int(n_clusters), x.size
@@ -706,6 +711,8 @@ def kmeans1d(image, n_clusters=2, random_state=0, n_init=1, transform=None, eps=
         for it in range(max_iter):
             lab = np.argmin(centers[None, :] ** 2 - 2 * xc[:, None] * centers[None, :], axis=1)
             counts = np.bincount(lab, minlength=k)
+            if not counts.all():
+                raise RuntimeError("a cluster ran empty during Lloyd iterations (scikit-learn would relocate it; not reproduced)")
             new = np.bincount(lab, weights=xc, minlength=k) / counts
             shift = ((new - centers) ** 2).sum()
             centers = new
@@ -716,8 +723,8 @@ def kmeans1d(image, n_clusters=2, random_state=0, n_init=1, transform=None, eps=
             counts_old = counts
         lab = np.argmin(centers[None, :] ** 2 - 2 * xc[:, None] * centers[None, :], axis=1)
         inertia = float(((xc - centers[lab]) ** 2).sum())
-        if best is None or (inertia < best[0] and not np.array_equal(np.sort(np.bincount(lab, minlength=k)[np.argsort(centers)]),
-                                                                      np.sort(best[4]))):
-            best = (inertia, centers + mean, lab, it + 1, np.bincount(lab, minlength=k)[np.argsort(centers)])
+        sizes = np.bincount(lab, minlength=k)[np.argsort(centers)]
+        if best is None or (inertia < best[0] and not np.array_equal(sizes, best[4])):
+            best = (inertia, centers + mean, lab, it + 1, sizes)
     labels, mask, _, _ = _kmeans_finish(img, valid, best[2], k)
     return best[1], labels, mask, best[3], best[0]

@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 
 sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
-from make_golden_kmeans import CASES, kmeans_case  # noqa: E402
+from make_golden_kmeans import CASES, case_image, kmeans_case  # noqa: E402
 
 GOLD = np.load(os.path.join(os.path.dirname(__file__), "golden", "kmeans_vectors.npz"))
 
@@ -21,7 +21,7 @@ def _sha(a):
 @pytest.mark.parametrize("i", range(len(CASES)))
 def test_restatement_matches_golden_sklearn(oracle, i):
     seed, k, n_init, tr, eps, pos = CASES[i]
-    img = kmeans_case(seed)
+    img = case_image(seed)
     assert np.array_equal(_sha(img), GOLD["case%d_img_sha256" % i])
     cen, labels, mask, n_iter, inertia = oracle.kmeans1d(img, k, 0, n_init, tr, eps, pos)
     np.testing.assert_allclose(cen, GOLD["case%d_centers" % i], rtol=0, atol=1e-12)
@@ -78,7 +78,7 @@ def _threshold_band(cen, x, delta):
 def test_gpu_kmeans_matches_sklearn_golden(torch_cuda, oracle, i):
     import hipr_b200
     seed, k, n_init, tr, eps, pos = CASES[i]
-    img = kmeans_case(seed)
+    img = case_image(seed)
     res = hipr_b200.kmeans_threshold(torch_cuda.from_numpy(img).cuda(), k, 0, n_init, tr, eps, pos)
     want_c = GOLD["case%d_centers" % i]
     np.testing.assert_allclose(res.cluster_centers_, want_c, rtol=0, atol=1e-9)      # the bar is 1e-6
