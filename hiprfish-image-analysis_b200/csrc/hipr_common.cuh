@@ -228,9 +228,11 @@ __device__ __forceinline__ double sum_channels_raw(const InT *__restrict__ p, in
 // DFMA) made the kernel latency-bound at a third of the HBM rate, so the quotient is formed as
 //   v / w = v*r0 * (1 + e + e^2 + O(e^3)),  r0 = RCP(w) in float32 (|e| <= ~1.2e-7),  e = 1 - w*r0
 // with v*r0 taken exactly in float64 (two 24-bit significands) and the O(1e-7) correction in
-// float32: the result differs from the correctly rounded quotient by <= ~2e-14 relative (the float32
-// rounding of the correction term), far inside what the fixed-point stencil resolves (4.6e-10 of the
-// image range).  One DFMA, three XU operations and four FFMA per channel.
+// float32: four float32 roundings (e, e + e^2, v*r0, the fma into the accumulator), each <= 2^-24
+// relative, of a correction <= 2^-23 of the term (rcp.approx is within 1 ulp) put a term within
+// 2^-45 + 2^-52 = 2.9e-14 of numpy's float64 quotient (tests/test_gpu_quotients.py checks every
+// divisor significand), far inside what the fixed-point stencil resolves (4.6e-10 of the image
+// range).  One DFMA, three XU operations and four FFMA per channel.
 __device__ __forceinline__ float rcp_approx(float w) {
     float r;
     asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(w));   // one MUFU.RCP, <= 1 ulp
@@ -272,9 +274,13 @@ __device__ __forceinline__ double sum_channels_div(const float *__restrict__ p, 
     const double total = ((a0 + a1) + (a2 + a3)) + (double)((k0 + k1) + (k2 + k3));
     // A divisor that is zero, denormal (flushed) or non-finite, or a non-finite numerator, makes r0 or e
     // infinite / NaN and therefore the total non-finite: that pixel is redone with numpy's own float64
-    // quotients, channel by channel (never taken on real flat fields).  A divisor above 2^126 has its
-    // reciprocal flushed to zero: the term becomes 0 instead of ~v * 1e-38.
-    if (!(fabs(total) < 1.7e308)) return sum_channels_div_exact(p, q, C);
+    // quotients, channel by channel (never taken on real flat fields).  So is a non-zero total below 2^-90:
+    // there the float32 correction terms (<= 2^-23 of a quotient) fall below 2^-126, and each denormal rounding
+    // loses up to 2^-150 absolute -- for denormal numerators the whole correction, up to 2^-23 of the total.
+    // Above 2^-90 those roundings stay below 2^-52 of the total.  A divisor above 2^126 has its reciprocal
+    // flushed to zero: the term becomes 0 instead of ~v * 1e-38 (the exact path, when taken, keeps it).
+    const double mag = fabs(total);
+    if (!(mag < 1.7e308) || (mag < 0x1p-90 && mag != 0.0)) return sum_channels_div_exact(p, q, C);
     return total;
 }
 
