@@ -165,7 +165,7 @@ extern "C" int hipr_paint_labels(const void *labels_dev, int label_bytes, int64_
                                  int64_t max_label, int dtype, void *out_dev, void *stream) {
     if (!labels_dev || !values_dev || !out_dev || npix < 1 || K < 1 || max_label < 0) return HIPR_E_ARG;
     if (label_bytes != 4 && label_bytes != 8) return HIPR_E_DTYPE;
-    if (dtype != HIPR_F32 && dtype != HIPR_F64) return HIPR_E_DTYPE;
+    if (dtype < HIPR_F32 || dtype > HIPR_U8) return HIPR_E_DTYPE;
     cudaStream_t st = (cudaStream_t)stream;
     int64_t blocks = (npix * K + 1023) / 1024;
     const int64_t cap = (int64_t)sm_count() * 16;
@@ -173,10 +173,17 @@ extern "C" int hipr_paint_labels(const void *labels_dev, int label_bytes, int64_
 #define HIPR_PAINT(LT, VT)                                                                                         \
     paint_kernel<LT, VT><<<(unsigned)blocks, 256, 0, st>>>((const LT *)labels_dev, npix, (const VT *)values_dev, K, \
                                                           max_label, (VT *)out_dev)
-    if (label_bytes == 4 && dtype == HIPR_F32) HIPR_PAINT(int, float);
-    else if (label_bytes == 4) HIPR_PAINT(int, double);
-    else if (dtype == HIPR_F32) HIPR_PAINT(long long, float);
-    else HIPR_PAINT(long long, double);
+#define HIPR_PAINT_VALUES(LT)                                 \
+    switch (dtype) {                                          \
+        case HIPR_F32: HIPR_PAINT(LT, float); break;          \
+        case HIPR_F64: HIPR_PAINT(LT, double); break;         \
+        case HIPR_I32: HIPR_PAINT(LT, int); break;            \
+        case HIPR_I64: HIPR_PAINT(LT, long long); break;      \
+        default: HIPR_PAINT(LT, uint8_t); break;              \
+    }
+    if (label_bytes == 4) { HIPR_PAINT_VALUES(int) }
+    else { HIPR_PAINT_VALUES(long long) }
+#undef HIPR_PAINT_VALUES
 #undef HIPR_PAINT
     return after_launch();
 }

@@ -6,7 +6,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(os.path.dirname(_HERE), "libhipr_b200.so")
 
-F32, F64 = 0, 1
+F32, F64, I32, I64, U8 = 0, 1, 2, 3, 4
 FLAVOURS = {"F1": 1, "F2": 2, "F3": 3, "ME2": 4, "V3": 5}
 
 _vp, _i, _i64 = C.c_void_p, C.c_int, C.c_int64
@@ -46,6 +46,10 @@ _SIGNATURES = {
     "hipr_cell_moments": (_i, [_vp, _i, _i, _i, _i64, _vp, _vp]),
     "hipr_cell_geometry_finalize": (_i, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "hipr_paint_labels": (_i, [_vp, _i, _i64, _vp, _i, _i64, _i, _vp, _vp]),
+    "hipr_label_workspace_bytes": (_i64, [_i, _i, _i, _i]),
+    "hipr_label": (_i, [_vp, _i, _i, _i, _i, _i, _i, _i, _vp, _i64, _vp, _i, _vp, _vp]),
+    "hipr_label_counts": (_i, [_vp, _i, _i, _i, _i, _i, _i, _i64, _vp, _vp, _vp]),
+    "hipr_label_clear": (_i, [_vp, _i, _vp, _i64, _vp, _i64, _vp, _vp]),
     "hipr_kmeans1d_workspace_bytes": (_i64, []),
     "hipr_kmeans1d_uniforms": (_i, [_i, _i]),
     "hipr_kmeans1d": (_i, [_vp, _i, _i64, _i, C.c_double, _i, _i, _i, _vp, _i, C.c_double, _vp, _vp, _i, _vp, _vp, _vp]),

@@ -13,6 +13,9 @@ Reference blocks replaced (paths relative to the reference repository):
   lne3d_dirs        bio/neighbor.pyx:186-263
   lne3d             bio/neighbor.pyx + bio/hiprfish_imaging_biofilm_analysis.py:812-817, 905-917, 1114-1125
   cell_spectra      syn/...measurement.py:167-172
+  label, remove_small_objects, binary_fill_holes, clear_border, relabel_sequential
+                    the segmentation back end, syn/...measurement.py:125-158, eco/...measurement.py:73-127,
+                    bio/...analysis.py:367-419, 463-501
 """
 import ctypes as C
 
@@ -20,9 +23,10 @@ import numpy as np
 import torch
 
 from . import tables
-from ._lib import F32, F64, FLAVOURS, check, lib
+from ._lib import F32, F64, FLAVOURS, I32, I64, U8, check, lib
 
 _DT = {torch.float32: F32, torch.float64: F64}
+_VT = {torch.float32: F32, torch.float64: F64, torch.int32: I32, torch.int64: I64, torch.uint8: U8, torch.bool: U8}
 
 
 def _stream():
@@ -796,9 +800,10 @@ def orientation_xy(geometry):
 def paint_labels(labels, values, max_label=None):
     """out[p] = values[labels[p]]: the `image[segmentation == label] = value` loops of
     eco/hiprfish_imaging_image_classification.py:64-70 / bio/...analysis.py:1247-1257 as one gather.
-    values: (max_label + 1,) or (max_label + 1, K) float32 / float64, row 0 = background."""
+    values: (max_label + 1,) or (max_label + 1, K) float32 / float64 (or int32 / int64 / uint8 / bool lookup
+    tables), row 0 = background."""
     labels = _dev(labels, "labels", (torch.int32, torch.int64))
-    values = _dev(values, "values")
+    values = _dev(values, "values", tuple(_VT))
     squeeze = values.dim() == 1
     v2 = values.reshape(values.shape[0], -1)
     if max_label is None:
@@ -809,9 +814,174 @@ def paint_labels(labels, values, max_label=None):
     out = torch.empty(tuple(labels.shape) + (() if squeeze else (K,)), dtype=values.dtype, device=labels.device)
     with torch.cuda.device(labels.device):
         check(lib().hipr_paint_labels(C.c_void_p(labels.data_ptr()), labels.element_size(), labels.numel(),
-                                      C.c_void_p(v2.data_ptr()), K, int(max_label), _DT[values.dtype],
+                                      C.c_void_p(v2.data_ptr()), K, int(max_label), _VT[values.dtype],
                                       C.c_void_p(out.data_ptr()), _stream()), "paint_labels")
     return out
+
+
+# ---------------------------------------------------------------------------------------------
+# connected components (K10, csrc/label.cu)
+# Per-pixel work runs in libhipr_b200's kernels.  The per-label tables between them (n + 1 or max_label + 1
+# entries: which components to keep, the new numbering) are built with torch on the device.
+# ---------------------------------------------------------------------------------------------
+
+_LABEL_DT = {torch.bool: U8, torch.uint8: U8, torch.int32: I32, torch.int64: I64}
+
+
+def _label_input(image, name, dtypes=tuple(_LABEL_DT)):
+    """-> (contiguous tensor, with bool viewed as uint8; dtype code; (ndim, d0, d1, d2))."""
+    image = _dev(image, name, dtypes)
+    if image.dim() not in (2, 3):
+        raise ValueError("%s must be a 2-D image or a 3-D volume, got shape %s" % (name, tuple(image.shape)))
+    if image.numel() == 0:
+        raise ValueError("%s is empty" % name)
+    raw = image.view(torch.uint8) if image.dtype == torch.bool else image
+    shape = tuple(image.shape) + (1,) * (3 - image.dim())
+    return raw, _LABEL_DT[image.dtype], (image.dim(),) + shape
+
+
+def _connectivity(connectivity, ndim):
+    if connectivity is None:
+        return ndim
+    if isinstance(connectivity, bool) or not isinstance(connectivity, (int, np.integer)):
+        raise TypeError("connectivity must be an integer")
+    if not 1 <= connectivity <= ndim:
+        raise ValueError("connectivity must be in [1, %d], got %d" % (ndim, connectivity))
+    return int(connectivity)
+
+
+def _label(raw, code, dims, connectivity, invert=False, dtype=torch.int32):
+    """Labels and the component count n (a 1-element int64 device tensor); no synchronisation."""
+    ws = lib().hipr_label_workspace_bytes(*dims)
+    if ws < 0:
+        check(int(ws), "label (an image of 2^31 pixels or more)")
+    dev = raw.device
+    work = torch.empty(int(ws), dtype=torch.uint8, device=dev)
+    out = torch.empty(raw.shape, dtype=dtype, device=dev)
+    n = torch.empty(1, dtype=torch.int64, device=dev)
+    with torch.cuda.device(dev):
+        check(lib().hipr_label(C.c_void_p(raw.data_ptr()), code, int(invert), *dims, connectivity,
+                               C.c_void_p(work.data_ptr()), int(ws), C.c_void_p(out.data_ptr()), out.element_size(),
+                               C.c_void_p(n.data_ptr()), _stream()), "label")
+    return out, n
+
+
+def _label_counts(labels, dims, max_label, border=-1):
+    """np.bincount(labels, minlength=max_label + 1) as int32 (border >= 0: only the pixels within `border` of an
+    edge), and the number of labels outside [0, max_label]."""
+    dev = labels.device
+    counts = torch.empty(max_label + 1, dtype=torch.int32, device=dev)
+    over = torch.empty(1, dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        check(lib().hipr_label_counts(C.c_void_p(labels.data_ptr()), labels.element_size(), *dims, int(border),
+                                      int(max_label), C.c_void_p(counts.data_ptr()), C.c_void_p(over.data_ptr()),
+                                      _stream()), "label_counts")
+    return counts, over
+
+
+def label(image, connectivity=None, return_num=False, dtype=torch.int32):
+    """skimage.measure.label(image, background=0, connectivity=connectivity) on the device.
+
+    image: 2-D (H, W) or 3-D (X, Y, Z) CUDA tensor.  bool / uint8 is a mask (non-zero is foreground, as
+    scipy.ndimage.label); int32 / int64 is a label image whose neighbours connect when their values are equal and
+    non-zero.  connectivity 1 .. ndim (default ndim): 4 / 8 neighbours in 2-D, 6 / 18 / 26 in 3-D.  Components are
+    numbered 1 .. n in raster order of their first pixel.  -> labels of `dtype` (int32 or int64), and n when
+    return_num (the only case that synchronises)."""
+    if dtype not in (torch.int32, torch.int64):
+        raise TypeError("dtype must be torch.int32 or torch.int64")
+    raw, code, dims = _label_input(image, "image")
+    out, n = _label(raw, code, dims, _connectivity(connectivity, dims[0]), dtype=dtype)
+    return (out, int(n.item())) if return_num else out
+
+
+def remove_small_objects(ar, min_size=64, connectivity=1):
+    """skimage.morphology.remove_small_objects(ar, min_size, connectivity) on the device.
+
+    bool ar: components (scipy.ndimage.label with that connectivity) of fewer than min_size pixels become False;
+    the result is bool.  int32 / int64 ar: a label image whose labels are the components as they are (np.bincount
+    sizes, connectivity unused); labels of fewer than min_size pixels become 0, the dtype is kept, and a negative
+    label raises ValueError as np.bincount does.  Synchronises once (bool) or twice (labels)."""
+    raw, code, dims = _label_input(ar, "ar", (torch.bool, torch.int32, torch.int64))
+    conn = _connectivity(connectivity, dims[0])
+    min_size = int(min_size)
+    if min_size == 0:
+        return ar.clone()
+    if ar.dtype == torch.bool:
+        lab, n = _label(raw, code, dims, conn)
+        counts, _ = _label_counts(lab, dims, int(n.item()))
+        keep = (counts >= min_size).to(torch.uint8)
+        keep[0] = 0
+        return paint_labels(lab, keep).view(torch.bool)
+    max_label = int(label_max(raw).item())
+    counts, over = _label_counts(raw, dims, max_label)
+    if int(over.item()):
+        raise ValueError("remove_small_objects: negative labels (np.bincount: 'list' argument must have no negative "
+                         "elements)")
+    lut = torch.arange(max_label + 1, dtype=ar.dtype, device=raw.device) * (counts >= min_size).to(ar.dtype)
+    return paint_labels(raw, lut)
+
+
+def binary_fill_holes(mask, connectivity=1):
+    """scipy.ndimage.binary_fill_holes(mask, generate_binary_structure(ndim, connectivity)) on the device: the
+    background components (at that connectivity) that touch no edge of the image are filled.  mask: bool / uint8
+    (or int32 / int64, non-zero is foreground) 2-D or 3-D CUDA tensor -> bool.  Synchronises once."""
+    raw, code, dims = _label_input(mask, "mask")
+    lab, n = _label(raw, code, dims, _connectivity(connectivity, dims[0]), invert=True)
+    on_edge, _ = _label_counts(lab, dims, int(n.item()), border=0)
+    fill = (on_edge == 0).to(torch.uint8)
+    fill[0] = 1                                        # label 0: the mask's own foreground
+    return paint_labels(lab, fill).view(torch.bool)
+
+
+def clear_border(labels, buffer_size=0, bgval=0):
+    """skimage.segmentation.clear_border(labels, buffer_size, bgval) on the device.
+
+    The image is relabelled with label(labels, background=0) at full connectivity; every component with a pixel
+    within buffer_size of an edge is set to bgval, all other pixels keep their values.  The background is itself a
+    component there: when a zero lies in that band, every zero becomes bgval.  labels: bool / uint8 / int32 / int64,
+    2-D or 3-D; the result has its dtype.  ValueError if buffer_size >= a dimension.  Synchronises once."""
+    raw, code, dims = _label_input(labels, "labels")
+    buffer_size = int(buffer_size)
+    if buffer_size < 0:
+        raise ValueError("buffer_size must be >= 0")
+    if any(buffer_size >= s for s in labels.shape):
+        raise ValueError("buffer size may not be greater than labels size")
+    bgval = int(bool(bgval)) if labels.dtype == torch.bool else int(bgval)
+    info = torch.iinfo(raw.dtype)
+    if not info.min <= bgval <= info.max:
+        raise ValueError("bgval %d does not fit %s" % (bgval, raw.dtype))
+    lab, n = _label(raw, code, dims, dims[0])
+    on_edge, _ = _label_counts(lab, dims, int(n.item()), border=buffer_size)
+    out = torch.empty_like(raw)
+    with torch.cuda.device(raw.device):
+        check(lib().hipr_label_clear(C.c_void_p(raw.data_ptr()), code, C.c_void_p(lab.data_ptr()), raw.numel(),
+                                     C.c_void_p(on_edge.data_ptr()), bgval, C.c_void_p(out.data_ptr()), _stream()),
+              "clear_border")
+    return out.view(torch.bool) if labels.dtype == torch.bool else out
+
+
+def relabel_sequential(labels, offset=1):
+    """skimage.segmentation.relabel_sequential(labels, offset) on the device: the non-zero labels present, in
+    ascending order, become offset, offset + 1, ...; 0 stays 0.  labels: int32 / int64 -> (relabelled,
+    forward_map (max_label + 1,), inverse_map (offset + n,)), with forward_map[old] = new and inverse_map[new] = old
+    (the arrays behind scikit-image's ArrayMap).  The result keeps the input dtype unless the largest new label
+    needs int64.  ValueError for offset < 1 or a negative label.  Synchronises twice."""
+    raw, code, dims = _label_input(labels, "labels", (torch.int32, torch.int64))
+    if isinstance(offset, bool) or not isinstance(offset, (int, np.integer)) or offset < 1:
+        raise ValueError("Offset must be strictly positive.")
+    offset = int(offset)
+    max_label = int(label_max(raw).item())
+    counts, over = _label_counts(raw, dims, max_label)
+    if int(over.item()):
+        raise ValueError("Cannot relabel array that contains negative values.")
+    present = torch.nonzero(counts[1:]).flatten() + 1
+    n = present.numel()
+    out_dtype = raw.dtype if offset + n - 1 <= torch.iinfo(raw.dtype).max else torch.int64
+    forward = torch.zeros(max_label + 1, dtype=out_dtype, device=raw.device)
+    forward[present] = torch.arange(offset, offset + n, dtype=out_dtype, device=raw.device)
+    inverse = torch.zeros(offset + n, dtype=raw.dtype, device=raw.device)
+    inverse[offset:] = present.to(raw.dtype)
+    return paint_labels(raw, forward), forward, inverse
 
 
 # ---------------------------------------------------------------------------------------------

@@ -11,7 +11,8 @@
  * Conventions
  *  - All arrays are C-contiguous, channel (or line sample) fastest, exactly as the reference's
  *    numpy arrays are.  "dev" pointers are device pointers, "host" pointers host memory.
- *  - dtype codes: HIPR_F32 = 0 (float), HIPR_F64 = 1 (double).
+ *  - dtype codes: HIPR_F32 = 0 (float), HIPR_F64 = 1 (double); the label entry points and
+ *    hipr_paint_labels also take HIPR_I32 = 2, HIPR_I64 = 3 and HIPR_U8 = 4 (uint8 / bool).
  *  - Every function returns 0 on success, a negative HIPR_E* code for a rejected argument, or
  *    a positive cudaError_t value.  hipr_error_string() describes either.
  *  - `stream` is a cudaStream_t passed as void* (NULL = legacy default stream).  Device entry
@@ -34,6 +35,9 @@ extern "C" {
 
 #define HIPR_F32 0
 #define HIPR_F64 1
+#define HIPR_I32 2
+#define HIPR_I64 3
+#define HIPR_U8  4
 
 /* epilogue flavours (SURVEY.md section 8a) */
 #define HIPR_FLAVOUR_F1  1  /* syn/..._measurement.py:111-124 */
@@ -330,7 +334,8 @@ int hipr_cell_spectra_finalize(const double *sums_dev, const int32_t *counts_dev
  * hipr_paint_labels replaces the `image[segmentation == label] = value` loops,
  *   eco/hiprfish_imaging_image_classification.py:64-70, bio/..._analysis.py:1247-1257:
  *   out_dev[p, :] = values_dev[labels_dev[p], :], values_dev (max_label + 1, K) of dtype (row 0 = background);
- *   labels outside [0, max_label] take row 0.
+ *   labels outside [0, max_label] take row 0.  dtype HIPR_F32 / HIPR_F64, or HIPR_I32 / HIPR_I64 / HIPR_U8 for the
+ *   per-label lookup tables of the connected-component operators below.
  */
 int hipr_cell_moments(const void *labels_dev, int label_bytes, int H, int W, int64_t max_label,
                       uint64_t *moments_dev, void *stream);
@@ -339,6 +344,39 @@ int hipr_cell_geometry_finalize(const uint64_t *moments_dev, int64_t max_label, 
                                 double *geometry_out, void *stream);
 int hipr_paint_labels(const void *labels_dev, int label_bytes, int64_t npix, const void *values_dev, int K,
                       int64_t max_label, int dtype, void *out_dev, void *stream);
+
+/* ---- connected components (csrc/label.cu) ----------------------------------------------------------------------
+ * The segmentation back end between the k-means mask and the label image: syn/..._measurement.py:125-158,
+ * eco/..._measurement.py:73-127, bio/..._analysis.py:367-419, 463-501.
+ * hipr_label: scipy.ndimage.label(mask, generate_binary_structure(ndim, connectivity)) for a mask, and
+ *   skimage.measure.label(image, background=0, connectivity=connectivity) for a label image (neighbours connect
+ *   when their values are equal and non-zero; negative values are ordinary values).
+ *   image_dev   C-order (d0, d1) (ndim 2) or (d0, d1, d2) (ndim 3); dtype HIPR_U8: a mask, non-zero is foreground
+ *               (invert != 0: zero is foreground); HIPR_I32 / HIPR_I64: a label image
+ *   connectivity 1 .. ndim (4 / 8 neighbours in 2-D, 6 / 18 / 26 in 3-D)
+ *   labels_out  label_bytes 4 (int32) or 8 (int64): components numbered 1 .. n in raster order of their first
+ *               pixel (scipy's and scikit-image's numbering), 0 for the background
+ *   n_dev       one int64: n
+ *   workspace   hipr_label_workspace_bytes(ndim, d0, d1, d2) bytes (negative: HIPR_E_RANGE when the image has
+ *               2^31 pixels or more); what it holds before the call does not matter
+ *   Five launches whatever the image holds; no host synchronisation.
+ * hipr_label_counts: np.bincount of a label image into counts_dev (max_label + 1) int32, zeroed by the call.
+ *   border >= 0: only pixels within `border` of an edge count (skimage clear_border's band of buffer_size + 1
+ *   pixels); border < 0: all pixels.  Labels below 0 or above max_label are counted in *overflow_dev (may be NULL).
+ * hipr_label_clear: clear_border's write, out[p] = flagged_dev[labels_dev[p]] != 0 ? fill : image[p];
+ *   image_dev and out_dev (npix) of dtype HIPR_U8 / HIPR_I32 / HIPR_I64, labels_dev (npix) int32 in [0, n],
+ *   flagged_dev (n + 1) int32 (the border counts of hipr_label_counts).
+ * The per-label tables between these calls go through hipr_paint_labels (integer and uint8 values) and
+ * hipr_label_max.
+ */
+int64_t hipr_label_workspace_bytes(int ndim, int d0, int d1, int d2);
+int hipr_label(const void *image_dev, int dtype, int invert, int ndim, int d0, int d1, int d2, int connectivity,
+               void *workspace_dev, int64_t workspace_bytes, void *labels_out, int label_bytes, int64_t *n_dev,
+               void *stream);
+int hipr_label_counts(const void *labels_dev, int label_bytes, int ndim, int d0, int d1, int d2, int border,
+                      int64_t max_label, int32_t *counts_dev, int32_t *overflow_dev, void *stream);
+int hipr_label_clear(const void *image_dev, int dtype, const int32_t *labels_dev, int64_t npix,
+                     const int32_t *flagged_dev, int64_t fill, void *out_dev, void *stream);
 
 /* ---- 1-D k-means thresholding ---------------------------------------------------------------------------
  * Replaces KMeans(n_clusters = k, random_state = seed).fit_predict(image.reshape(-1, 1)) on the score map, the
