@@ -284,6 +284,27 @@ __device__ __forceinline__ double sum_channels_div(const float *__restrict__ p, 
     return total;
 }
 
+// ---------------------------------------------------------------------------------------
+// Grid barrier of the persistent cooperative kernels (K8, K11).  *counter is zeroed before the launch; every CTA
+// adds one per barrier and waits until the count reaches its target (gridDim.x per barrier passed so far).  The
+// comparison is wrap-safe, so the count may pass 2^32 in a long run.
+// ---------------------------------------------------------------------------------------
+__device__ __forceinline__ unsigned int ld_acquire_gpu(const unsigned int *p) {
+    unsigned int v;
+    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+    return v;
+}
+__device__ __forceinline__ void grid_barrier(unsigned int *counter, unsigned int &target) {
+    __syncthreads();
+    target += (unsigned)gridDim.x;
+    if (threadIdx.x == 0) {
+        __threadfence();
+        atomicAdd(counter, 1u);
+        while ((int)(ld_acquire_gpu(counter) - target) < 0) {}
+    }
+    __syncthreads();
+}
+
 __device__ __forceinline__ float warp_max(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));

@@ -41,12 +41,6 @@ struct KmWork {                       // global scratch, zeroed (first 64 bytes)
     double part[2][KM_MAXGRID][KM_SLOT];
 };
 
-__device__ __forceinline__ unsigned int ld_acquire_gpu(const unsigned int *p) {
-    unsigned int v;
-    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-
 struct KmCtx {
     const void *x;
     int dtype;         // HIPR_F32 / HIPR_F64
@@ -92,16 +86,7 @@ kmeans1d_kernel(KmCtx ctx, int64_t n, int k, int n_init, int max_iter, double to
     const int64_t w0 = c0 + (int64_t)warp * piece;
     const int64_t w1 = (w0 + piece < n) ? w0 + piece : n;
 
-    auto grid_barrier = [&]() {
-        __syncthreads();
-        bar_target += (unsigned)G;
-        if (tid == 0) {
-            __threadfence();
-            atomicAdd(&work->barrier, 1u);
-            while (ld_acquire_gpu(&work->barrier) < bar_target) {}
-        }
-        __syncthreads();
-    };
+    auto grid_barrier = [&]() { hipr::grid_barrier(&work->barrier, bar_target); };
     // every thread holds `nv` partial values v[0..nv): reduce over the block, publish the block partial in this
     // parity's slot, barrier, then every CTA sums all block partials in block order into tot[] (identical everywhere)
     auto reduce_all = [&](double *v, int nv, double *tot) {

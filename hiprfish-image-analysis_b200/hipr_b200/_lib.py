@@ -50,6 +50,8 @@ _SIGNATURES = {
     "hipr_label": (_i, [_vp, _i, _i, _i, _i, _i, _i, _i, _vp, _i64, _vp, _i, _vp, _vp]),
     "hipr_label_counts": (_i, [_vp, _i, _i, _i, _i, _i, _i, _i64, _vp, _vp, _vp]),
     "hipr_label_clear": (_i, [_vp, _i, _vp, _i64, _vp, _i64, _vp, _vp]),
+    "hipr_watershed_workspace_bytes": (_i64, [_i, _i, _i, _i, _i, _i]),
+    "hipr_watershed": (_i, [_vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _i, _vp, _i64, _vp, _vp, _vp]),
     "hipr_kmeans1d_workspace_bytes": (_i64, []),
     "hipr_kmeans1d_uniforms": (_i, [_i, _i]),
     "hipr_kmeans1d": (_i, [_vp, _i, _i64, _i, C.c_double, _i, _i, _i, _vp, _i, C.c_double, _vp, _vp, _i, _vp, _vp, _vp]),

@@ -13,8 +13,8 @@ Reference blocks replaced (paths relative to the reference repository):
   lne3d_dirs        bio/neighbor.pyx:186-263
   lne3d             bio/neighbor.pyx + bio/hiprfish_imaging_biofilm_analysis.py:812-817, 905-917, 1114-1125
   cell_spectra      syn/...measurement.py:167-172
-  label, remove_small_objects, binary_fill_holes, clear_border, relabel_sequential
-                    the segmentation back end, syn/...measurement.py:125-158, eco/...measurement.py:73-127,
+  label, remove_small_objects, binary_fill_holes, clear_border, relabel_sequential, watershed
+                    the segmentation back end, syn/...measurement.py:125-158, eco/...measurement.py:44-127,
                     bio/...analysis.py:367-419, 463-501
 """
 import ctypes as C
@@ -23,7 +23,7 @@ import numpy as np
 import torch
 
 from . import tables
-from ._lib import F32, F64, FLAVOURS, I32, I64, U8, check, lib
+from ._lib import F32, F64, FLAVOURS, I32, I64, U8, HiprError, check, lib
 
 _DT = {torch.float32: F32, torch.float64: F64}
 _VT = {torch.float32: F32, torch.float64: F64, torch.int32: I32, torch.int64: I64, torch.uint8: U8, torch.bool: U8}
@@ -985,6 +985,77 @@ def relabel_sequential(labels, offset=1):
 
 
 # ---------------------------------------------------------------------------------------------
+# marker watershed (K11, csrc/watershed.cu)
+# ---------------------------------------------------------------------------------------------
+
+# integer images become the float type that holds every value exactly
+_WS_EXACT = {torch.uint8: torch.float32, torch.uint16: torch.float32, torch.int32: torch.float64}
+
+
+def _watershed(image, markers, connectivity=1, mask=None):
+    """watershed's checks and launch -> (labels, status): status is the kernel's 8 int64 status words on the device
+    (hipr_b200.h: status, rounds and tile visits per phase, CTAs).  Synchronises once, for the NaN check."""
+    image = _dev(image, "image", (torch.float32, torch.float64) + tuple(_WS_EXACT))
+    markers = _dev(markers, "markers", (torch.int32, torch.int64))
+    if image.dim() not in (2, 3):
+        raise ValueError("image must be a 2-D image or a 3-D volume, got shape %s" % (tuple(image.shape),))
+    if image.numel() == 0:
+        raise ValueError("image is empty")
+    if markers.shape != image.shape:
+        raise ValueError("markers %s and image %s differ in shape" % (tuple(markers.shape), tuple(image.shape)))
+    if image.device != markers.device:
+        raise ValueError("image and markers are on different devices")
+    if mask is not None:
+        mask = _dev(mask, "mask", (torch.bool, torch.uint8))
+        if mask.shape != image.shape:
+            raise ValueError("mask %s and image %s differ in shape" % (tuple(mask.shape), tuple(image.shape)))
+        if mask.device != image.device:
+            raise ValueError("image and mask are on different devices")
+        mask = mask.view(torch.uint8) if mask.dtype == torch.bool else mask
+    conn = _connectivity(connectivity, image.dim())
+    if image.dtype in _WS_EXACT:
+        image = image.to(_WS_EXACT[image.dtype])
+    else:
+        nan = torch.isnan(image) if mask is None else torch.isnan(image) & (mask != 0)
+        if bool(nan.any()):
+            raise ValueError("image has NaN inside the mask: the flooding order is undefined there")
+    dims = (image.dim(),) + tuple(image.shape) + (1,) * (3 - image.dim())
+    code, lb = _DT[image.dtype], markers.element_size()
+    ws = lib().hipr_watershed_workspace_bytes(*dims, code, lb)
+    if ws < 0:
+        check(int(ws), "watershed (an image of 2^31 pixels or more)")
+    dev = image.device
+    work = torch.empty(int(ws), dtype=torch.uint8, device=dev)
+    out = torch.empty_like(markers)
+    status = torch.empty(8, dtype=torch.int64, device=dev)
+    with torch.cuda.device(dev):
+        check(lib().hipr_watershed(C.c_void_p(image.data_ptr()), code, C.c_void_p(markers.data_ptr()), lb,
+                                   C.c_void_p(mask.data_ptr()) if mask is not None else None, *dims, conn,
+                                   C.c_void_p(work.data_ptr()), int(ws), C.c_void_p(out.data_ptr()),
+                                   C.c_void_p(status.data_ptr()), _stream()), "watershed")
+    return out, status
+
+
+def watershed(image, markers, connectivity=1, mask=None):
+    """skimage.segmentation.watershed(image, markers, connectivity=connectivity, mask=mask) on the device.
+
+    image: 2-D (H, W) or 3-D (X, Y, Z) CUDA tensor, float32 / float64 (uint8, uint16 and int32 are converted to a float
+    type that holds them exactly).  markers: int32 / int64 of the same shape; every non-zero value is a marker,
+    negative ones too; markers outside the mask are dropped.  mask: None or bool / uint8.  connectivity 1 .. ndim.
+    -> labels with the markers' dtype: 0 outside the mask and where no marker reaches.
+
+    Equal to scikit-image's heap flood wherever no pixel is tie-decided (two neighbours of minimal level with
+    different labels); at ties it follows the deterministic rule of DESIGN.md K11 (markers first, then fewer hops
+    within the level, then the smaller label) instead of scikit-image's age order.  ValueError for NaN inside the
+    mask.  Synchronises twice: the NaN check and the status read."""
+    out, status = _watershed(image, markers, connectivity, mask)
+    st = int(status[0].item())
+    if st:
+        raise HiprError("watershed: phase %d did not converge within its round cap" % st)
+    return out
+
+
+# ---------------------------------------------------------------------------------------------
 # 1-D k-means thresholding
 # ---------------------------------------------------------------------------------------------
 
@@ -1205,8 +1276,8 @@ class Fov:
 
         with hipr_b200.Fov(image_registered) as fov:
             image_final = fov.score("F1")
-            ...                                  # watershed on the host
-            labels, area, avgint, avgint_norm = fov.cell_spectra(image_seg)
+            ...                                  # k-means mask, label, watershed, clear_border on the device
+            labels, area, avgint, avgint_norm = fov.cell_spectra(image_seg)   # image_seg: a CUDA tensor
     """
 
     def __init__(self, cube):
@@ -1216,6 +1287,8 @@ class Fov:
         if cube.ndim != 3:
             raise ValueError("cube must be (H, W, C)")
         self.shape = cube.shape
+        # hipr_fov_upload uses the current device (needed only to check device labels against it)
+        self._device = torch.cuda.current_device() if torch.cuda.is_available() else None
         h = C.c_void_p()
         check(lib().hipr_fov_upload(cube.ctypes.data_as(C.c_void_p), cube.shape[0], cube.shape[1], cube.shape[2],
                                     C.byref(h)), "fov_upload")
@@ -1237,6 +1310,11 @@ class Fov:
         return (score, s) if return_sum else score
 
     def cell_spectra(self, labels):
+        """-> (labels, area, avgint, avgint_norm) numpy arrays, rows in ascending label order.  labels: the (H, W)
+        int32 / int64 label image, as a numpy array (uploaded) or as a CUDA tensor on the handle's device (read in
+        place, stream-ordered on torch's current stream: a label image from `watershed` never leaves the device)."""
+        if isinstance(labels, torch.Tensor):
+            return self._cell_spectra_device(labels)
         labels = np.ascontiguousarray(labels)
         if labels.dtype not in (np.int32, np.int64):
             raise TypeError("labels must be int32 or int64, got %s" % labels.dtype)
@@ -1257,6 +1335,30 @@ class Fov:
             check(code, "fov_cell_spectra")
             k = int(n.value)
             return lab[:k], area[:k], avg[:k], norm[:k]
+
+    def _cell_spectra_device(self, labels):
+        labels = _dev(labels, "labels", (torch.int32, torch.int64))
+        H, W, Cn = self.shape
+        if tuple(labels.shape) != (H, W):
+            raise ValueError("labels must be (%d, %d)" % (H, W))
+        if labels.device.index != self._device:
+            raise ValueError("labels live on cuda:%d, this field of view on cuda:%d" % (labels.device.index,
+                                                                                       self._device))
+        cube = C.c_void_p(self.device_arrays()[0])
+        max_label = int(label_max(labels).item())
+        if max_label <= 0:
+            return (np.empty(0, np.int64), np.empty(0, np.int64), np.empty((0, Cn), np.float64),
+                    np.empty((0, Cn), np.float64))
+        sums = torch.empty((max_label + 1, Cn), dtype=torch.float64, device=labels.device)
+        counts = torch.empty(max_label + 1, dtype=torch.int32, device=labels.device)
+        with torch.cuda.device(labels.device):
+            check(lib().hipr_cell_spectra_reset(C.c_void_p(sums.data_ptr()), C.c_void_p(counts.data_ptr()), max_label,
+                                                Cn, _stream()), "cell_spectra_reset")
+            check(lib().hipr_cell_spectra_accumulate(cube, C.c_void_p(labels.data_ptr()), labels.element_size(),
+                                                     H * W, W, Cn, max_label, C.c_void_p(sums.data_ptr()),
+                                                     C.c_void_p(counts.data_ptr()), None, _stream()),
+                  "cell_spectra_accumulate")
+        return tuple(t.cpu().numpy() for t in cell_spectra_finalize(sums, counts))
 
     def device_arrays(self):
         """(cube, channel sums, range keys) device pointers as ints, for callers that continue on the device."""

@@ -378,6 +378,38 @@ int hipr_label_counts(const void *labels_dev, int label_bytes, int ndim, int d0,
 int hipr_label_clear(const void *image_dev, int dtype, const int32_t *labels_dev, int64_t npix,
                      const int32_t *flagged_dev, int64_t fill, void *out_dev, void *stream);
 
+/* ---- marker watershed (csrc/watershed.cu) -----------------------------------------------------------------------
+ * skimage.segmentation.watershed(image, markers, connectivity=connectivity, mask=mask) (no compactness, no watershed
+ * line), the last step of the segmentation back end: syn/..._measurement.py:125-158, eco/..._measurement.py:44-127,
+ * bio/..._analysis.py:367-419, 463-501.  scikit-image floods from a heap keyed by (value, age); where two neighbours of
+ * a pixel tie for the lowest level with different labels ("tie-decided" pixels: plateaus, quantised data, markers of
+ * equal value) its answer depends on the age order.  This entry point computes a fully specified rule instead, which
+ * equals the heap wherever no pixel is tie-decided (DESIGN.md K11): every flooded pixel gets the key (L, d, l) --
+ * level (minimax path value from the markers, -0.0 equal to +0.0), hop count within the level group, label (signed)
+ * -- a marker (v, 0, its label), any other in-mask pixel f(min over its in-mask neighbours of their keys), with
+ * f((L, d, l), p) = (L, d + 1, l) if v(p) <= L, else (v(p), 1, l); its label is l.  At ties it prefers markers, then
+ * fewer hops, then the smaller label.  Parity unpinned (scikit-image is not pinned by the reference).
+ *   image_dev    C-order (d0, d1) (ndim 2) or (d0, d1, d2) (ndim 3) of image_dtype HIPR_F32 / HIPR_F64; no NaN inside
+ *                the mask (the result is unspecified there)
+ *   markers_dev  same shape, int32 (label_bytes 4) or int64 (8): any non-zero value is a marker; markers outside the
+ *                mask are dropped (scikit-image's markers * mask)
+ *   mask_dev     NULL (every pixel) or uint8, non-zero = inside
+ *   connectivity 1 .. ndim, the offsets of hipr_label
+ *   labels_out   same shape and dtype as the markers: the label of every flooded pixel; 0 outside the mask and
+ *                where no marker reaches
+ *   status_dev   8 int64, written by the call: [0] status (0 ok; k = 1, 2, 3: phase k still changed after its cap of
+ *                npix + 1 rounds, which the algorithm never reaches -- treat as an internal error), [1..3] rounds of
+ *                the three phases, [4..6] tile visits of the three phases, [7] CTAs of the launch
+ *   workspace    hipr_watershed_workspace_bytes(...) bytes (negative: HIPR_E_RANGE when the image has 2^31 pixels or
+ *                more); what it holds before the call does not matter
+ * One memset and one cooperative launch whatever the image holds (HIPR_E_UNSUPPORTED without cooperative launch);
+ * no host synchronisation.
+ */
+int64_t hipr_watershed_workspace_bytes(int ndim, int d0, int d1, int d2, int image_dtype, int label_bytes);
+int hipr_watershed(const void *image_dev, int image_dtype, const void *markers_dev, int label_bytes,
+                   const uint8_t *mask_dev, int ndim, int d0, int d1, int d2, int connectivity, void *workspace_dev,
+                   int64_t workspace_bytes, void *labels_out, int64_t *status_dev, void *stream);
+
 /* ---- 1-D k-means thresholding ---------------------------------------------------------------------------
  * Replaces KMeans(n_clusters = k, random_state = seed).fit_predict(image.reshape(-1, 1)) on the score map, the
  * denoised sum image or their logarithms, and the mask orientation that follows it:
