@@ -1,7 +1,9 @@
 // ABI housekeeping and the host-buffer entry points: what a numpy caller binds.  The cube is
 // streamed host -> device in row bands on a copy stream while the channel sum (or the per-cell
 // accumulation) of the previous band runs on a compute stream, so the end-to-end time is the
-// PCIe time of the cube plus a short tail.
+// PCIe time of the cube plus a short tail.  Every entry point on the per-device workspace opens a
+// CallScope; cubes go up through upload_bands, large results come down through banded_to_host,
+// and the 2-D score tail is score2d.
 #include <mutex>
 #include <string.h>
 #include <cstdlib>
@@ -33,57 +35,84 @@ int gather_launch(const T *src, int64_t stride_a, int64_t stride_b, int inner, i
                   const int *offs, T *out, cudaStream_t st);
 int check_table(const int32_t *table, int n_dirs, int P, int ndim);
 
+// A grow-only device (or page-locked host) buffer.  The recorded size is 0 until a new allocation has succeeded, so a
+// failed reserve is retried by the next call.
+template <bool HOST>
+struct Buf {
+    void *p = nullptr;
+    size_t bytes = 0;
+    int reserve(size_t n) {
+        if (n <= bytes) return HIPR_OK;
+        release();
+        HIPR_CUDA(HOST ? cudaHostAlloc(&p, n, cudaHostAllocDefault) : cudaMalloc(&p, n));
+        bytes = n;
+        return HIPR_OK;
+    }
+    void release() {
+        if (p) HOST ? cudaFreeHost(p) : cudaFree(p);
+        p = nullptr;
+        bytes = 0;
+    }
+};
+using DevBuf = Buf<false>;
+using HostBuf = Buf<true>;
+
+// An error return after the first enqueue must not leave copies from the caller's buffers (or into them) in flight:
+// the caller may free them.  Unless disarmed, the guard synchronises its streams on scope exit.
+struct Drain {
+    cudaStream_t s[3] = {};
+    bool armed = true;
+    ~Drain() {
+        if (!armed) return;
+        for (cudaStream_t st : s)
+            if (st) cudaStreamSynchronize(st);
+    }
+};
+
 constexpr int NBUF = 3;
 struct Workspace {
     std::mutex mu;
     cudaStream_t copy = nullptr, comp = nullptr;
-    cudaEvent_t copied[NBUF] = {}, freed[NBUF] = {}, done = nullptr;
+    cudaEvent_t copied[NBUF] = {}, freed[NBUF] = {};
+    cudaEvent_t staged_out[NBUF] = {};   // the copy out of stage[i] has completed
     cudaEvent_t t0 = nullptr, t1 = nullptr;   // device-side timing of the last host call
     float last_ms = -1.f;
-    void *band[NBUF] = {};
-    size_t band_bytes = 0;
-    void *aux[6] = {};
-    size_t aux_bytes[6] = {};
+    DevBuf band[NBUF];
     // pageable callers: page-locked staging ring the caller's array is copied through by a few host threads
-    void *stage[NBUF] = {};
-    size_t stage_bytes = 0;
-    cudaEvent_t staged_out[NBUF] = {};   // the H2D copy out of stage[i] has completed
+    HostBuf stage[NBUF];
     // batch entry point (hipr_neighbor2d_host_batch): a third stream for denoise + stencil + score read-back of FOV i
-    // while FOV i + 1 is uploaded and summed, and two sets of per-FOV buffers
+    // while FOV i + 1 is uploaded and summed, and two sets of per-image buffers (the other entry points use img[0])
     cudaStream_t post = nullptr;
     cudaEvent_t summed[2] = {}, post_done[2] = {};
-    void *baux[2][4] = {};
-    size_t baux_bytes[2][4] = {};
-    // the cell table of the last hipr_cell_spectra_host call stays in aux[5] for hipr_cell_spectra_host_fetch
+    struct Image {
+        DevBuf sum;       // float64 channel sums
+        DevBuf score;     // float32 score, then the float32 normalised sum
+        DevBuf keys;      // range keys (64 bytes)
+        DevBuf scratch;   // float64: the denoised image, then the float64 score
+    } img[2];
+    DevBuf input;         // an input uploaded whole: the padded gather input, a label image
+    DevBuf extra;         // the 3-D denoise's padded copy
+    // the cell table of the last hipr_cell_spectra_host call stays here for hipr_cell_spectra_host_fetch
+    DevBuf cells;
     int64_t last_cells = -1, last_max_label = 0;
     int last_C = 0;
     bool ready = false;
+
+    void release() {
+        for (int i = 0; i < NBUF; ++i) {
+            band[i].release();
+            stage[i].release();
+        }
+        for (Image &m : img)
+            for (DevBuf *b : {&m.sum, &m.score, &m.keys, &m.scratch}) b->release();
+        for (DevBuf *b : {&input, &extra, &cells}) b->release();
+    }
 };
 // One workspace per device: its streams, events and buffers belong to the device that was current when they were
 // created, so a process that drives several GPUs (or switches devices between calls) never shares them.
 constexpr int kMaxDevices = 32;
 static Workspace g_ws_dev[kMaxDevices];
-static Workspace *ws_current() {
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= kMaxDevices) return nullptr;
-    return &g_ws_dev[dev];
-}
 static thread_local float t_last_ms = -1.f;      // hipr_host_last_elapsed_ms: the calling thread's last host call
-
-// An error return after the first enqueue must not leave copies from the caller's buffers (or into them) in flight:
-// the caller may free them.  Unless dismissed, the guard drains both streams on scope exit.
-struct DrainOnError {
-    Workspace &w;
-    bool armed = true;
-    explicit DrainOnError(Workspace &ws) : w(ws) {}
-    void dismiss() { armed = false; }
-    ~DrainOnError() {
-        if (!armed) return;
-        if (w.copy) cudaStreamSynchronize(w.copy);
-        if (w.comp) cudaStreamSynchronize(w.comp);
-        if (w.post) cudaStreamSynchronize(w.post);
-    }
-};
 
 // host threads that copy a pageable array into the page-locked staging ring (HIPR_HOST_COPY_THREADS overrides)
 static int host_copy_threads() {
@@ -106,8 +135,8 @@ static int ws_init(Workspace &w) {
     for (int i = 0; i < NBUF; ++i) {
         HIPR_CUDA(cudaEventCreateWithFlags(&w.copied[i], cudaEventDisableTiming));
         HIPR_CUDA(cudaEventCreateWithFlags(&w.freed[i], cudaEventDisableTiming));
+        HIPR_CUDA(cudaEventCreateWithFlags(&w.staged_out[i], cudaEventDisableTiming));
     }
-    HIPR_CUDA(cudaEventCreateWithFlags(&w.done, cudaEventDisableTiming));
     HIPR_CUDA(cudaStreamCreateWithFlags(&w.post, cudaStreamNonBlocking));
     for (int i = 0; i < 2; ++i) {
         HIPR_CUDA(cudaEventCreateWithFlags(&w.summed[i], cudaEventDisableTiming));
@@ -118,27 +147,49 @@ static int ws_init(Workspace &w) {
     w.ready = true;
     return HIPR_OK;
 }
-static int ws_bands(Workspace &w, size_t bytes) {
-    if (bytes <= w.band_bytes) return HIPR_OK;
-    for (int i = 0; i < NBUF; ++i) {
-        if (w.band[i]) cudaFree(w.band[i]);
-        w.band[i] = nullptr;
+
+// One entry point's use of the current device's workspace: open() finds it, takes its lock, creates its streams and
+// events on first use and arms the drain over its three streams.  finish(last) ends a timed call: t1 on `last`, every
+// stream synchronised, the device time from t0 stored for hipr_host_last_elapsed_ms.  done() ends an untimed one.
+struct CallScope {
+    Workspace *w = nullptr;
+    std::unique_lock<std::mutex> lock;
+    Drain drain{{}, false};          // armed by open(); declared after the lock, so it drains before the unlock
+    int open() {
+        int dev = 0;
+        if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= kMaxDevices) return HIPR_E_NODEVICE;
+        w = &g_ws_dev[dev];
+        lock = std::unique_lock<std::mutex>(w->mu);
+        int e = ws_init(*w);
+        if (e) return e;
+        drain.s[0] = w->copy;
+        drain.s[1] = w->comp;
+        drain.s[2] = w->post;
+        drain.armed = true;
+        return HIPR_OK;
     }
-    w.band_bytes = 0;
-    for (int i = 0; i < NBUF; ++i) HIPR_CUDA(cudaMalloc(&w.band[i], bytes));
-    w.band_bytes = bytes;
-    return HIPR_OK;
-}
-static int ws_stage(Workspace &w, size_t bytes) {
-    if (bytes <= w.stage_bytes) return HIPR_OK;
-    for (int i = 0; i < NBUF; ++i) {
-        if (w.stage[i]) cudaFreeHost(w.stage[i]);
-        w.stage[i] = nullptr;
-        if (!w.staged_out[i]) HIPR_CUDA(cudaEventCreateWithFlags(&w.staged_out[i], cudaEventDisableTiming));
+    int done() {
+        for (cudaStream_t st : drain.s) HIPR_CUDA(cudaStreamSynchronize(st));
+        drain.armed = false;
+        return HIPR_OK;
     }
-    w.stage_bytes = 0;
-    for (int i = 0; i < NBUF; ++i) HIPR_CUDA(cudaHostAlloc(&w.stage[i], bytes, cudaHostAllocDefault));
-    w.stage_bytes = bytes;
+    int finish(cudaStream_t last) {
+        HIPR_CUDA(cudaEventRecord(w->t1, last));
+        int e = done();
+        if (e) return e;
+        HIPR_CUDA(cudaEventElapsedTime(&w->last_ms, w->t0, w->t1));
+        t_last_ms = w->last_ms;
+        return HIPR_OK;
+    }
+};
+
+// band ring (and, for a pageable source or destination, the staging ring) of `bytes` per band
+static int ws_ring(Workspace &w, size_t bytes, bool staged) {
+    int e;
+    for (int i = 0; i < NBUF; ++i) {
+        if ((e = w.band[i].reserve(bytes))) return e;
+        if (staged && (e = w.stage[i].reserve(bytes))) return e;
+    }
     return HIPR_OK;
 }
 
@@ -171,32 +222,130 @@ static void parallel_copy(void *dst, const void *src, size_t bytes, int nthreads
     for (auto &t : th) t.join();
 }
 
-static int ws_aux(Workspace &w, int slot, size_t bytes) {
-    if (bytes <= w.aux_bytes[slot]) return HIPR_OK;
-    if (w.aux[slot]) cudaFree(w.aux[slot]);
-    w.aux[slot] = nullptr;
-    w.aux_bytes[slot] = 0;
-    HIPR_CUDA(cudaMalloc(&w.aux[slot], bytes));
-    w.aux_bytes[slot] = bytes;
-    return HIPR_OK;
-}
-
-static int ws_baux(Workspace &w, int set, int slot, size_t bytes) {
-    if (bytes <= w.baux_bytes[set][slot]) return HIPR_OK;
-    if (w.baux[set][slot]) cudaFree(w.baux[set][slot]);
-    w.baux[set][slot] = nullptr;
-    w.baux_bytes[set][slot] = 0;
-    HIPR_CUDA(cudaMalloc(&w.baux[set][slot], bytes));
-    w.baux_bytes[set][slot] = bytes;
-    return HIPR_OK;
-}
-
 // rows per band so that a band is ~32 MiB and a whole number of rows
 static int band_rows(int64_t row_bytes, int64_t nrows) {
     int64_t r = (32ll << 20) / (row_bytes > 0 ? row_bytes : 1);
     if (r < 1) r = 1;
     if (r > nrows) r = nrows;
     return (int)r;
+}
+
+// Host -> device in bands: `units` units of `unit_bytes` from src, `units_per_band` per band, through the band ring on
+// the copy stream, while `consume(u0, nu, band_dev, comp)` reads the previous band on the compute stream.  A pageable
+// src goes through the staging ring: host threads copy band b into it while band b - 1 crosses PCIe and band b - 2
+// is consumed.  `band` counts the bands since the start of the call, so the ring slots carry over from one upload to
+// the next.  The caller reserves the rings (ws_ring) for units_per_band units.
+template <typename Consume>
+static int upload_bands(Workspace &w, const void *src, int64_t units, int64_t unit_bytes, int64_t units_per_band,
+                        int &band, Consume consume) {
+    int e;
+    const bool pageable = is_pageable(src);
+    const int copy_threads = host_copy_threads();
+    for (int64_t u0 = 0; u0 < units; u0 += units_per_band, ++band) {
+        const int64_t nu = (units - u0 < units_per_band) ? units - u0 : units_per_band;
+        const size_t bytes = (size_t)(nu * unit_bytes);
+        const int slot = band % NBUF;
+        const void *from = (const char *)src + u0 * unit_bytes;
+        if (pageable) {
+            if (band >= NBUF) HIPR_CUDA(cudaEventSynchronize(w.staged_out[slot]));
+            parallel_copy(w.stage[slot].p, from, bytes, copy_threads);
+            from = w.stage[slot].p;
+        }
+        if (band >= NBUF) HIPR_CUDA(cudaStreamWaitEvent(w.copy, w.freed[slot], 0));
+        HIPR_CUDA(cudaMemcpyAsync(w.band[slot].p, from, bytes, cudaMemcpyHostToDevice, w.copy));
+        if (pageable) HIPR_CUDA(cudaEventRecord(w.staged_out[slot], w.copy));
+        HIPR_CUDA(cudaEventRecord(w.copied[slot], w.copy));
+        HIPR_CUDA(cudaStreamWaitEvent(w.comp, w.copied[slot], 0));
+        if ((e = consume(u0, nu, (const void *)w.band[slot].p, w.comp))) return e;
+        HIPR_CUDA(cudaEventRecord(w.freed[slot], w.comp));
+    }
+    return HIPR_OK;
+}
+
+// range keys before the first channel sum: max 0, min all ones
+static int reset_keys(unsigned long long *keys, cudaStream_t st) {
+    HIPR_CUDA(cudaMemsetAsync(keys, 0x00, 8, st));
+    HIPR_CUDA(cudaMemsetAsync(keys + 1, 0xff, 8, st));
+    return HIPR_OK;
+}
+
+// The 2-D score of an (H, W) float64 channel-sum image with its range keys, into the float32 `score` on `st`.
+// denoise_h > 0: syn/..._measurement.py:106-124 in full, /max (in place) -> NL-means -> float64 stencil (the denoised
+// image is too smooth for the fixed-point grid, DESIGN.md).  Otherwise the fixed-point stencil for the (11, 9) table
+// every pipeline uses (F1 / F2: every tile quantised with its own range, the finest grid and the same as the
+// device-resident pipeline, bit for bit; F3's epsilon needs the global range), and the float64 stencil for other
+// parameters.  The float64 routes reserve `scratch` for 2 H W doubles: the denoised image, then the float64 score.
+static int score2d(double *sum, const unsigned long long *keys, int H, int W, int patch_size, int n_dirs,
+                   const int32_t *table, int flavour, double denoise_h, DevBuf &scratch, float *score, cudaStream_t st) {
+    const int64_t npix = (int64_t)H * W;
+    const uint64_t *range = (const uint64_t *)keys;
+    int e;
+    if (denoise_h <= 0.0) {
+        const bool tile_local = (flavour == HIPR_FLAVOUR_F1 || flavour == HIPR_FLAVOUR_F2);
+        e = hipr_lne2d_q(sum, H, W, W, 0, HIPR_F64, patch_size, n_dirs, table, flavour, tile_local ? nullptr : range,
+                         score, st);
+        if (e != HIPR_E_TABLE || (patch_size == 11 && n_dirs == 9)) return e;
+    }
+    if ((e = scratch.reserve((size_t)npix * 2 * sizeof(double)))) return e;
+    double *den = (double *)scratch.p, *score64 = den + npix;
+    const double *src = sum;
+    if (denoise_h > 0.0) {
+        if ((e = hipr_normalize(sum, HIPR_F64, npix, range, st))) return e;
+        if ((e = hipr_denoise_nl_means_2d(sum, H, W, HIPR_F64, 7, 11, denoise_h, den, st))) return e;
+        src = den;
+        range = nullptr;
+    }
+    if ((e = hipr_lne2d(src, H, W, W, 0, HIPR_F64, patch_size, n_dirs, table, flavour, range, score64, st))) return e;
+    return hipr_normalize_cast(score64, npix, nullptr, score, st);
+}
+
+// Per-cell table in one device buffer: the accumulators (sums (max_label + 1, C) float64, counts int32 padded to 16
+// bytes, 16 bytes more; zeroed before the pass), then the finalized table: n (16 bytes), labels and areas (max_label)
+// int64, avgint and avgint_norm (max_label, C) float64 -- the first n rows are valid.
+struct CellTable {
+    double *sums;
+    int32_t *counts, *n;
+    int64_t *labels, *area;
+    double *avg, *norm;
+    size_t acc_bytes;
+};
+static int cell_table(DevBuf &buf, int64_t max_label, int C, CellTable &t) {
+    const size_t row_bytes = (size_t)C * 8, sums_bytes = (size_t)(max_label + 1) * row_bytes;
+    const size_t cnt_bytes = ((size_t)(max_label + 1) * 4 + 15) & ~(size_t)15;
+    t.acc_bytes = sums_bytes + cnt_bytes + 16;
+    int e = buf.reserve(t.acc_bytes + 16 + (size_t)max_label * (16 + 2 * row_bytes));
+    if (e) return e;
+    char *base = (char *)buf.p, *fin = base + t.acc_bytes;
+    t.sums = (double *)base;
+    t.counts = (int32_t *)(base + sums_bytes);
+    t.n = (int32_t *)fin;
+    t.labels = (int64_t *)(fin + 16);
+    t.area = t.labels + max_label;
+    t.avg = (double *)(t.area + max_label);
+    t.norm = t.avg + (size_t)max_label * C;
+    return HIPR_OK;
+}
+static int copy_cell_table(const CellTable &t, int64_t n, int C, int64_t *labels_out, int64_t *area_out,
+                           double *avgint_out, double *avgint_norm_out, cudaStream_t st) {
+    HIPR_CUDA(cudaMemcpyAsync(labels_out, t.labels, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
+    HIPR_CUDA(cudaMemcpyAsync(area_out, t.area, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
+    HIPR_CUDA(cudaMemcpyAsync(avgint_out, t.avg, (size_t)n * C * 8, cudaMemcpyDeviceToHost, st));
+    HIPR_CUDA(cudaMemcpyAsync(avgint_norm_out, t.norm, (size_t)n * C * 8, cudaMemcpyDeviceToHost, st));
+    return HIPR_OK;
+}
+// finalize the accumulated table, read n back (*n_cells), and enqueue the copy of the table when it fits the caller's
+// capacity; HIPR_E_RANGE when it does not (everything enqueued has then completed)
+static int finalize_cells(const CellTable &t, int64_t max_label, int C, int64_t capacity, int64_t *n_cells,
+                          int64_t *labels_out, int64_t *area_out, double *avgint_out, double *avgint_norm_out,
+                          cudaStream_t st) {
+    int e = hipr_cell_spectra_finalize(t.sums, t.counts, max_label, C, t.n, t.labels, t.area, t.avg, t.norm, st);
+    if (e) return e;
+    int32_t n = 0;
+    HIPR_CUDA(cudaMemcpyAsync(&n, t.n, 4, cudaMemcpyDeviceToHost, st));
+    HIPR_CUDA(cudaStreamSynchronize(st));
+    *n_cells = n;
+    if (n > capacity) return HIPR_E_RANGE;
+    return n ? copy_cell_table(t, n, C, labels_out, area_out, avgint_out, avgint_norm_out, st) : HIPR_OK;
 }
 
 }  // namespace hipr
@@ -245,33 +394,12 @@ extern "C" int hipr_host_free(void *ptr) {
 static void fov_cache_release_current_device();
 extern "C" int hipr_host_release_workspace(void) {
     fov_cache_release_current_device();
-    Workspace *wp = ws_current();
-    if (!wp) return HIPR_E_NODEVICE;
-    Workspace &w = *wp;
-    std::lock_guard<std::mutex> lock(w.mu);
+    CallScope call;
+    int e = call.open();
+    if (e) return e;
     cudaDeviceSynchronize();
-    for (int i = 0; i < NBUF; ++i) {
-        if (w.band[i]) cudaFree(w.band[i]);
-        w.band[i] = nullptr;
-    }
-    w.band_bytes = 0;
-    for (int i = 0; i < NBUF; ++i) {
-        if (w.stage[i]) cudaFreeHost(w.stage[i]);
-        w.stage[i] = nullptr;
-    }
-    w.stage_bytes = 0;
-    for (int i = 0; i < 6; ++i) {
-        if (w.aux[i]) cudaFree(w.aux[i]);
-        w.aux[i] = nullptr;
-        w.aux_bytes[i] = 0;
-    }
-    for (int k = 0; k < 2; ++k)
-        for (int i = 0; i < 4; ++i) {
-            if (w.baux[k][i]) cudaFree(w.baux[k][i]);
-            w.baux[k][i] = nullptr;
-            w.baux_bytes[k][i] = 0;
-        }
-    return HIPR_OK;
+    call.w->release();
+    return call.done();
 }
 
 // cube_host: (H, W, C) samples of `sample_bytes` (4 = float32; 2 / 1 = raw uint16 / uint8 counts, value =
@@ -280,101 +408,40 @@ static int neighbor2d_host_impl(const void *cube_host, int sample_bytes, float s
                                 int patch_size, int n_dirs, const int32_t *table_host, int flavour, float *score_host,
                                 float *sum_host, double denoise_h = 0.0) {
     if (!cube_host || !score_host || H < 1 || W < 1 || C < 1) return HIPR_E_ARG;
-    Workspace *wp = ws_current();
-    if (!wp) return HIPR_E_NODEVICE;
-    Workspace &w = *wp;
-    std::lock_guard<std::mutex> lock(w.mu);
-    int e = ws_init(w);
+    CallScope call;
+    int e = call.open();
     if (e) return e;
-    DrainOnError guard(w);
+    Workspace &w = *call.w;
+    Workspace::Image &m = w.img[0];
     const int64_t row_bytes = (int64_t)W * C * sample_bytes;
     const int rows = band_rows(row_bytes, H);
-    if ((e = ws_bands(w, (size_t)rows * row_bytes))) return e;
     const size_t img_bytes = (size_t)H * W * 4;
-    if ((e = ws_aux(w, 0, 4 * img_bytes))) return e;  // float64 sum image (+ float64 score, general parameters)
-    if ((e = ws_aux(w, 1, img_bytes))) return e;      // score, then the float32 normalised sum
-    if ((e = ws_aux(w, 2, 64))) return e;             // max / min keys
-    double *sum_dev = (double *)w.aux[0];
-    float *score_dev = (float *)w.aux[1];
-    unsigned long long *key = (unsigned long long *)w.aux[2];
+    if ((e = ws_ring(w, (size_t)rows * row_bytes, is_pageable(cube_host))) || (e = m.sum.reserve(2 * img_bytes)) ||
+        (e = m.score.reserve(img_bytes)) || (e = m.keys.reserve(64)))
+        return e;
+    double *sum_dev = (double *)m.sum.p;
+    float *score_dev = (float *)m.score.p;
+    unsigned long long *key = (unsigned long long *)m.keys.p;
     HIPR_CUDA(cudaEventRecord(w.t0, w.copy));            // device clock starts before the first H2D
     HIPR_CUDA(cudaStreamWaitEvent(w.comp, w.t0, 0));
-    HIPR_CUDA(cudaMemsetAsync(key, 0x00, 8, w.comp));
-    HIPR_CUDA(cudaMemsetAsync(key + 1, 0xff, 8, w.comp));
-    const bool pageable = is_pageable(cube_host);
-    const int copy_threads = host_copy_threads();
-    if (pageable && (e = ws_stage(w, (size_t)rows * row_bytes))) return e;
+    if ((e = reset_keys(key, w.comp))) return e;
     int b = 0;
-    for (int r0 = 0; r0 < H; r0 += rows, ++b) {
-        const int nr = (H - r0 < rows) ? H - r0 : rows;
-        const int slot = b % NBUF;
-        const void *src = (const char *)cube_host + (int64_t)r0 * row_bytes;
-        if (pageable) {
-            // host threads copy band b into the page-locked ring while band b - 1 crosses PCIe and band b - 2 is summed
-            if (b >= NBUF) HIPR_CUDA(cudaEventSynchronize(w.staged_out[slot]));
-            parallel_copy(w.stage[slot], src, (size_t)nr * row_bytes, copy_threads);
-            src = w.stage[slot];
-        }
-        if (b >= NBUF) HIPR_CUDA(cudaStreamWaitEvent(w.copy, w.freed[slot], 0));
-        HIPR_CUDA(cudaMemcpyAsync(w.band[slot], src, (size_t)nr * row_bytes, cudaMemcpyHostToDevice, w.copy));
-        if (pageable) HIPR_CUDA(cudaEventRecord(w.staged_out[slot], w.copy));
-        HIPR_CUDA(cudaEventRecord(w.copied[slot], w.copy));
-        HIPR_CUDA(cudaStreamWaitEvent(w.comp, w.copied[slot], 0));
-        if ((e = chansum_band(w.band[slot], sample_bytes, scale, (int64_t)nr * W, C, sum_dev + (int64_t)r0 * W, key,
-                              w.comp)))
-            return e;
-        HIPR_CUDA(cudaEventRecord(w.freed[slot], w.comp));
-    }
-    if (denoise_h > 0.0) {
-        // syn/..._measurement.py:106-124 in full: /max -> NL-means -> float64 stencil (the denoised image is too smooth
-        // for the fixed-point grid, DESIGN.md).  aux[0] holds the sums and, behind them, the denoised image; aux[3]
-        // the float64 score.
-        double *den = sum_dev + (size_t)H * W;
-        if ((e = ws_aux(w, 3, 2 * img_bytes))) return e;
-        double *score64 = (double *)w.aux[3];
-        if ((e = hipr_normalize(sum_dev, HIPR_F64, (int64_t)H * W, (const uint64_t *)key, w.comp))) return e;
-        if ((e = hipr_denoise_nl_means_2d(sum_dev, H, W, HIPR_F64, 7, 11, denoise_h, den, w.comp))) return e;
-        if ((e = hipr_lne2d(den, H, W, W, 0, HIPR_F64, patch_size, n_dirs, table_host, flavour, nullptr, score64, w.comp)))
-            return e;
-        if ((e = hipr_normalize_cast(score64, (int64_t)H * W, nullptr, score_dev, w.comp))) return e;
-        HIPR_CUDA(cudaMemcpyAsync(score_host, score_dev, img_bytes, cudaMemcpyDeviceToHost, w.comp));
-        if (sum_host) {
-            if ((e = hipr_normalize_cast(den, (int64_t)H * W, nullptr, score_dev, w.comp))) return e;
-            HIPR_CUDA(cudaMemcpyAsync(sum_host, score_dev, img_bytes, cudaMemcpyDeviceToHost, w.comp));
-        }
-        HIPR_CUDA(cudaEventRecord(w.t1, w.comp));
-        HIPR_CUDA(cudaStreamSynchronize(w.comp));
-        HIPR_CUDA(cudaEventElapsedTime(&w.last_ms, w.t0, w.t1));
-        t_last_ms = w.last_ms;
-        guard.dismiss();
-        return HIPR_OK;
-    }
-    // fixed-point stencil for the (11, 9) table every pipeline uses; float64 kernel otherwise
-    // (F1 / F2: every tile quantised with its own range, the finest grid and the same as the device-resident
-    // pipeline, bit for bit; F3's epsilon needs the global range)
-    const bool tile_local = (flavour == HIPR_FLAVOUR_F1 || flavour == HIPR_FLAVOUR_F2);
-    e = hipr_lne2d_q(sum_dev, H, W, W, 0, HIPR_F64, patch_size, n_dirs, table_host, flavour,
-                     tile_local ? nullptr : (const uint64_t *)key, score_dev, w.comp);
-    if (e == HIPR_E_TABLE && !(patch_size == 11 && n_dirs == 9)) {
-        // general parameters: float64 stencil into the upper half of aux[0], then cast
-        double *score64 = sum_dev + (size_t)H * W;
-        if ((e = hipr_lne2d(sum_dev, H, W, W, 0, HIPR_F64, patch_size, n_dirs, table_host, flavour,
-                            (const uint64_t *)key, score64, w.comp)))
-            return e;
-        e = hipr_normalize_cast(score64, (int64_t)H * W, nullptr, score_dev, w.comp);
-    }
-    if (e) return e;
+    e = upload_bands(w, cube_host, H, row_bytes, rows, b, [&](int64_t r0, int64_t nr, const void *band, cudaStream_t st) {
+        return chansum_band(band, sample_bytes, scale, nr * W, C, sum_dev + r0 * W, key, st);
+    });
+    if (e || (e = score2d(sum_dev, key, H, W, patch_size, n_dirs, table_host, flavour, denoise_h, m.scratch, score_dev,
+                          w.comp)))
+        return e;
     HIPR_CUDA(cudaMemcpyAsync(score_host, score_dev, img_bytes, cudaMemcpyDeviceToHost, w.comp));
     if (sum_host) {
-        if ((e = hipr_normalize_cast(sum_dev, (int64_t)H * W, (const uint64_t *)key, score_dev, w.comp))) return e;
+        // the normalised denoised image, or the sums with the range keys
+        const bool den = denoise_h > 0.0;
+        if ((e = hipr_normalize_cast(den ? (const double *)m.scratch.p : sum_dev, (int64_t)H * W,
+                                     den ? nullptr : (const uint64_t *)key, score_dev, w.comp)))
+            return e;
         HIPR_CUDA(cudaMemcpyAsync(sum_host, score_dev, img_bytes, cudaMemcpyDeviceToHost, w.comp));
     }
-    HIPR_CUDA(cudaEventRecord(w.t1, w.comp));            // ... and stops after the last D2H
-    HIPR_CUDA(cudaStreamSynchronize(w.comp));
-    HIPR_CUDA(cudaEventElapsedTime(&w.last_ms, w.t0, w.t1));
-    t_last_ms = w.last_ms;
-    guard.dismiss();
-    return HIPR_OK;
+    return call.finish(w.comp);                          // ... and stops after the last D2H
 }
 
 extern "C" int hipr_neighbor2d_host(const float *cube_host, int H, int W, int C, int patch_size, int n_dirs,
@@ -391,10 +458,9 @@ template <typename Produce>
 static int banded_to_host(Workspace &w, int64_t nrows, int64_t row_bytes, void *out_host, Produce produce) {
     int e;
     const int rows = band_rows(row_bytes, nrows);
-    if ((e = ws_bands(w, (size_t)rows * row_bytes))) return e;
     const bool pageable = is_pageable(out_host);
     const int copy_threads = host_copy_threads();
-    if (pageable && (e = ws_stage(w, (size_t)rows * row_bytes))) return e;
+    if ((e = ws_ring(w, (size_t)rows * row_bytes, pageable))) return e;
     struct Pending { int slot; int64_t off; size_t bytes; };
     std::vector<Pending> pend;          // pageable: bands whose staged copy still has to reach out_host
     size_t drained = 0;
@@ -402,7 +468,7 @@ static int banded_to_host(Workspace &w, int64_t nrows, int64_t row_bytes, void *
         for (; drained < upto; ++drained) {
             const Pending &q = pend[drained];
             HIPR_CUDA(cudaEventSynchronize(w.staged_out[q.slot]));
-            parallel_copy((char *)out_host + q.off, w.stage[q.slot], q.bytes, copy_threads);
+            parallel_copy((char *)out_host + q.off, w.stage[q.slot].p, q.bytes, copy_threads);
         }
         return HIPR_OK;
     };
@@ -411,28 +477,43 @@ static int banded_to_host(Workspace &w, int64_t nrows, int64_t row_bytes, void *
         const int nr = (int)((nrows - r0 < rows) ? nrows - r0 : rows);
         const int slot = b % NBUF;
         const size_t bytes = (size_t)nr * row_bytes;
+        void *band = w.band[slot].p;
         if (b >= NBUF) HIPR_CUDA(cudaStreamWaitEvent(w.comp, w.freed[slot], 0));   // its previous band has left the device
-        if ((e = produce(r0, nr, w.band[slot], w.comp))) return e;
+        if ((e = produce(r0, nr, band, w.comp))) return e;
         HIPR_CUDA(cudaEventRecord(w.copied[slot], w.comp));
         HIPR_CUDA(cudaStreamWaitEvent(w.copy, w.copied[slot], 0));
         if (pageable) {
             // stage[slot] is free once the host has copied band b - NBUF out of it
             if (b >= NBUF && (e = drain((size_t)(b - NBUF + 1)))) return e;
-            HIPR_CUDA(cudaMemcpyAsync(w.stage[slot], w.band[slot], bytes, cudaMemcpyDeviceToHost, w.copy));
+            HIPR_CUDA(cudaMemcpyAsync(w.stage[slot].p, band, bytes, cudaMemcpyDeviceToHost, w.copy));
             HIPR_CUDA(cudaEventRecord(w.staged_out[slot], w.copy));
             pend.push_back(Pending{slot, r0 * row_bytes, bytes});
         } else {
-            HIPR_CUDA(cudaMemcpyAsync((char *)out_host + r0 * row_bytes, w.band[slot], bytes, cudaMemcpyDeviceToHost, w.copy));
+            HIPR_CUDA(cudaMemcpyAsync((char *)out_host + r0 * row_bytes, band, bytes, cudaMemcpyDeviceToHost, w.copy));
         }
         HIPR_CUDA(cudaEventRecord(w.freed[slot], w.copy));
     }
     if (pageable && (e = drain(pend.size()))) return e;
-    HIPR_CUDA(cudaEventRecord(w.t1, w.copy));
-    HIPR_CUDA(cudaStreamSynchronize(w.copy));
-    HIPR_CUDA(cudaStreamSynchronize(w.comp));
-    HIPR_CUDA(cudaEventElapsedTime(&w.last_ms, w.t0, w.t1));
-    t_last_ms = w.last_ms;
     return HIPR_OK;
+}
+
+// The host gathers: the padded float64 input (`in_count` values) is uploaded once, then banded_to_host runs
+// `produce(in_dev, r0, nr, band_dev, stream)` over `nrows` output rows of `row_bytes`.
+template <typename Produce>
+static int gather_to_host(const double *in_host, size_t in_count, int64_t nrows, int64_t row_bytes, double *out_host,
+                          Produce produce) {
+    CallScope call;
+    int e = call.open();
+    if (e) return e;
+    Workspace &w = *call.w;
+    if ((e = w.input.reserve(in_count * sizeof(double)))) return e;
+    const double *in_dev = (const double *)w.input.p;
+    HIPR_CUDA(cudaEventRecord(w.t0, w.comp));
+    HIPR_CUDA(cudaMemcpyAsync(w.input.p, in_host, in_count * sizeof(double), cudaMemcpyHostToDevice, w.comp));
+    e = banded_to_host(w, nrows, row_bytes, out_host, [&](int64_t r0, int nr, void *band, cudaStream_t st) {
+        return produce(in_dev, r0, nr, band, st);
+    });
+    return e ? e : call.finish(w.copy);
 }
 
 // The strict drop-in of line_profile_2d_v2 (eco/neighbor2d.pyx:8-64) from and to HOST arrays: padded float64 image in,
@@ -451,23 +532,10 @@ extern "C" int hipr_line_profile_2d_host(const double *image_padded_host, int Hp
         if (dy < 0 || dy >= P || dx < 0 || dx >= P) return HIPR_E_TABLE;
         lin[i] = dy * Wp + dx;
     }
-    Workspace *wp = ws_current();
-    if (!wp) return HIPR_E_NODEVICE;
-    Workspace &w = *wp;
-    std::lock_guard<std::mutex> lock(w.mu);
-    if ((e = ws_init(w))) return e;
-    DrainOnError guard(w);
-    if ((e = ws_aux(w, 0, (size_t)Hp * Wp * sizeof(double)))) return e;
-    double *img_dev = (double *)w.aux[0];
-    HIPR_CUDA(cudaEventRecord(w.t0, w.comp));
-    HIPR_CUDA(cudaMemcpyAsync(img_dev, image_padded_host, (size_t)Hp * Wp * sizeof(double), cudaMemcpyHostToDevice, w.comp));
-    e = banded_to_host(w, H, (int64_t)W * K * sizeof(double), out_host,
-                       [&](int64_t r0, int nr, void *band, cudaStream_t st) {
-                           return gather_launch<double>(img_dev + r0 * Wp, Wp, 0, 1, nr, W, K, lin, (double *)band, st);
-                       });
-    if (e) return e;
-    guard.dismiss();
-    return HIPR_OK;
+    return gather_to_host(image_padded_host, (size_t)Hp * Wp, H, (int64_t)W * K * sizeof(double), out_host,
+                          [&](const double *img_dev, int64_t r0, int nr, void *band, cudaStream_t st) {
+                              return gather_launch<double>(img_dev + r0 * Wp, Wp, 0, 1, nr, W, K, lin, (double *)band, st);
+                          });
 }
 
 // line_profile_v2 (bio/neighbor.pyx:115-181) from and to host arrays: (X, Y, Z, n_dirs, P) float64, 6,336 B per voxel at
@@ -478,26 +546,11 @@ extern "C" int hipr_line_profile_3d_host(const double *volume_padded_host, int X
     if (!volume_padded_host || !out_host || patch_size < 1) return HIPR_E_ARG;
     const int P = patch_size, X = Xp - (P - 1), Y = Yp - (P - 1), Z = Zp - (P - 1);
     if (X < 1 || Y < 1 || Z < 1) return HIPR_E_PATCH;
-    Workspace *wp = ws_current();
-    if (!wp) return HIPR_E_NODEVICE;
-    Workspace &w = *wp;
-    std::lock_guard<std::mutex> lock(w.mu);
-    int e = ws_init(w);
-    if (e) return e;
-    DrainOnError guard(w);
-    const size_t vol_bytes = (size_t)Xp * Yp * Zp * sizeof(double);
-    if ((e = ws_aux(w, 0, vol_bytes))) return e;
-    double *vol_dev = (double *)w.aux[0];
-    HIPR_CUDA(cudaEventRecord(w.t0, w.comp));
-    HIPR_CUDA(cudaMemcpyAsync(vol_dev, volume_padded_host, vol_bytes, cudaMemcpyHostToDevice, w.comp));
-    e = banded_to_host(w, X, (int64_t)Y * Z * n_dirs * P * sizeof(double), out_host,
-                       [&](int64_t x0, int nx, void *band, cudaStream_t st) {
-                           return hipr_line_profile_3d(vol_dev + x0 * (int64_t)Yp * Zp, nx + P - 1, Yp, Zp, HIPR_F64, P, n_dirs,
-                                                       table_host, band, st);
-                       });
-    if (e) return e;
-    guard.dismiss();
-    return HIPR_OK;
+    return gather_to_host(volume_padded_host, (size_t)Xp * Yp * Zp, X, (int64_t)Y * Z * n_dirs * P * sizeof(double),
+                          out_host, [&](const double *vol_dev, int64_t x0, int nx, void *band, cudaStream_t st) {
+                              return hipr_line_profile_3d(vol_dev + x0 * (int64_t)Yp * Zp, nx + P - 1, Yp, Zp, HIPR_F64, P,
+                                                          n_dirs, table_host, band, st);
+                          });
 }
 
 // The same for line_profile_memory_efficient_v2 (bio/neighbor.pyx:186-263), the 3-D stencil the z-stack pipelines
@@ -508,27 +561,12 @@ extern "C" int hipr_lne3d_dirs_host(const double *volume_padded_host, int Xp, in
     if (!volume_padded_host || !out_host || patch_size < 1) return HIPR_E_ARG;
     const int P = patch_size, X = Xp - (P - 1), Y = Yp - (P - 1), Z = Zp - (P - 1);
     if (X < 1 || Y < 1 || Z < 1) return HIPR_E_PATCH;
-    Workspace *wp = ws_current();
-    if (!wp) return HIPR_E_NODEVICE;
-    Workspace &w = *wp;
-    std::lock_guard<std::mutex> lock(w.mu);
-    int e = ws_init(w);
-    if (e) return e;
-    DrainOnError guard(w);
-    const size_t vol_bytes = (size_t)Xp * Yp * Zp * sizeof(double);
-    if ((e = ws_aux(w, 0, vol_bytes))) return e;
-    double *vol_dev = (double *)w.aux[0];
-    HIPR_CUDA(cudaEventRecord(w.t0, w.comp));
-    HIPR_CUDA(cudaMemcpyAsync(vol_dev, volume_padded_host, vol_bytes, cudaMemcpyHostToDevice, w.comp));
-    e = banded_to_host(w, X, (int64_t)Y * Z * n_dirs * sizeof(double), out_host,
-                       [&](int64_t x0, int nx, void *band, cudaStream_t st) {
-                           // output planes [x0, x0 + nx) read padded planes [x0, x0 + nx + P - 1)
-                           return hipr_lne3d_dirs(vol_dev + x0 * (int64_t)Yp * Zp, nx + P - 1, Yp, Zp, 1, HIPR_F64, P, n_dirs,
-                                                  table_host, nullptr, band, st);
-                       });
-    if (e) return e;
-    guard.dismiss();
-    return HIPR_OK;
+    return gather_to_host(volume_padded_host, (size_t)Xp * Yp * Zp, X, (int64_t)Y * Z * n_dirs * sizeof(double), out_host,
+                          [&](const double *vol_dev, int64_t x0, int nx, void *band, cudaStream_t st) {
+                              // output planes [x0, x0 + nx) read padded planes [x0, x0 + nx + P - 1)
+                              return hipr_lne3d_dirs(vol_dev + x0 * (int64_t)Yp * Zp, nx + P - 1, Yp, Zp, 1, HIPR_F64, P,
+                                                     n_dirs, table_host, nullptr, band, st);
+                          });
 }
 
 // 3-D: cube_host (X, Y, Z, C) float32 -> score_host (X, Y, Z) float32: channel sum -> /max -> edge pad -> 72 x 11 line
@@ -538,89 +576,56 @@ static int neighbor3d_host_impl(const float *cube_host, int X, int Y, int Z, int
                                 const int32_t *table_host, int flavour, float *score_host, double denoise_h,
                                 int denoise_distance) {
     if (!cube_host || !score_host || !table_host || X < 1 || Y < 1 || Z < 1 || C < 1) return HIPR_E_ARG;
-    Workspace *wp = ws_current();
-    if (!wp) return HIPR_E_NODEVICE;
-    Workspace &w = *wp;
-    std::lock_guard<std::mutex> lock(w.mu);
-    int e = ws_init(w);
+    CallScope call;
+    int e = call.open();
     if (e) return e;
-    DrainOnError guard(w);
+    Workspace &w = *call.w;
+    Workspace::Image &m = w.img[0];
     const int64_t plane_px = (int64_t)Y * Z, plane_bytes = plane_px * C * 4, nvox = (int64_t)X * plane_px;
     const int planes = band_rows(plane_bytes, X);
-    if ((e = ws_bands(w, (size_t)planes * plane_bytes))) return e;
-    if ((e = ws_aux(w, 0, (size_t)nvox * 8))) return e;     // float64 sum volume
-    if ((e = ws_aux(w, 1, (size_t)nvox * 4))) return e;     // score
-    if ((e = ws_aux(w, 2, 64))) return e;
-    double *sum_dev = (double *)w.aux[0];
-    float *score_dev = (float *)w.aux[1];
-    unsigned long long *key = (unsigned long long *)w.aux[2];
+    if ((e = ws_ring(w, (size_t)planes * plane_bytes, is_pageable(cube_host))) || (e = m.sum.reserve((size_t)nvox * 8)) ||
+        (e = m.score.reserve((size_t)nvox * 4)) || (e = m.keys.reserve(64)))
+        return e;
+    double *sum_dev = (double *)m.sum.p;
+    float *score_dev = (float *)m.score.p;
+    unsigned long long *key = (unsigned long long *)m.keys.p;
     HIPR_CUDA(cudaEventRecord(w.t0, w.copy));
     HIPR_CUDA(cudaStreamWaitEvent(w.comp, w.t0, 0));
-    HIPR_CUDA(cudaMemsetAsync(key, 0x00, 8, w.comp));
-    HIPR_CUDA(cudaMemsetAsync(key + 1, 0xff, 8, w.comp));
-    const bool pageable = is_pageable(cube_host);
-    const int copy_threads = host_copy_threads();
-    if (pageable && (e = ws_stage(w, (size_t)planes * plane_bytes))) return e;
+    if ((e = reset_keys(key, w.comp))) return e;
     int b = 0;
-    for (int x0 = 0; x0 < X; x0 += planes, ++b) {
-        const int nx = (X - x0 < planes) ? X - x0 : planes;
-        const int slot = b % NBUF;
-        const void *src = (const char *)cube_host + (int64_t)x0 * plane_bytes;
-        if (pageable) {
-            if (b >= NBUF) HIPR_CUDA(cudaEventSynchronize(w.staged_out[slot]));
-            parallel_copy(w.stage[slot], src, (size_t)nx * plane_bytes, copy_threads);
-            src = w.stage[slot];
-        }
-        if (b >= NBUF) HIPR_CUDA(cudaStreamWaitEvent(w.copy, w.freed[slot], 0));
-        HIPR_CUDA(cudaMemcpyAsync(w.band[slot], src, (size_t)nx * plane_bytes, cudaMemcpyHostToDevice, w.copy));
-        if (pageable) HIPR_CUDA(cudaEventRecord(w.staged_out[slot], w.copy));
-        HIPR_CUDA(cudaEventRecord(w.copied[slot], w.copy));
-        HIPR_CUDA(cudaStreamWaitEvent(w.comp, w.copied[slot], 0));
-        if ((e = chansum_band(w.band[slot], 4, 1.f, (int64_t)nx * plane_px, C, sum_dev + (int64_t)x0 * plane_px, key, w.comp)))
-            return e;
-        HIPR_CUDA(cudaEventRecord(w.freed[slot], w.comp));
-    }
+    e = upload_bands(w, cube_host, X, plane_bytes, planes, b, [&](int64_t x0, int64_t nx, const void *band, cudaStream_t st) {
+        return chansum_band(band, 4, 1.f, nx * plane_px, C, sum_dev + x0 * plane_px, key, st);
+    });
+    if (e) return e;
     if (denoise_h > 0.0) {
         // bio/..._analysis.py:452-462 in full: /max -> 3-D NL-means -> float64 stencil (the denoised volume is too smooth
-        // for the fixed-point grid, as in 2-D) -> float32 score.  aux[3]: denoised volume, then the float64 score;
-        // aux[4]: the reflect-padded copy the denoise works on
+        // for the fixed-point grid, as in 2-D) -> float32 score.  scratch: denoised volume; the float64 score goes back
+        // into the sums; extra: the reflect-padded copy the denoise works on
         const int64_t wbytes = hipr_denoise_nl_means_3d_workspace(X, Y, Z, denoise_distance);
         if (wbytes < 0) return HIPR_E_UNSUPPORTED;
-        if ((e = ws_aux(w, 3, (size_t)nvox * 8))) return e;
-        if ((e = ws_aux(w, 4, (size_t)wbytes))) return e;
-        double *den = (double *)w.aux[3];
+        if ((e = m.scratch.reserve((size_t)nvox * 8)) || (e = w.extra.reserve((size_t)wbytes))) return e;
+        double *den = (double *)m.scratch.p;
         if ((e = hipr_normalize(sum_dev, HIPR_F64, nvox, (const uint64_t *)key, w.comp))) return e;
-        if ((e = hipr_denoise_nl_means_3d(sum_dev, X, Y, Z, HIPR_F64, 7, denoise_distance, denoise_h, den, w.aux[4], wbytes, w.comp)))
+        if ((e = hipr_denoise_nl_means_3d(sum_dev, X, Y, Z, HIPR_F64, 7, denoise_distance, denoise_h, den, w.extra.p, wbytes, w.comp)))
             return e;
         if ((e = hipr_lne3d(den, X, Y, Z, 0, HIPR_F64, patch_size, n_dirs, table_host, flavour, nullptr, sum_dev, w.comp))) return e;
         if ((e = hipr_normalize_cast(sum_dev, nvox, nullptr, score_dev, w.comp))) return e;
-        HIPR_CUDA(cudaMemcpyAsync(score_host, score_dev, (size_t)nvox * 4, cudaMemcpyDeviceToHost, w.comp));
-        HIPR_CUDA(cudaEventRecord(w.t1, w.comp));
-        HIPR_CUDA(cudaStreamSynchronize(w.comp));
-        HIPR_CUDA(cudaEventElapsedTime(&w.last_ms, w.t0, w.t1));
-        t_last_ms = w.last_ms;
-        guard.dismiss();
-        return HIPR_OK;
+    } else {
+        // fixed-point stencil for the reference's (11, 9, 9) table; the float64 stencil for any other table
+        e = hipr_lne3d_q(sum_dev, X, Y, Z, 0, HIPR_F64, patch_size, n_dirs, table_host, flavour, 0, (const uint64_t *)key,
+                         score_dev, w.comp);
+        if (e == HIPR_E_UNSUPPORTED) {
+            if ((e = m.scratch.reserve((size_t)nvox * 8))) return e;
+            double *score64 = (double *)m.scratch.p;
+            if ((e = hipr_lne3d(sum_dev, X, Y, Z, 0, HIPR_F64, patch_size, n_dirs, table_host, flavour, (const uint64_t *)key,
+                                score64, w.comp)))
+                return e;
+            e = hipr_normalize_cast(score64, nvox, nullptr, score_dev, w.comp);
+        }
+        if (e) return e;
     }
-    // fixed-point stencil for the reference's (11, 9, 9) table; the float64 stencil for any other table
-    e = hipr_lne3d_q(sum_dev, X, Y, Z, 0, HIPR_F64, patch_size, n_dirs, table_host, flavour, 0, (const uint64_t *)key,
-                     score_dev, w.comp);
-    if (e == HIPR_E_UNSUPPORTED) {
-        if ((e = ws_aux(w, 3, (size_t)nvox * 8))) return e;
-        double *score64 = (double *)w.aux[3];
-        if ((e = hipr_lne3d(sum_dev, X, Y, Z, 0, HIPR_F64, patch_size, n_dirs, table_host, flavour, (const uint64_t *)key,
-                            score64, w.comp)))
-            return e;
-        e = hipr_normalize_cast(score64, nvox, nullptr, score_dev, w.comp);
-    }
-    if (e) return e;
     HIPR_CUDA(cudaMemcpyAsync(score_host, score_dev, (size_t)nvox * 4, cudaMemcpyDeviceToHost, w.comp));
-    HIPR_CUDA(cudaEventRecord(w.t1, w.comp));
-    HIPR_CUDA(cudaStreamSynchronize(w.comp));
-    HIPR_CUDA(cudaEventElapsedTime(&w.last_ms, w.t0, w.t1));
-    t_last_ms = w.last_ms;
-    guard.dismiss();
-    return HIPR_OK;
+    return call.finish(w.comp);
 }
 
 extern "C" int hipr_neighbor3d_host(const float *cube_host, int X, int Y, int Z, int C, int patch_size, int n_dirs,
@@ -656,90 +661,44 @@ extern "C" int hipr_neighbor2d_host_batch(const float *const *cubes_host, int n_
     if (!cubes_host || !scores_host || n_fov < 1 || H < 1 || W < 1 || C < 1 || denoise_h < 0.0) return HIPR_E_ARG;
     for (int i = 0; i < n_fov; ++i)
         if (!cubes_host[i] || !scores_host[i]) return HIPR_E_ARG;
-    Workspace *wp = ws_current();
-    if (!wp) return HIPR_E_NODEVICE;
-    Workspace &w = *wp;
-    std::lock_guard<std::mutex> lock(w.mu);
-    int e = ws_init(w);
+    CallScope call;
+    int e = call.open();
     if (e) return e;
-    DrainOnError guard(w);
+    Workspace &w = *call.w;
     const int64_t row_bytes = (int64_t)W * C * 4;
     const int rows = band_rows(row_bytes, H);
-    if ((e = ws_bands(w, (size_t)rows * row_bytes))) return e;
     const size_t img_bytes = (size_t)H * W * 4;
-    for (int k = 0; k < 2; ++k) {
-        if ((e = ws_baux(w, k, 0, 4 * img_bytes))) return e;   // float64 sums + float64 denoised image
-        if ((e = ws_baux(w, k, 1, img_bytes))) return e;       // float32 score
-        if ((e = ws_baux(w, k, 2, 64))) return e;              // range keys
-        if ((e = ws_baux(w, k, 3, 2 * img_bytes))) return e;   // float64 score (denoise / general parameters)
-    }
-    const int copy_threads = host_copy_threads();
     bool any_pageable = false;
     for (int i = 0; i < n_fov; ++i) any_pageable = any_pageable || is_pageable(cubes_host[i]);
-    if (any_pageable && (e = ws_stage(w, (size_t)rows * row_bytes))) return e;
+    if ((e = ws_ring(w, (size_t)rows * row_bytes, any_pageable))) return e;
+    for (Workspace::Image &m : w.img)
+        if ((e = m.sum.reserve(2 * img_bytes)) || (e = m.score.reserve(img_bytes)) || (e = m.keys.reserve(64))) return e;
     HIPR_CUDA(cudaEventRecord(w.t0, w.copy));
     HIPR_CUDA(cudaStreamWaitEvent(w.comp, w.t0, 0));
     HIPR_CUDA(cudaStreamWaitEvent(w.post, w.t0, 0));
     int b = 0;                                                 // bands since the start of the call (ring slots carry over)
     for (int i = 0; i < n_fov; ++i) {
         const int k = i & 1;
-        double *sum_dev = (double *)w.baux[k][0];
-        float *score_dev = (float *)w.baux[k][1];
-        unsigned long long *key = (unsigned long long *)w.baux[k][2];
-        double *score64 = (double *)w.baux[k][3];
+        Workspace::Image &m = w.img[k];
+        double *sum_dev = (double *)m.sum.p;
+        float *score_dev = (float *)m.score.p;
+        unsigned long long *key = (unsigned long long *)m.keys.p;
         if (i >= 2) HIPR_CUDA(cudaStreamWaitEvent(w.comp, w.post_done[k], 0));   // FOV i - 2 has left this set
-        HIPR_CUDA(cudaMemsetAsync(key, 0x00, 8, w.comp));
-        HIPR_CUDA(cudaMemsetAsync(key + 1, 0xff, 8, w.comp));
-        const bool pageable = is_pageable(cubes_host[i]);
-        for (int r0 = 0; r0 < H; r0 += rows, ++b) {
-            const int nr = (H - r0 < rows) ? H - r0 : rows;
-            const int slot = b % NBUF;
-            const void *src = (const char *)cubes_host[i] + (int64_t)r0 * row_bytes;
-            if (pageable) {
-                if (b >= NBUF) HIPR_CUDA(cudaEventSynchronize(w.staged_out[slot]));
-                parallel_copy(w.stage[slot], src, (size_t)nr * row_bytes, copy_threads);
-                src = w.stage[slot];
-            }
-            if (b >= NBUF) HIPR_CUDA(cudaStreamWaitEvent(w.copy, w.freed[slot], 0));
-            HIPR_CUDA(cudaMemcpyAsync(w.band[slot], src, (size_t)nr * row_bytes, cudaMemcpyHostToDevice, w.copy));
-            if (any_pageable) HIPR_CUDA(cudaEventRecord(w.staged_out[slot], w.copy));   // (the ring's events exist only then)
-            HIPR_CUDA(cudaEventRecord(w.copied[slot], w.copy));
-            HIPR_CUDA(cudaStreamWaitEvent(w.comp, w.copied[slot], 0));
-            if ((e = chansum_band(w.band[slot], 4, 1.f, (int64_t)nr * W, C, sum_dev + (int64_t)r0 * W, key, w.comp))) return e;
-            HIPR_CUDA(cudaEventRecord(w.freed[slot], w.comp));
-        }
+        if ((e = reset_keys(key, w.comp))) return e;
+        e = upload_bands(w, cubes_host[i], H, row_bytes, rows, b,
+                         [&](int64_t r0, int64_t nr, const void *band, cudaStream_t st) {
+                             return chansum_band(band, 4, 1.f, nr * W, C, sum_dev + r0 * W, key, st);
+                         });
+        if (e) return e;
         HIPR_CUDA(cudaEventRecord(w.summed[k], w.comp));
         HIPR_CUDA(cudaStreamWaitEvent(w.post, w.summed[k], 0));
-        if (denoise_h > 0.0) {
-            double *den = sum_dev + (size_t)H * W;
-            if ((e = hipr_normalize(sum_dev, HIPR_F64, (int64_t)H * W, (const uint64_t *)key, w.post))) return e;
-            if ((e = hipr_denoise_nl_means_2d(sum_dev, H, W, HIPR_F64, 7, 11, denoise_h, den, w.post))) return e;
-            if ((e = hipr_lne2d(den, H, W, W, 0, HIPR_F64, patch_size, n_dirs, table_host, flavour, nullptr, score64, w.post)))
-                return e;
-            if ((e = hipr_normalize_cast(score64, (int64_t)H * W, nullptr, score_dev, w.post))) return e;
-        } else {
-            const bool tile_local = (flavour == HIPR_FLAVOUR_F1 || flavour == HIPR_FLAVOUR_F2);
-            e = hipr_lne2d_q(sum_dev, H, W, W, 0, HIPR_F64, patch_size, n_dirs, table_host, flavour,
-                             tile_local ? nullptr : (const uint64_t *)key, score_dev, w.post);
-            if (e == HIPR_E_TABLE && !(patch_size == 11 && n_dirs == 9)) {
-                if ((e = hipr_lne2d(sum_dev, H, W, W, 0, HIPR_F64, patch_size, n_dirs, table_host, flavour,
-                                    (const uint64_t *)key, score64, w.post)))
-                    return e;
-                e = hipr_normalize_cast(score64, (int64_t)H * W, nullptr, score_dev, w.post);
-            }
-            if (e) return e;
-        }
+        if ((e = score2d(sum_dev, key, H, W, patch_size, n_dirs, table_host, flavour, denoise_h, m.scratch, score_dev,
+                         w.post)))
+            return e;
         HIPR_CUDA(cudaMemcpyAsync(scores_host[i], score_dev, img_bytes, cudaMemcpyDeviceToHost, w.post));
         HIPR_CUDA(cudaEventRecord(w.post_done[k], w.post));
     }
-    HIPR_CUDA(cudaEventRecord(w.t1, w.post));
-    HIPR_CUDA(cudaStreamSynchronize(w.post));
-    HIPR_CUDA(cudaStreamSynchronize(w.comp));
-    HIPR_CUDA(cudaStreamSynchronize(w.copy));
-    HIPR_CUDA(cudaEventElapsedTime(&w.last_ms, w.t0, w.t1));
-    t_last_ms = w.last_ms;
-    guard.dismiss();
-    return HIPR_OK;
+    return call.finish(w.post);
 }
 
 extern "C" int hipr_neighbor2d_host_raw(const void *cube_host, int sample_bytes, double scale, int H, int W, int C,
@@ -761,34 +720,25 @@ extern "C" int hipr_cell_spectra_host(const float *cube_host, const void *labels
         npix < 1 || C < 1 || capacity < 0)
         return HIPR_E_ARG;
     if (label_bytes != 4 && label_bytes != 8) return HIPR_E_DTYPE;
-    Workspace *wp = ws_current();
-    if (!wp) return HIPR_E_NODEVICE;
-    Workspace &w = *wp;
-    std::lock_guard<std::mutex> lock(w.mu);
-    int e = ws_init(w);
+    CallScope call;
+    int e = call.open();
     if (e) return e;
-    DrainOnError guard(w);
+    Workspace &w = *call.w;
     // labels first (small), max label back to the host to size the accumulators
-    if ((e = ws_aux(w, 3, (size_t)npix * label_bytes))) return e;
-    if ((e = ws_aux(w, 2, 64))) return e;
-    void *labels_dev = w.aux[3];
-    int64_t *scalar_dev = (int64_t *)w.aux[2];
-    HIPR_CUDA(cudaMemcpyAsync(labels_dev, labels_host, (size_t)npix * label_bytes, cudaMemcpyHostToDevice, w.comp));
+    if ((e = w.input.reserve((size_t)npix * label_bytes)) || (e = w.img[0].keys.reserve(64))) return e;
+    const void *labels_dev = w.input.p;
+    int64_t *scalar_dev = (int64_t *)w.img[0].keys.p;
+    HIPR_CUDA(cudaMemcpyAsync(w.input.p, labels_host, (size_t)npix * label_bytes, cudaMemcpyHostToDevice, w.comp));
     if ((e = hipr_label_max(labels_dev, label_bytes, npix, scalar_dev, w.comp))) return e;
     int64_t max_label = 0;
     HIPR_CUDA(cudaMemcpyAsync(&max_label, scalar_dev, 8, cudaMemcpyDeviceToHost, w.comp));
     HIPR_CUDA(cudaStreamSynchronize(w.comp));
     *n_cells = 0;
-    if (max_label <= 0) {
-        guard.dismiss();
-        return HIPR_OK;
-    }
-    const size_t sums_bytes = (size_t)(max_label + 1) * C * 8;
-    const size_t cnt_bytes = (size_t)(max_label + 1) * 4;
-    if ((e = ws_aux(w, 4, sums_bytes + cnt_bytes + 16))) return e;
-    double *sums = (double *)w.aux[4];
-    int32_t *counts = (int32_t *)((char *)w.aux[4] + sums_bytes);
-    HIPR_CUDA(cudaMemsetAsync(w.aux[4], 0, sums_bytes + cnt_bytes + 16, w.comp));
+    if (max_label <= 0) return call.done();
+    w.last_cells = -1;                                   // the table buffer is rewritten from here on
+    CellTable t;
+    if ((e = cell_table(w.cells, max_label, C, t))) return e;
+    HIPR_CUDA(cudaMemsetAsync(t.sums, 0, t.acc_bytes, w.comp));
     const int64_t px_bytes = (int64_t)C * 4;
     int64_t band_px = (32ll << 20) / px_bytes;
     const int64_t W = (row_len > 0 && npix % row_len == 0) ? row_len : npix;
@@ -799,87 +749,37 @@ extern "C" int hipr_cell_spectra_host(const float *cube_host, const void *labels
         band_px &= ~31ll;
         if (band_px < 32) band_px = 32;
     }
-    if ((e = ws_bands(w, (size_t)band_px * px_bytes))) return e;
-    const bool pageable = is_pageable(cube_host);
-    const int copy_threads = host_copy_threads();
-    if (pageable && (e = ws_stage(w, (size_t)band_px * px_bytes))) return e;
+    if ((e = ws_ring(w, (size_t)(band_px * px_bytes), is_pageable(cube_host)))) return e;
     int b = 0;
-    for (int64_t p0 = 0; p0 < npix; p0 += band_px, ++b) {
-        const int64_t np = (npix - p0 < band_px) ? npix - p0 : band_px;
-        const int slot = b % NBUF;
-        const void *src = cube_host + p0 * C;
-        if (pageable) {
-            if (b >= NBUF) HIPR_CUDA(cudaEventSynchronize(w.staged_out[slot]));
-            parallel_copy(w.stage[slot], src, (size_t)np * px_bytes, copy_threads);
-            src = w.stage[slot];
-        }
-        if (b >= NBUF) HIPR_CUDA(cudaStreamWaitEvent(w.copy, w.freed[slot], 0));
-        HIPR_CUDA(cudaMemcpyAsync(w.band[slot], src, (size_t)np * px_bytes, cudaMemcpyHostToDevice, w.copy));
-        if (pageable) HIPR_CUDA(cudaEventRecord(w.staged_out[slot], w.copy));
-        HIPR_CUDA(cudaEventRecord(w.copied[slot], w.copy));
-        HIPR_CUDA(cudaStreamWaitEvent(w.comp, w.copied[slot], 0));
-        if ((e = hipr_cell_spectra_accumulate((const float *)w.band[slot], (const char *)labels_dev + p0 * label_bytes,
-                                              label_bytes, np, (W < npix) ? W : 0, C, max_label, sums, counts, nullptr,
-                                              w.comp)))
-            return e;
-        HIPR_CUDA(cudaEventRecord(w.freed[slot], w.comp));
-    }
-    // finalize into device scratch sized by max_label, then copy the valid rows back
-    const size_t row_bytes = (size_t)C * 8;
-    const size_t fin_bytes = 16 + (size_t)max_label * (16 + 2 * row_bytes);
-    if ((e = ws_aux(w, 5, fin_bytes))) return e;
-    char *fin = (char *)w.aux[5];
-    int32_t *n_dev = (int32_t *)fin;
-    int64_t *lab_dev = (int64_t *)(fin + 16);
-    int64_t *area_dev = lab_dev + max_label;
-    double *avg_dev = (double *)(area_dev + max_label);
-    double *norm_dev = avg_dev + (size_t)max_label * C;
-    if ((e = hipr_cell_spectra_finalize(sums, counts, max_label, C, n_dev, lab_dev, area_dev, avg_dev, norm_dev,
-                                        w.comp)))
-        return e;
-    int32_t n = 0;
-    HIPR_CUDA(cudaMemcpyAsync(&n, n_dev, 4, cudaMemcpyDeviceToHost, w.comp));
-    HIPR_CUDA(cudaStreamSynchronize(w.comp));
-    *n_cells = n;
-    w.last_cells = n;
+    e = upload_bands(w, cube_host, npix, px_bytes, band_px, b, [&](int64_t p0, int64_t np, const void *band, cudaStream_t st) {
+        return hipr_cell_spectra_accumulate((const float *)band, (const char *)labels_dev + p0 * label_bytes, label_bytes,
+                                            np, (W < npix) ? W : 0, C, max_label, t.sums, t.counts, nullptr, st);
+    });
+    if (e) return e;
+    e = finalize_cells(t, max_label, C, capacity, n_cells, labels_out, area_out, avgint_out, avgint_norm_out, w.comp);
+    if (e && e != HIPR_E_RANGE) return e;
+    w.last_cells = *n_cells;              // HIPR_E_RANGE: the table stays on the device (hipr_cell_spectra_host_fetch)
     w.last_max_label = max_label;
     w.last_C = C;
-    if (n > capacity || n == 0) {
-        guard.dismiss();                       // everything enqueued so far has completed
-        return n ? HIPR_E_RANGE : HIPR_OK;     // n > capacity: the table stays on the device (hipr_cell_spectra_host_fetch)
-    }
-    HIPR_CUDA(cudaMemcpyAsync(labels_out, lab_dev, (size_t)n * 8, cudaMemcpyDeviceToHost, w.comp));
-    HIPR_CUDA(cudaMemcpyAsync(area_out, area_dev, (size_t)n * 8, cudaMemcpyDeviceToHost, w.comp));
-    HIPR_CUDA(cudaMemcpyAsync(avgint_out, avg_dev, (size_t)n * row_bytes, cudaMemcpyDeviceToHost, w.comp));
-    HIPR_CUDA(cudaMemcpyAsync(avgint_norm_out, norm_dev, (size_t)n * row_bytes, cudaMemcpyDeviceToHost, w.comp));
-    HIPR_CUDA(cudaStreamSynchronize(w.comp));
-    guard.dismiss();
-    return HIPR_OK;
+    const int d = call.done();
+    return d ? d : e;
 }
 
 extern "C" int hipr_cell_spectra_host_fetch(int64_t capacity, int64_t *labels_out, int64_t *area_out, double *avgint_out,
                                             double *avgint_norm_out) {
     if (!labels_out || !area_out || !avgint_out || !avgint_norm_out) return HIPR_E_ARG;
-    Workspace *wp = ws_current();
-    if (!wp) return HIPR_E_NODEVICE;
-    Workspace &w = *wp;
-    std::lock_guard<std::mutex> lock(w.mu);
-    if (w.last_cells < 0 || !w.aux[5]) return HIPR_E_ARG;      // no table to fetch
-    const int64_t n = w.last_cells, max_label = w.last_max_label;
+    CallScope call;
+    int e = call.open();
+    if (e) return e;
+    Workspace &w = *call.w;
+    if (w.last_cells < 0 || !w.cells.p) return HIPR_E_ARG;      // no table to fetch
+    const int64_t n = w.last_cells;
     if (n > capacity) return HIPR_E_RANGE;
     if (n == 0) return HIPR_OK;
-    const size_t row_bytes = (size_t)w.last_C * 8;
-    char *fin = (char *)w.aux[5];
-    int64_t *lab_dev = (int64_t *)(fin + 16);
-    int64_t *area_dev = lab_dev + max_label;
-    double *avg_dev = (double *)(area_dev + max_label);
-    double *norm_dev = avg_dev + (size_t)max_label * w.last_C;
-    HIPR_CUDA(cudaMemcpyAsync(labels_out, lab_dev, (size_t)n * 8, cudaMemcpyDeviceToHost, w.comp));
-    HIPR_CUDA(cudaMemcpyAsync(area_out, area_dev, (size_t)n * 8, cudaMemcpyDeviceToHost, w.comp));
-    HIPR_CUDA(cudaMemcpyAsync(avgint_out, avg_dev, (size_t)n * row_bytes, cudaMemcpyDeviceToHost, w.comp));
-    HIPR_CUDA(cudaMemcpyAsync(avgint_norm_out, norm_dev, (size_t)n * row_bytes, cudaMemcpyDeviceToHost, w.comp));
-    HIPR_CUDA(cudaStreamSynchronize(w.comp));
-    return HIPR_OK;
+    CellTable t;
+    if ((e = cell_table(w.cells, w.last_max_label, w.last_C, t))) return e;   // the buffer already holds it
+    if ((e = copy_cell_table(t, n, w.last_C, labels_out, area_out, avgint_out, avgint_norm_out, w.comp))) return e;
+    return call.done();
 }
 
 
@@ -898,10 +798,9 @@ struct Fov {
     double *sum = nullptr;
     float *score = nullptr;            // (H, W) float32 scratch: score, then the normalised sum
     unsigned long long *keys = nullptr;
-    void *labels = nullptr;            // grown on demand
-    size_t labels_bytes = 0;
-    void *cells = nullptr;             // accumulators + compacted table
-    size_t cells_bytes = 0;
+    DevBuf scratch;                    // float64 score, general stencil parameters only
+    DevBuf labels;
+    DevBuf cells;                      // the cell table
     cudaStream_t copy = nullptr, comp = nullptr;
     cudaEvent_t copied = nullptr, t0 = nullptr, t1 = nullptr;
     float last_ms = -1.f;
@@ -926,14 +825,22 @@ static void fov_free(Fov *f) {
     cudaFree(f->sum);
     cudaFree(f->score);
     cudaFree(f->keys);
-    cudaFree(f->labels);
-    cudaFree(f->cells);
+    for (DevBuf *b : {&f->scratch, &f->labels, &f->cells}) b->release();
     if (f->copied) cudaEventDestroy(f->copied);
     if (f->t0) cudaEventDestroy(f->t0);
     if (f->t1) cudaEventDestroy(f->t1);
     if (f->copy) cudaStreamDestroy(f->copy);
     if (f->comp) cudaStreamDestroy(f->comp);
     delete f;
+}
+// the end of a timed handle call: t1 after the last read-back, the device time from t0
+static int fov_finish(Fov *f, Drain &drain) {
+    HIPR_CUDA(cudaEventRecord(f->t1, f->comp));
+    HIPR_CUDA(cudaStreamSynchronize(f->comp));
+    drain.armed = false;
+    HIPR_CUDA(cudaEventElapsedTime(&f->last_ms, f->t0, f->t1));
+    t_last_ms = f->last_ms;
+    return HIPR_OK;
 }
 }  // namespace hipr
 
@@ -993,8 +900,7 @@ extern "C" int hipr_fov_upload(const float *cube_host, int H, int W, int C, void
     }
     HIPR_FOV(cudaEventRecord(f->t0, f->copy));
     HIPR_FOV(cudaStreamWaitEvent(f->comp, f->t0, 0));
-    HIPR_FOV(cudaMemsetAsync(f->keys, 0x00, 8, f->comp));
-    HIPR_FOV(cudaMemsetAsync(f->keys + 1, 0xff, 8, f->comp));
+    if ((e = reset_keys(f->keys, f->comp))) return fail(e);
     // bands of ~32 MiB straight into the resident cube; the channel sum of band b runs under the copy of band b + 1.
     // Page-locked memory (hipr_host_alloc) goes at the PCIe rate; pageable memory is staged by the driver.
     const int64_t row_bytes = (int64_t)W * C * 4;
@@ -1053,24 +959,9 @@ extern "C" int hipr_fov_score(void *handle, int patch_size, int n_dirs, const in
     if (!scope.ok) return HIPR_E_NODEVICE;
     const int H = f->H, W = f->W;
     const size_t img_bytes = (size_t)H * W * 4;
-    struct Drain {
-        cudaStream_t s;
-        bool armed = true;
-        ~Drain() { if (armed) cudaStreamSynchronize(s); }
-    } drain{f->comp};
+    Drain drain{{f->comp}};
     HIPR_CUDA(cudaEventRecord(f->t0, f->comp));
-    const bool tile_local = (flavour == HIPR_FLAVOUR_F1 || flavour == HIPR_FLAVOUR_F2);
-    int e = hipr_lne2d_q(f->sum, H, W, W, 0, HIPR_F64, patch_size, n_dirs, table_host, flavour,
-                         tile_local ? nullptr : reinterpret_cast<const uint64_t *>(f->keys), f->score, f->comp);
-    if (e == HIPR_E_TABLE && !(patch_size == 11 && n_dirs == 9)) {
-        // general parameters: float64 stencil into scratch, then cast
-        double *score64 = nullptr;
-        HIPR_CUDA(cudaMallocAsync((void **)&score64, (size_t)H * W * 8, f->comp));
-        e = hipr_lne2d(f->sum, H, W, W, 0, HIPR_F64, patch_size, n_dirs, table_host, flavour,
-                       reinterpret_cast<const uint64_t *>(f->keys), score64, f->comp);
-        if (!e) e = hipr_normalize_cast(score64, (int64_t)H * W, nullptr, f->score, f->comp);
-        cudaFreeAsync(score64, f->comp);
-    }
+    int e = score2d(f->sum, f->keys, H, W, patch_size, n_dirs, table_host, flavour, 0.0, f->scratch, f->score, f->comp);
     if (e) return e;
     HIPR_CUDA(cudaMemcpyAsync(score_host, f->score, img_bytes, cudaMemcpyDeviceToHost, f->comp));
     if (sum_host) {
@@ -1078,12 +969,7 @@ extern "C" int hipr_fov_score(void *handle, int patch_size, int n_dirs, const in
             return e;
         HIPR_CUDA(cudaMemcpyAsync(sum_host, f->score, img_bytes, cudaMemcpyDeviceToHost, f->comp));
     }
-    HIPR_CUDA(cudaEventRecord(f->t1, f->comp));
-    HIPR_CUDA(cudaStreamSynchronize(f->comp));
-    drain.armed = false;
-    HIPR_CUDA(cudaEventElapsedTime(&f->last_ms, f->t0, f->t1));
-    t_last_ms = f->last_ms;
-    return HIPR_OK;
+    return fov_finish(f, drain);
 }
 
 extern "C" int hipr_fov_cell_spectra(void *handle, const void *labels_host, int label_bytes, int64_t capacity,
@@ -1098,23 +984,13 @@ extern "C" int hipr_fov_cell_spectra(void *handle, const void *labels_host, int 
     if (!scope.ok) return HIPR_E_NODEVICE;
     const int64_t npix = (int64_t)f->H * f->W;
     const int C = f->C;
-    struct Drain {
-        cudaStream_t s;
-        bool armed = true;
-        ~Drain() { if (armed) cudaStreamSynchronize(s); }
-    } drain{f->comp};
-    if ((size_t)npix * label_bytes > f->labels_bytes) {
-        cudaFree(f->labels);
-        f->labels = nullptr;
-        f->labels_bytes = 0;
-        HIPR_CUDA(cudaMalloc(&f->labels, (size_t)npix * label_bytes));
-        f->labels_bytes = (size_t)npix * label_bytes;
-    }
-    HIPR_CUDA(cudaEventRecord(f->t0, f->comp));
-    HIPR_CUDA(cudaMemcpyAsync(f->labels, labels_host, (size_t)npix * label_bytes, cudaMemcpyHostToDevice, f->comp));
-    int64_t *scalar_dev = reinterpret_cast<int64_t *>(f->keys + 4);      // the handle's 64-byte scratch, past the keys
-    int e = hipr_label_max(f->labels, label_bytes, npix, scalar_dev, f->comp);
+    Drain drain{{f->comp}};
+    int e = f->labels.reserve((size_t)npix * label_bytes);
     if (e) return e;
+    HIPR_CUDA(cudaEventRecord(f->t0, f->comp));
+    HIPR_CUDA(cudaMemcpyAsync(f->labels.p, labels_host, (size_t)npix * label_bytes, cudaMemcpyHostToDevice, f->comp));
+    int64_t *scalar_dev = reinterpret_cast<int64_t *>(f->keys + 4);      // the handle's 64-byte scratch, past the keys
+    if ((e = hipr_label_max(f->labels.p, label_bytes, npix, scalar_dev, f->comp))) return e;
     int64_t max_label = 0;
     HIPR_CUDA(cudaMemcpyAsync(&max_label, scalar_dev, 8, cudaMemcpyDeviceToHost, f->comp));
     HIPR_CUDA(cudaStreamSynchronize(f->comp));
@@ -1123,47 +999,16 @@ extern "C" int hipr_fov_cell_spectra(void *handle, const void *labels_host, int 
         drain.armed = false;
         return HIPR_OK;
     }
-    const size_t row_bytes = (size_t)C * 8;
-    const size_t sums_bytes = (size_t)(max_label + 1) * row_bytes, cnt_bytes = ((size_t)(max_label + 1) * 4 + 15) & ~(size_t)15;
-    const size_t fin_off = sums_bytes + cnt_bytes + 16;
-    const size_t need = fin_off + 16 + (size_t)max_label * (16 + 2 * row_bytes);
-    if (need > f->cells_bytes) {
-        cudaFree(f->cells);
-        f->cells = nullptr;
-        f->cells_bytes = 0;
-        HIPR_CUDA(cudaMalloc(&f->cells, need));
-        f->cells_bytes = need;
-    }
-    double *sums = reinterpret_cast<double *>(f->cells);
-    int32_t *counts = reinterpret_cast<int32_t *>((char *)f->cells + sums_bytes);
-    char *fin = (char *)f->cells + fin_off;
-    int32_t *n_dev = reinterpret_cast<int32_t *>(fin);
-    int64_t *lab_dev = reinterpret_cast<int64_t *>(fin + 16);
-    int64_t *area_dev = lab_dev + max_label;
-    double *avg_dev = reinterpret_cast<double *>(area_dev + max_label);
-    double *norm_dev = avg_dev + (size_t)max_label * C;
-    HIPR_CUDA(cudaMemsetAsync(f->cells, 0, fin_off, f->comp));
-    if ((e = hipr_cell_spectra_accumulate(f->cube, f->labels, label_bytes, npix, f->W, C, max_label, sums, counts, nullptr,
-                                          f->comp)))
+    CellTable t;
+    if ((e = cell_table(f->cells, max_label, C, t))) return e;
+    HIPR_CUDA(cudaMemsetAsync(t.sums, 0, t.acc_bytes, f->comp));
+    if ((e = hipr_cell_spectra_accumulate(f->cube, f->labels.p, label_bytes, npix, f->W, C, max_label, t.sums, t.counts,
+                                          nullptr, f->comp)))
         return e;
-    if ((e = hipr_cell_spectra_finalize(sums, counts, max_label, C, n_dev, lab_dev, area_dev, avg_dev, norm_dev, f->comp)))
-        return e;
-    int32_t n = 0;
-    HIPR_CUDA(cudaMemcpyAsync(&n, n_dev, 4, cudaMemcpyDeviceToHost, f->comp));
-    HIPR_CUDA(cudaStreamSynchronize(f->comp));
-    *n_cells = n;
-    if (n > capacity || n == 0) {
+    e = finalize_cells(t, max_label, C, capacity, n_cells, labels_out, area_out, avgint_out, avgint_norm_out, f->comp);
+    if (e == HIPR_E_RANGE || (!e && *n_cells == 0)) {
         drain.armed = false;
-        return n ? HIPR_E_RANGE : HIPR_OK;    // HIPR_E_RANGE: call again with capacity >= *n_cells (the cube is resident)
+        return e;                              // HIPR_E_RANGE: call again with capacity >= *n_cells (the cube is resident)
     }
-    HIPR_CUDA(cudaMemcpyAsync(labels_out, lab_dev, (size_t)n * 8, cudaMemcpyDeviceToHost, f->comp));
-    HIPR_CUDA(cudaMemcpyAsync(area_out, area_dev, (size_t)n * 8, cudaMemcpyDeviceToHost, f->comp));
-    HIPR_CUDA(cudaMemcpyAsync(avgint_out, avg_dev, (size_t)n * row_bytes, cudaMemcpyDeviceToHost, f->comp));
-    HIPR_CUDA(cudaMemcpyAsync(avgint_norm_out, norm_dev, (size_t)n * row_bytes, cudaMemcpyDeviceToHost, f->comp));
-    HIPR_CUDA(cudaEventRecord(f->t1, f->comp));
-    HIPR_CUDA(cudaStreamSynchronize(f->comp));
-    drain.armed = false;
-    HIPR_CUDA(cudaEventElapsedTime(&f->last_ms, f->t0, f->t1));
-    t_last_ms = f->last_ms;
-    return HIPR_OK;
+    return e ? e : fov_finish(f, drain);
 }

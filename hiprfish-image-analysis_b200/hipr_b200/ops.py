@@ -486,29 +486,35 @@ def line_profile_2d(image_padded, patch_size, phi_range):
     return out
 
 
+def _host_gather(name, image_padded, ndim, table_args, what, per_sample, out, pinned):
+    """The host gathers, hipr_<name>: a padded float64 image / volume in; out: the caller's C-contiguous float64
+    array, or a new one (backed by page-locked memory with pinned=True) of the unpadded shape + (n_dirs,) and, with
+    per_sample, + (P,)."""
+    a = np.ascontiguousarray(image_padded)
+    if a.dtype != np.float64:
+        raise TypeError("image_padded must be float64, got %s" % a.dtype)
+    if a.ndim != ndim:
+        raise ValueError("Buffer has wrong number of dimensions (expected %d, got %d)" % (ndim, a.ndim))
+    tab = (tables.line_table_2d if ndim == 2 else tables.line_table_3d)(*table_args)
+    R, P = tab.shape[0], tab.shape[1]
+    if min(a.shape) < P:
+        raise ValueError("%s smaller than the patch" % what)
+    shape = tuple(d - P + 1 for d in a.shape) + ((R, P) if per_sample else (R,))
+    if out is None:
+        out = torch.empty(shape, dtype=torch.float64, pin_memory=True).numpy() if pinned else np.empty(shape, dtype=np.float64)
+    elif out.shape != shape or out.dtype != np.float64 or not out.flags.c_contiguous:
+        raise ValueError("out must be a C-contiguous float64 array of shape %s" % (shape,))
+    check(getattr(lib(), "hipr_" + name)(a.ctypes.data_as(C.c_void_p), *a.shape, P, R, _tab_ptr(tab),
+                                         out.ctypes.data_as(C.c_void_p)), name)
+    return out
+
+
 def line_profile_2d_host(image_padded, patch_size, phi_range, out=None, pinned=False):
     """numpy float64 (Hp, Wp) -> numpy float64 (Hp-P+1, Wp-P+1, phi_range, P) through hipr_line_profile_2d_host: the
     gather runs in row bands on the device under the device -> host copy of the previous bands.  out: a caller's
     array (page-locked or not); pinned=True returns an array backed by page-locked memory (torch's caching host
     allocator), which the copy reaches at the PCIe rate without the staging ring."""
-    a = np.ascontiguousarray(image_padded)
-    if a.dtype != np.float64:
-        raise TypeError("image_padded must be float64, got %s" % a.dtype)
-    if a.ndim != 2:
-        raise ValueError("Buffer has wrong number of dimensions (expected 2, got %d)" % a.ndim)
-    tab = tables.line_table_2d(patch_size, phi_range)
-    R, P = tab.shape[0], tab.shape[1]
-    Hp, Wp = a.shape
-    if Hp < P or Wp < P:
-        raise ValueError("image smaller than the patch")
-    shape = (Hp - P + 1, Wp - P + 1, R, P)
-    if out is None:
-        out = torch.empty(shape, dtype=torch.float64, pin_memory=True).numpy() if pinned else np.empty(shape, dtype=np.float64)
-    elif out.shape != shape or out.dtype != np.float64 or not out.flags.c_contiguous:
-        raise ValueError("out must be a C-contiguous float64 array of shape %s" % (shape,))
-    check(lib().hipr_line_profile_2d_host(a.ctypes.data_as(C.c_void_p), Hp, Wp, P, R, _tab_ptr(tab),
-                                          out.ctypes.data_as(C.c_void_p)), "line_profile_2d_host")
-    return out
+    return _host_gather("line_profile_2d_host", image_padded, 2, (patch_size, phi_range), "image", True, out, pinned)
 
 
 def _vol(volume, name):
@@ -553,47 +559,15 @@ def lne3d_dirs(volume, patch_size=11, theta_range=9, phi_range=9, padded=True, m
 def lne3d_dirs_host(volume_padded, patch_size=11, theta_range=9, phi_range=9, out=None, pinned=False):
     """numpy float64 (Xp, Yp, Zp) -> numpy float64 (X, Y, Z, T) through hipr_lne3d_dirs_host
     (line_profile_memory_efficient_v2 for host arrays: bands of x-planes under the device -> host copy)."""
-    a = np.ascontiguousarray(volume_padded)
-    if a.dtype != np.float64:
-        raise TypeError("image_padded must be float64, got %s" % a.dtype)
-    if a.ndim != 3:
-        raise ValueError("Buffer has wrong number of dimensions (expected 3, got %d)" % a.ndim)
-    tab = tables.line_table_3d(patch_size, theta_range, phi_range)
-    T, P = tab.shape[0], tab.shape[1]
-    Xp, Yp, Zp = a.shape
-    if min(a.shape) < P:
-        raise ValueError("volume smaller than the patch")
-    shape = (Xp - P + 1, Yp - P + 1, Zp - P + 1, T)
-    if out is None:
-        out = torch.empty(shape, dtype=torch.float64, pin_memory=True).numpy() if pinned else np.empty(shape, dtype=np.float64)
-    elif out.shape != shape or out.dtype != np.float64 or not out.flags.c_contiguous:
-        raise ValueError("out must be a C-contiguous float64 array of shape %s" % (shape,))
-    check(lib().hipr_lne3d_dirs_host(a.ctypes.data_as(C.c_void_p), Xp, Yp, Zp, P, T, _tab_ptr(tab),
-                                     out.ctypes.data_as(C.c_void_p)), "lne3d_dirs_host")
-    return out
+    return _host_gather("lne3d_dirs_host", volume_padded, 3, (patch_size, theta_range, phi_range), "volume", False,
+                        out, pinned)
 
 
 def line_profile_3d_host(volume_padded, patch_size=11, theta_range=9, phi_range=9, out=None, pinned=False):
     """numpy float64 (Xp, Yp, Zp) -> numpy float64 (X, Y, Z, T, P) through hipr_line_profile_3d_host
     (line_profile_v2 for host arrays: bands of x-planes under the device -> host copy)."""
-    a = np.ascontiguousarray(volume_padded)
-    if a.dtype != np.float64:
-        raise TypeError("image_padded must be float64, got %s" % a.dtype)
-    if a.ndim != 3:
-        raise ValueError("Buffer has wrong number of dimensions (expected 3, got %d)" % a.ndim)
-    tab = tables.line_table_3d(patch_size, theta_range, phi_range)
-    T, P = tab.shape[0], tab.shape[1]
-    Xp, Yp, Zp = a.shape
-    if min(a.shape) < P:
-        raise ValueError("volume smaller than the patch")
-    shape = (Xp - P + 1, Yp - P + 1, Zp - P + 1, T, P)
-    if out is None:
-        out = torch.empty(shape, dtype=torch.float64, pin_memory=True).numpy() if pinned else np.empty(shape, dtype=np.float64)
-    elif out.shape != shape or out.dtype != np.float64 or not out.flags.c_contiguous:
-        raise ValueError("out must be a C-contiguous float64 array of shape %s" % (shape,))
-    check(lib().hipr_line_profile_3d_host(a.ctypes.data_as(C.c_void_p), Xp, Yp, Zp, P, T, _tab_ptr(tab),
-                                     out.ctypes.data_as(C.c_void_p)), "line_profile_3d_host")
-    return out
+    return _host_gather("line_profile_3d_host", volume_padded, 3, (patch_size, theta_range, phi_range), "volume", True,
+                        out, pinned)
 
 
 def lne3d(volume, flavour="F2", patch_size=11, theta_range=9, phi_range=9, padded=False, maxkey=None):
@@ -1156,16 +1130,10 @@ def neighbor2d_score_host(cube, flavour="F1", patch_size=11, phi_range=9, return
     tab = tables.line_table_2d(patch_size, phi_range)
     score = out if out is not None else np.empty((H, W), dtype=np.float32)
     s = np.empty((H, W), dtype=np.float32) if return_sum else None
-    if denoise_h is not None:
-        check(lib().hipr_neighbor2d_host_denoise(cube.ctypes.data_as(C.c_void_p), H, W, Cn, tab.shape[1], tab.shape[0],
-                                                 _tab_ptr(tab), _flavour(flavour), float(denoise_h),
-                                                 score.ctypes.data_as(C.c_void_p),
-                                                 s.ctypes.data_as(C.c_void_p) if return_sum else None),
-              "neighbor2d_host_denoise")
-        return (score, s) if return_sum else score
-    check(lib().hipr_neighbor2d_host(cube.ctypes.data_as(C.c_void_p), H, W, Cn, tab.shape[1], tab.shape[0],
-                                     _tab_ptr(tab), _flavour(flavour), score.ctypes.data_as(C.c_void_p),
-                                     s.ctypes.data_as(C.c_void_p) if return_sum else None), "neighbor2d_host")
+    name, denoise = ("neighbor2d_host", ()) if denoise_h is None else ("neighbor2d_host_denoise", (float(denoise_h),))
+    check(getattr(lib(), "hipr_" + name)(cube.ctypes.data_as(C.c_void_p), H, W, Cn, tab.shape[1], tab.shape[0],
+                                         _tab_ptr(tab), _flavour(flavour), *denoise, score.ctypes.data_as(C.c_void_p),
+                                         s.ctypes.data_as(C.c_void_p) if return_sum else None), name)
     return (score, s) if return_sum else score
 
 
