@@ -24,11 +24,9 @@
 //                       4 pixels per thread, and writes the float32 scores.
 // Neighbouring strips re-read 16 of 144 window columns; they run in lock step, so the second
 // read is an L2 hit.  Bands re-read 10 halo rows each (4 % at 2048 rows / 9 bands).
-#include <cstdlib>
-#include <type_traits>
 #include "hipr_common.cuh"
 #include "lne_math.cuh"
-#include "baked_tables.cuh"
+#include "lne_fixed.cuh"
 
 namespace hipr {
 
@@ -43,19 +41,7 @@ constexpr int FU_QW = FU_WT + 10, FU_QH = FU_RB + 10;               // 138 x 18 
 constexpr int FU_MAX_STAGES = 4;
 constexpr int FU_SMEM_FIXED = 256 + FU_RING * FU_WIN * 8 + FU_QH * FU_QW * 4 + 256;
 constexpr int FU_SMEM_BUDGET = 227 * 1024;
-constexpr uint32_t FU_BIAS = 0x00800000u;
-constexpr double FU_SPAN = (double)0x7E000000u;
 
-constexpr int fu_baked_off(int t, int li) {
-    return kBaked2D[(t * 11 + li) * 2] * FU_QW + kBaked2D[(t * 11 + li) * 2 + 1];
-}
-template <int I, int N, typename F>
-__device__ __forceinline__ void fu_static_for(F &&f) {
-    if constexpr (I < N) {
-        f(std::integral_constant<int, I>{});
-        fu_static_for<I + 1, N>(f);
-    }
-}
 __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
     asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
@@ -205,15 +191,14 @@ fused2d_kernel(const float *__restrict__ cube, const FusedGeom g, float *__restr
             wmax = fmax(wmax, red[j * 2]);
             wmin = fmin(wmin, red[j * 2 + 1]);
         }
-        const double K = (wmax > wmin) ? FU_SPAN / (wmax - wmin) : 0.0;
+        const double K = q_scale(wmax, wmin);
         // 2. fixed-point tile
         for (int e = st; e < FU_QH * FU_QW; e += NST) {
             const int ty = e / FU_QW, tx = e - ty * FU_QW;
             const int wy = min(max(r - 5 + ty, 0), H - 1), wx = min(max(x0 - 5 + tx, 0), W - 1);
             double v = ring[(wy % FU_RING) * FU_WIN + (wx - xa)];
             if (v != v) v = 0.0;
-            const double qd = fmin(fmax((v - wmin) * K, 0.0), FU_SPAN);
-            qtile[e] = __uint_as_float(__double2uint_rn(qd) + FU_BIAS);
+            qtile[e] = q_encode(v, wmin, K);
         }
         named_bar_sync(1, NST);
         // the ring rows of this block are no longer needed
@@ -228,36 +213,27 @@ fused2d_kernel(const float *__restrict__ cube, const FusedGeom g, float *__restr
                 if (x >= W) break;
                 const float *base = qtile + sw * FU_QW + lx;
                 float rr[9];
-                fu_static_for<0, 9>([&](auto tc) {
+                static_for<0, 9>([&](auto tc) {
                     constexpr int t = decltype(tc)::value;
-                    constexpr int o0 = fu_baked_off(t, 0);
+                    constexpr int o0 = baked2d_off<FU_QW>(t, 0);
                     float mn = base[o0], mx = mn;
-                    fu_static_for<1, 11>([&](auto lc) {
-                        constexpr int off = fu_baked_off(t, decltype(lc)::value);
+                    static_for<1, 11>([&](auto lc) {
+                        constexpr int off = baked2d_off<FU_QW>(t, decltype(lc)::value);
                         const float s = base[off];
                         mn = fminf(mn, s);
                         mx = fmaxf(mx, s);
                     });
-                    constexpr int oc = fu_baked_off(t, 5);
-                    const float c = base[oc];
-                    const float dq = __uint2float_rn(__float_as_uint(c) - __float_as_uint(mn));
-                    const float rq = __uint2float_rn(__float_as_uint(mx) - __float_as_uint(mn));
-                    rr[t] = __fdividef(dq, rq);               // 0/0 -> NaN on a flat line, as numpy
+                    constexpr int oc = baked2d_off<FU_QW>(t, 5);
+                    rr[t] = q_line<FLAVOUR>(base[oc], mn, mx, 0.f);
                 });
                 float sum = 0.f;
 #pragma unroll
                 for (int q = 0; q < 9; ++q) sum += rr[q];
                 const float mean = sum * (1.0f / 9.0f);
                 sort_network<float, 9>(rr);
-                const float lq = rr[2], uq = rr[6];
-                float factor;
-                if (FLAVOUR == HIPR_FLAVOUR_F1) {
-                    factor = (uq > 0.f) ? __fdiv_rn(2.f * lq + 1e-8f, uq + lq + 1e-8f) : 1.f;
-                } else {
-                    const float sden = uq + lq;
-                    factor = (sden == 0.f) ? 1.f : __fdiv_rn(2.f * lq, sden);
-                }
-                score[(int64_t)y * W + x] = mean * factor;
+                float A, B;
+                bool unit;
+                score[(int64_t)y * W + x] = mean * q_factor<FLAVOUR>(rr[2], rr[6], A, B, unit);
             }
         }
         // all warps must be done with qtile / red before the next block rewrites them

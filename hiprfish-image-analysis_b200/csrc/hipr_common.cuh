@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <atomic>
+#include <type_traits>
 #include "hipr_b200.h"
 
 #ifndef __CUDA_ARCH__
@@ -314,6 +315,16 @@ __device__ __forceinline__ double warp_max(double v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, o));
     return v;
+}
+
+// f(std::integral_constant<int, i>{}) for i = I .. N-1: the index is a constant expression inside f (LDS immediates,
+// compile-time register indices)
+template <int I, int N, typename F>
+__device__ __forceinline__ void static_for(F &&f) {
+    if constexpr (I < N) {
+        f(std::integral_constant<int, I>{});
+        static_for<I + 1, N>(f);
+    }
 }
 #endif  // __CUDACC__
 

@@ -4,72 +4,43 @@
 // range is ~1/10 of the value, so any rounding of the sum image is amplified ~10-20x.  A
 // float32 sum image (6e-8 relative) lands at ~6e-6 in the score -- outside the 1e-5 parity gate
 // on some pixels -- and a float64 stencil costs 3-4x the instructions (no DMNMX on sm_100).
-// Instead the tile loader maps the float64 channel sums affinely onto integers,
-//     q = (S - min) * (0x7E000000 / (max - min)) + 0x00800000,
-// with the global min / max that K1 produced.  F1/F2 scores are invariant under that map; F3 and
-// ME2 carry their 1e-8 epsilon into q units (eps_q = 1e-8 * max * K).  The integers are stored as
-// the bit patterns of positive normal floats, whose ordering is the integer ordering, so the
-// 11-sample min / max run on FMNMX3 exactly as a float kernel would -- but every min, max and
-// difference is EXACT; the only roundings left are two int->float conversions and one divide
-// per line (~1e-7).  Quantisation step: (max - min) * 4.7e-10.
+// Instead the tile loader maps the float64 channel sums onto the 31-bit fixed-point grid of
+// lne_fixed.cuh, with the global min / max that K1 produced or the tile's own.  The 11-sample
+// min / max run on FMNMX3 exactly as a float kernel would -- but every min, max and difference is
+// EXACT; the only roundings left are two int->float conversions and one divide per line (~1e-7).
+// Quantisation step: (max - min) * 4.7e-10.
 //
 // With the pinned (11, 9) table the sample offsets are compile-time immediates of the LDS
 // instructions (baked_tables.cuh); any other 11x9 table takes the parameter-bank variant.
-#include <cstdlib>
-#include <type_traits>
 #include "hipr_common.cuh"
 #include "lne_math.cuh"
-#include "baked_tables.cuh"
+#include "lne_fixed.cuh"
 
 namespace hipr {
 
 constexpr int Q_TW = 32, Q_TH = 32, Q_P = 11, Q_R = 9, Q_HALF = 5;
 constexpr int Q_SW = Q_TW + Q_P - 1;  // 42
 constexpr int Q_SH = Q_TH + Q_P - 1;  // 42
-constexpr uint32_t Q_BIAS = 0x00800000u;          // smallest positive normal float
-constexpr double Q_SPAN = (double)0x7E000000u;    // BIAS + SPAN = 0x7E800000 < +inf
 
 struct TableQ {
     int off[Q_R * Q_P];  // dy * Q_SW + dx
 };
 
-constexpr int q_baked_off(int t, int li) {
-    return kBaked2D[(t * Q_P + li) * 2] * Q_SW + kBaked2D[(t * Q_P + li) * 2 + 1];
-}
 // T and LI are compile-time, so the baked offset is a constant expression (an LDS immediate)
 template <bool BAKED, int T, int LI>
 __device__ __forceinline__ int q_off(const TableQ &tab) {
     if constexpr (BAKED) {
-        constexpr int off = q_baked_off(T, LI);
+        constexpr int off = baked2d_off<Q_SW>(T, LI);
         return off;
     } else {
         return tab.off[T * Q_P + LI];
     }
 }
-template <int I, int N, typename F>
-__device__ __forceinline__ void static_for(F &&f) {
-    if constexpr (I < N) {
-        f(std::integral_constant<int, I>{});
-        static_for<I + 1, N>(f);
-    }
-}
 
-// Pixels the grid cannot resolve to 1e-5 RELATIVE.  Every sample is off by at most half a grid unit, so the two
-// differences of a line value r_t = dq_t / rq_t are each off by at most one unit and
-//     |delta r_t| <= (1 + r_t) * e_t,   e_t = 1 / rq_t,
-// whatever the size of r_t: a small non-zero lq, uq or mean (a pixel that is almost, but not quite, the minimum of
-// its lines) keeps that absolute error and loses relative accuracy.  Line values that are exactly 0 on the grid are
-// exact (the grid preserves order, so the centre is the line's minimum).  The bound is propagated through
-//     score = mean * (2 lq + eps) / (uq + lq + eps)
-// (the mean and the order statistics are 1-Lipschitz in the r_t) and the pixel is marked when the bound on the
-// relative error exceeds Q_REFINE_THR = 8e-6, which
-// leaves 2e-6 for the float32 roundings of the epilogue.  Marked pixels (~0.3 % of a synthetic field of view) are
-// written as a sentinel no score can take and recomputed from the float64 image by lne2d_refine_kernel, which packs
-// them densely (refining inside the stencil CTA was measured slower: its shared-memory footprint and its thinly
-// populated warps kept the stencil from running beside the channel sum of the next field of view; a list in global
-// memory needs an allocation per call).
-constexpr float Q_REFINE_THR = 8e-6f;
-constexpr float Q_SENTINEL = -2.0f;
+// Marked pixels (~0.3 % of a synthetic field of view, see the bound in lne_fixed.cuh) are recomputed from the float64
+// image by lne2d_refine_kernel, which packs them densely (refining inside the stencil CTA was measured slower: its
+// shared-memory footprint and its thinly populated warps kept the stencil from running beside the channel sum of the
+// next field of view; a list in global memory needs an allocation per call).
 constexpr int Q_RPIX = 28;     // marked pixels per refinement round of a CTA: 28 * 9 = 252 (pixel, line) pairs
 
 // n / d to ~1e-14 relative without the float64 divide subroutine: float32 reciprocal + one Newton step in float64
@@ -80,7 +51,6 @@ __device__ __forceinline__ double q_fast_div(double n, double d) {
     return fma(fma(-q0, d, n), rc, q0);
 }
 
-// (1 - qcv) without the cancellation: 1 - (uq-lq)/(uq+lq+e) = (2 lq + e)/(uq+lq+e)
 // inv[t] = 1 / (range of line t in grid units) = e_t
 template <int FLAVOUR, bool REFINE>
 __device__ __forceinline__ float q_reduce(float (&r)[Q_R], const float (&inv)[Q_R]) {
@@ -95,57 +65,28 @@ __device__ __forceinline__ float q_reduce(float (&r)[Q_R], const float (&inv)[Q_
     }
     sort_network<float, Q_R>(r);
     const float lq = r[2], uq = r[6];  // np.percentile(.., 25 / 75) of 9 values: order statistics 2 and 6
-    float factor, A, B;
-    bool unit = false;                 // factor is exactly 1
-    if (FLAVOUR == HIPR_FLAVOUR_F1) {
-        A = 2.f * lq + 1e-8f;
-        B = uq + lq + 1e-8f;
-        unit = !(uq > 0.f);
-        factor = unit ? 1.f : __fdiv_rn(A, B);
-    } else if (FLAVOUR == HIPR_FLAVOUR_F2 || FLAVOUR == HIPR_FLAVOUR_ME2) {
-        A = 2.f * lq;
-        B = uq + lq;
-        unit = (B == 0.f);
-        factor = unit ? 1.f : __fdiv_rn(A, B);   // nan_to_num(0/0) = 0 -> factor 1
-    } else {
-        A = 2.f * lq + 1e-8f;
-        B = uq + lq + 1e-8f;
-        factor = __fdiv_rn(A, B);
-    }
+    float A, B;
+    bool unit;
+    const float factor = q_factor<FLAVOUR>(lq, uq, A, B, unit);
     if (REFINE) {
-        // bound on the relative error: d_mean / mean + d_A / A + d_B / B > thr, divisions multiplied out, with
-        //   d_mean <= (1 + mean) e_max,  d_lq = (1 + lq) e_lq [lq > 0],  d_uq = (1 + uq) e_uq [uq > 0],
-        //   d_A = 2 d_lq,  d_B = d_lq + d_uq.
-        // First with e_max for e_lq, e_uq (cheap, passes ~97 % of the pixels); the rest look up the e of the lines
-        // that gave lq and uq.  NaN (a flat line) compares false and keeps the fixed-point result's NaN.
+        // First with e_max for the e of every line (cheap, passes ~97 % of the pixels); the rest look up the e of the
+        // lines that gave lq and uq and sum the exact mean term.
         float e_max = inv[0];
 #pragma unroll
         for (int i = 1; i < Q_R; ++i) e_max = fmaxf(e_max, inv[i]);
-        const float thr_mean = Q_REFINE_THR * mean;
-        bool mark;
-        if (unit) mark = fmaf(mean, e_max, e_max) > thr_mean;
-        else {
-            const float d_lq = (lq > 0.f) ? fmaf(lq, e_max, e_max) : 0.f;
-            const float d_uq = (uq > 0.f) ? fmaf(uq, e_max, e_max) : 0.f;
-            mark = fmaf(mean, 2.f * d_lq * B + (d_lq + d_uq) * A, fmaf(mean, e_max, e_max) * A * B) > thr_mean * A * B;
-        }
+        bool mark = q_mark<true>(unit, mean, q_err(lq, e_max), q_err(uq, e_max), fmaf(mean, e_max, e_max), A, B);
         if (mark) {
-            // exact terms: d_mean = sum over the lines with r > 0 of (1 + r_t) e_t / 9 (a line value that is exactly
-            // 0 on the grid is exact), e of the lines that gave lq and uq (ties: the largest)
+            // exact terms: d_mean = sum over the lines of their bound / 9, e of the lines that gave lq and uq (ties: the
+            // largest)
             float d_sum = 0.f, e_lq = 0.f, e_uq = 0.f;
 #pragma unroll
             for (int i = 0; i < Q_R; ++i) {
-                d_sum += (r0[i] > 0.f) ? fmaf(r0[i], inv[i], inv[i]) : 0.f;
+                d_sum += q_err(r0[i], inv[i]);
                 e_lq = (r0[i] == lq) ? fmaxf(e_lq, inv[i]) : e_lq;
                 e_uq = (r0[i] == uq) ? fmaxf(e_uq, inv[i]) : e_uq;
             }
             const float d_mean = d_sum * (1.0f / Q_R);
-            if (unit) mark = d_mean > thr_mean;
-            else {
-                const float p_lq = (lq > 0.f) ? fmaf(lq, e_lq, e_lq) : 0.f;
-                const float p_uq = (uq > 0.f) ? fmaf(uq, e_uq, e_uq) : 0.f;
-                mark = fmaf(mean, 2.f * p_lq * B + (p_lq + p_uq) * A, d_mean * A * B) > thr_mean * A * B;
-            }
+            mark = q_mark<true>(unit, mean, q_err(lq, e_lq), q_err(uq, e_uq), d_mean, A, B);
         }
         if (mark) return Q_SENTINEL;
     }
@@ -186,28 +127,14 @@ lne2d_q_kernel(const SrcT *__restrict__ img, int Hs, int Ws, int64_t ld, int src
     } else {
         // LOCAL range: F1/F2 are invariant to any affine map, so the tile's own min/max serve (and
         // give a finer grid); the stencil then does not depend on a global reduction
-        vmax = warp_max(vmax);
-        vmin = -warp_max(-vmin);
-        if ((threadIdx.x & 31) == 0) {
-            red[(threadIdx.x >> 5) * 2] = vmax;
-            red[(threadIdx.x >> 5) * 2 + 1] = vmin;
-        }
-        __syncthreads();
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            vmax = fmax(vmax, red[2 * j]);
-            vmin = fmin(vmin, red[2 * j + 1]);
-        }
+        block8_minmax(vmax, vmin, red, threadIdx.x, [] { __syncthreads(); });
     }
-    const double K = (vmax > vmin) ? Q_SPAN / (vmax - vmin) : 0.0;
-    const float eps_q = (K > 0.0) ? (float)(1e-8 * fabs(vmax) * K) : 1.0f;
+    const double K = q_scale(vmax, vmin);
+    const float eps_q = q_eps(vmax, K);
 #pragma unroll
     for (int k = 0; k < PER; ++k) {
         const int i = threadIdx.x + 256 * k;
-        if (i < Q_SH * Q_SW) {
-            const double qd = fmin(fmax((vals[k] - vmin) * K, 0.0), Q_SPAN);
-            tile[i] = __uint_as_float(__double2uint_rn(qd) + Q_BIAS);
-        }
+        if (i < Q_SH * Q_SW) tile[i] = q_encode(vals[k], vmin, K);
     }
     __syncthreads();
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
@@ -227,16 +154,7 @@ lne2d_q_kernel(const SrcT *__restrict__ img, int Hs, int Ws, int64_t ld, int src
                 mn = fminf(mn, s);
                 mx = fmaxf(mx, s);
             });
-            const float c = base[q_off<BAKED, t, Q_HALF>(tab)];
-            const float dq = __uint2float_rn(__float_as_uint(c) - __float_as_uint(mn));
-            const float rq = __uint2float_rn(__float_as_uint(mx) - __float_as_uint(mn));
-            float den;
-            if (FLAVOUR == HIPR_FLAVOUR_F1 || FLAVOUR == HIPR_FLAVOUR_F2) den = rq;   // 0/0 -> NaN on a flat line
-            else if (FLAVOUR == HIPR_FLAVOUR_F3) den = rq + eps_q;
-            else den = fmaxf(rq, eps_q);
-            const float inv = __fdividef(1.0f, den);             // MUFU.RCP; dq * inv is what __fdividef(dq, den) does
-            r[t] = dq * inv;
-            e[t] = inv;
+            r[t] = q_line<FLAVOUR>(base[q_off<BAKED, t, Q_HALF>(tab)], mn, mx, eps_q, &e[t]);
         });
         out[(int64_t)y * W + x] = q_reduce<FLAVOUR, REFINE>(r, e);   // Q_SENTINEL where marked
     }
@@ -293,9 +211,7 @@ lne2d_refine_kernel(const SrcT *__restrict__ img, int Hs, int Ws, int64_t ld, in
                 mn = fmin(mn, v[li]);
                 mx = fmax(mx, v[li]);
             }
-            double den = mx - mn;
-            if (FLAVOUR == HIPR_FLAVOUR_F3) den += eps;
-            else if (FLAVOUR != HIPR_FLAVOUR_F1 && FLAVOUR != HIPR_FLAVOUR_F2) den = fmax(den, eps);
+            const double den = q_den<FLAVOUR>(mx - mn, eps);
             rbuf[j][t] = q_fast_div(v[Q_HALF] - mn, den);
         }
         __syncthreads();
@@ -322,24 +238,14 @@ lne2d_refine_kernel(const SrcT *__restrict__ img, int Hs, int Ws, int64_t ld, in
     }
 }
 
-// strict relative parity is on unless HIPR_LNE2D_REFINE=0 (the fixed-point result alone: rtol 1e-5 + atol 5e-7);
-// HIPR_LNE2D_REFINE=2 is a diagnostic: mark only, leave the sentinels in the score map
-static int refine_mode() {
-    static const int mode = [] {
-        const char *e = getenv("HIPR_LNE2D_REFINE");
-        return (e && e[0] >= '0' && e[0] <= '2') ? e[0] - '0' : 1;
-    }();
-    return mode;
-}
-
+// mode: refine_mode("HIPR_LNE2D_REFINE"); without the refinement the fixed-point result alone holds rtol 1e-5 + atol 5e-7
 template <typename SrcT, bool BAKED>
 static int lne2d_q_launch(const SrcT *img, int Hs, int Ws, int64_t ld, int src_off, int y_begin, int H, int W,
-                          const TableQ &tab, int flavour, const unsigned long long *range, float *out,
+                          const TableQ &tab, int flavour, const unsigned long long *range, float *out, int mode,
                           cudaStream_t st) {
     // rows [y_begin, H) of the output are computed
     dim3 grid((W + Q_TW - 1) / Q_TW, (H - y_begin + Q_TH - 1) / Q_TH);
     dim3 grid_rf((W + RF_W - 1) / RF_W, (H - y_begin + RF_H - 1) / RF_H);
-    const int mode = refine_mode();
     const bool refine = mode != 0;
 #define HIPR_Q_LAUNCH(F)                                                                                                    \
     if (refine) {                                                                                                           \
@@ -383,12 +289,13 @@ int lne2d_q_rows(const void *image_dev, int Hs, int Ws, int64_t ld, int padded, 
         baked = baked && dy == kBaked2D[2 * i] && dx == kBaked2D[2 * i + 1];
     }
     const unsigned long long *rg = reinterpret_cast<const unsigned long long *>(range_dev);
+    static const int mode = refine_mode("HIPR_LNE2D_REFINE");
     if (dtype == HIPR_F64) {
-        if (baked) return lne2d_q_launch<double, true>((const double *)image_dev, Hs, Ws, ld, src_off, y_begin, y_end, W, tab, flavour, rg, out_dev, st);
-        return lne2d_q_launch<double, false>((const double *)image_dev, Hs, Ws, ld, src_off, y_begin, y_end, W, tab, flavour, rg, out_dev, st);
+        if (baked) return lne2d_q_launch<double, true>((const double *)image_dev, Hs, Ws, ld, src_off, y_begin, y_end, W, tab, flavour, rg, out_dev, mode, st);
+        return lne2d_q_launch<double, false>((const double *)image_dev, Hs, Ws, ld, src_off, y_begin, y_end, W, tab, flavour, rg, out_dev, mode, st);
     }
-    if (baked) return lne2d_q_launch<float, true>((const float *)image_dev, Hs, Ws, ld, src_off, y_begin, y_end, W, tab, flavour, rg, out_dev, st);
-    return lne2d_q_launch<float, false>((const float *)image_dev, Hs, Ws, ld, src_off, y_begin, y_end, W, tab, flavour, rg, out_dev, st);
+    if (baked) return lne2d_q_launch<float, true>((const float *)image_dev, Hs, Ws, ld, src_off, y_begin, y_end, W, tab, flavour, rg, out_dev, mode, st);
+    return lne2d_q_launch<float, false>((const float *)image_dev, Hs, Ws, ld, src_off, y_begin, y_end, W, tab, flavour, rg, out_dev, mode, st);
 }
 }  // namespace hipr
 

@@ -6,11 +6,9 @@
 // shared memory (z fastest, lanes along z: conflict-free), each thread walks TX voxels.  The
 // 792-entry offset table rides in the kernel parameter bank.  This kernel is shared-memory /
 // min-max-ALU bound (792 samples + a 72-value rank selection per voxel), not HBM bound.
-#include <cstdlib>
-#include <type_traits>
 #include "hipr_common.cuh"
 #include "lne_math.cuh"
-#include "baked_tables.cuh"
+#include "lne_fixed.cuh"
 
 namespace hipr {
 
@@ -36,13 +34,6 @@ constexpr int L3_SZ = L3_TZ + L3_P - 1;  // 42
 constexpr int l3_baked_off(int t, int li) {
     return (kBaked3D[(t * L3_P + li) * 3] * L3_SY + kBaked3D[(t * L3_P + li) * 3 + 1]) * L3_SZ +
            kBaked3D[(t * L3_P + li) * 3 + 2];
-}
-template <int I, int N, typename F>
-__device__ __forceinline__ void l3_static_for(F &&f) {
-    if constexpr (I < N) {
-        f(std::integral_constant<int, I>{});
-        l3_static_for<I + 1, N>(f);
-    }
 }
 // Lines of the pinned table that repeat an earlier line (same 11 voxels, in either order): 6 of the 72.  Their
 // min, max and centre are the earlier line's, so their value is copied instead of recomputed.
@@ -120,12 +111,12 @@ lne3d_p11t72_kernel(const T *__restrict__ vol, int Xs, int Ys, int Zs, int src_o
         const T *base = tile + (lx * L3_SY + ty) * L3_SZ + tz;
         T r[L3_T];
         if constexpr (BAKED) {
-            l3_static_for<0, L3_T>([&](auto tc) {
+            static_for<0, L3_T>([&](auto tc) {
                 constexpr int t = decltype(tc)::value;
                 constexpr int o0 = l3_baked_off(t, 0);
                 T mn = base[o0], mx = mn;
                 bool bad = (mn != mn);
-                l3_static_for<1, L3_P>([&](auto lc) {
+                static_for<1, L3_P>([&](auto lc) {
                     constexpr int off = l3_baked_off(t, decltype(lc)::value);
                     const T s = base[off];
                     mn = Num<T>::mn(mn, s);
@@ -163,41 +154,20 @@ lne3d_p11t72_kernel(const T *__restrict__ vol, int Xs, int Ys, int Zs, int src_o
 }
 
 // ---------------------------------------------------------------------------------------
-// Fixed-point variant (see lne2d_q.cu for why): the brick is mapped onto 31-bit integers with the
-// BRICK's own min/max and stored as positive-float bit patterns; min / max / differences along
-// the 72 lines are exact, so float64 channel sums keep their precision at float32 speed and no
-// NaN bookkeeping is needed (NaN samples become 0).  F2 is invariant to the affine map; F3 / ME2
-// carry their 1e-8 into q units with the global max (`maxkey`; NULL = the volume is already
-// normalised).  Baked (11, 9, 9) table only.
+// Fixed-point variant: the brick is mapped onto the 31-bit grid of lne_fixed.cuh with the BRICK's
+// own min/max; min / max / differences along the 72 lines are exact, so float64 channel sums keep
+// their precision at float32 speed and no NaN bookkeeping is needed (NaN samples become 0).  F2 is
+// invariant to the affine map; F3 / ME2 carry their 1e-8 into q units with the global max
+// (`maxkey`; NULL = the volume is already normalised).  Baked (11, 9, 9) table only.
+// Strict relative parity, as in 2-D: e_max, the largest e_t, stands in for the e of the quartile
+// lines, and a voxel whose bound exceeds Q_REFINE_THR is written as a sentinel and recomputed in
+// float64 by lne3d_refine_kernel (~2 % of a synthetic z-stack).
 // ---------------------------------------------------------------------------------------
-constexpr uint32_t L3Q_BIAS = 0x00800000u;
-constexpr double L3Q_SPAN = (double)0x7E000000u;
-// Strict relative parity, as in 2-D (csrc/lne2d_q.cu): a line value r_t = dq_t / den_t is off by at most
-// (1 + r_t) e_t, e_t = 1 / den_t in grid units; the bound is propagated through mean * (2 lq) / (uq + lq) with e_max,
-// the largest e_t, standing in for the e of the quartile lines, and a voxel whose bound exceeds L3Q_REFINE_THR is
-// written as a sentinel and recomputed in float64 by lne3d_refine_kernel (~2 % of a synthetic z-stack).
-constexpr float L3Q_REFINE_THR = 8e-6f;
-constexpr float L3Q_SENTINEL = -2.0f;
-
 // mean * (1 - qcv) over the 72 directions without the cancellation of 1 - (uq - lq) / (uq + lq)
 struct L3QResult {
     float score, mean, r17, r18, r53, r54;
     bool mark;
 };
-template <int FLAVOUR>
-__device__ __forceinline__ void l3q_factor(float lq, float uq, float &A, float &B, bool &unit, float &factor) {
-    unit = false;
-    if (FLAVOUR == HIPR_FLAVOUR_F3) {
-        A = 2.f * lq + 1e-8f;
-        B = uq + lq + 1e-8f;
-        factor = __fdiv_rn(A, B);
-    } else {                       // F2, ME2: qcv = nan_to_num((uq - lq) / (uq + lq)); 0 / 0 -> 0 -> factor 1
-        A = 2.f * lq;
-        B = uq + lq;
-        unit = (B == 0.f);
-        factor = unit ? 1.f : __fdiv_rn(A, B);
-    }
-}
 template <int FLAVOUR, bool REFINE>
 __device__ __forceinline__ L3QResult l3q_reduce(float (&r)[L3_T], float e_max) {
     L3QResult res;
@@ -208,10 +178,9 @@ __device__ __forceinline__ L3QResult l3q_reduce(float (&r)[L3_T], float e_max) {
     sort_network<float, L3_T>(r);
     const float lq = quartile_sorted<float, L3_T, 1>(r);
     const float uq = quartile_sorted<float, L3_T, 3>(r);
-    float A, B, factor;
+    float A, B;
     bool unit;
-    l3q_factor<FLAVOUR>(lq, uq, A, B, unit, factor);
-    res.score = mean * factor;
+    res.score = mean * q_factor<FLAVOUR>(lq, uq, A, B, unit);
     res.mean = mean;
     res.r17 = r[17];
     res.r18 = r[18];
@@ -221,12 +190,7 @@ __device__ __forceinline__ L3QResult l3q_reduce(float (&r)[L3_T], float e_max) {
     if (REFINE) {
         // first opinion: e_max, the largest e_t of the voxel, stands in for the e of the quartile lines
         const float d_mean = fmaf(mean, e_max, e_max);
-        if (unit) res.mark = d_mean > L3Q_REFINE_THR * mean;
-        else {
-            const float d_lq = (lq > 0.f) ? fmaf(lq, e_max, e_max) : 0.f;
-            const float d_uq = (uq > 0.f) ? fmaf(uq, e_max, e_max) : 0.f;
-            res.mark = fmaf(mean, 2.f * d_lq * B + (d_lq + d_uq) * A, d_mean * A * B) > L3Q_REFINE_THR * A * B * mean;
-        }                                    // NaN (a flat line, F2) compares false and stays NaN
+        res.mark = q_mark<false>(unit, mean, q_err(lq, e_max), q_err(uq, e_max), d_mean, A, B);
     }
     return res;
 }
@@ -265,21 +229,9 @@ lne3d_q_kernel(const SrcT *__restrict__ vol, int Xs, int Ys, int Zs, int src_off
         bmax = fmax(bmax, v);
         bmin = fmin(bmin, v);
     }
-    bmax = warp_max(bmax);
-    bmin = -warp_max(-bmin);
-    if ((threadIdx.x & 31) == 0) {
-        red[(threadIdx.x >> 5) * 2] = bmax;
-        red[(threadIdx.x >> 5) * 2 + 1] = bmin;
-    }
-    __syncthreads();
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-        bmax = fmax(bmax, red[2 * j]);
-        bmin = fmin(bmin, red[2 * j + 1]);
-    }
-    const double K = (bmax > bmin) ? L3Q_SPAN / (bmax - bmin) : 0.0;
-    const double gmax = maxkey ? fabs(double_of_key(*maxkey)) : 1.0;
-    const float eps_q = (K > 0.0) ? (float)(1e-8 * gmax * K) : 1.0f;
+    block8_minmax(bmax, bmin, red, threadIdx.x, [] { __syncthreads(); });
+    const double K = q_scale(bmax, bmin);
+    const float eps_q = q_eps(maxkey ? fabs(double_of_key(*maxkey)) : 1.0, K);
     for (int i = threadIdx.x; i < SX * L3_SY * L3_SZ; i += 256) {
         const int lz = i % L3_SZ, rest = i / L3_SZ;
         const int ly = rest % L3_SY, lx = rest / L3_SY;
@@ -288,8 +240,7 @@ lne3d_q_kernel(const SrcT *__restrict__ vol, int Xs, int Ys, int Zs, int src_off
         const int sz = min(max(z0 + lz - L3_HALF + src_off, 0), Zs - 1);
         double v = (double)vol[((int64_t)sx * Ys + sy) * Zs + sz];   // second read: L1/L2 hit
         if (v != v) v = 0.0;
-        const double qd = fmin(fmax((v - bmin) * K, 0.0), L3Q_SPAN);
-        tile[i] = __uint_as_float(__double2uint_rn(qd) + L3Q_BIAS);
+        tile[i] = q_encode(v, bmin, K);
     }
     __syncthreads();
     const int tz = threadIdx.x & 31, ty = threadIdx.x >> 5;
@@ -299,22 +250,14 @@ lne3d_q_kernel(const SrcT *__restrict__ vol, int Xs, int Ys, int Zs, int src_off
         constexpr int t = decltype(tc)::value;
         constexpr int o0 = l3_baked_off(t, 0);
         float mn = base[o0], mx = mn;
-        l3_static_for<1, L3_P>([&](auto lc) {
+        static_for<1, L3_P>([&](auto lc) {
             constexpr int off = l3_baked_off(t, decltype(lc)::value);
             const float s = base[off];
             mn = fminf(mn, s);
             mx = fmaxf(mx, s);
         });
         constexpr int oc = l3_baked_off(t, L3_HALF);
-        const float c = base[oc];
-        const float dq = __uint2float_rn(__float_as_uint(c) - __float_as_uint(mn));
-        const float rq = __uint2float_rn(__float_as_uint(mx) - __float_as_uint(mn));
-        float den;
-        if (FLAVOUR == HIPR_FLAVOUR_F2) den = rq;                         // 0/0 -> NaN on a flat line
-        else if (FLAVOUR == HIPR_FLAVOUR_F3) den = rq + eps_q;
-        else den = fmaxf(rq, eps_q);
-        inv = __fdividef(1.0f, den);
-        rv = dq * inv;
+        rv = q_line<FLAVOUR>(base[oc], mn, mx, eps_q, &inv);
     };
     if (z < Z && y < Y) {
 #pragma unroll 1
@@ -324,7 +267,7 @@ lne3d_q_kernel(const SrcT *__restrict__ vol, int Xs, int Ys, int Zs, int src_off
             const float *base = tile + (lx * L3_SY + ty) * L3_SZ + tz;
             float r[L3_T];
             float e_max = 0.f;
-            l3_static_for<0, L3_T>([&](auto tc) {
+            static_for<0, L3_T>([&](auto tc) {
                 constexpr int t = decltype(tc)::value;
                 constexpr int dup = l3_dup_of(t);
                 if constexpr (dup >= 0) {
@@ -335,7 +278,7 @@ lne3d_q_kernel(const SrcT *__restrict__ vol, int Xs, int Ys, int Zs, int src_off
                     if (REFINE) {
                         if (MODE == 0) {
                             // per-direction output: mark the value itself when (1 + r) e > thr * r
-                            if (rv > 0.f && fmaf(rv, inv, inv) > L3Q_REFINE_THR * rv) rv = L3Q_SENTINEL;
+                            if (rv > 0.f && fmaf(rv, inv, inv) > Q_REFINE_THR * rv) rv = Q_SENTINEL;
                         } else {
                             e_max = fmaxf(e_max, inv);
                         }
@@ -358,7 +301,7 @@ lne3d_q_kernel(const SrcT *__restrict__ vol, int Xs, int Ys, int Zs, int src_off
                                                    (lx * L3_TY + ty) * L3_TZ + tz};
                         continue;                       // written after the second opinion
                     }
-                    score = L3Q_SENTINEL;
+                    score = Q_SENTINEL;
                 }
                 out[v] = score;
             }
@@ -375,13 +318,13 @@ lne3d_q_kernel(const SrcT *__restrict__ vol, int Xs, int Ys, int Zs, int src_off
         const int pty = rest % L3_TY, plx = rest / L3_TY;
         const float *base = tile + (plx * L3_SY + pty) * L3_SZ + ptz;
         float e17 = 0.f, e18 = 0.f, e53 = 0.f, e54 = 0.f, d_sum = 0.f;
-        l3_static_for<0, L3_T>([&](auto tc) {
+        static_for<0, L3_T>([&](auto tc) {
             constexpr int t = decltype(tc)::value;
             if constexpr (l3_dup_of(t) < 0) {
                 float rv, inv;
                 line(base, tc, rv, inv);
                 constexpr float mult = (float)l3_mult(t);
-                d_sum += (rv > 0.f) ? mult * fmaf(rv, inv, inv) : 0.f;
+                d_sum += mult * q_err(rv, inv);
                 e17 = (rv == pd.r17) ? fmaxf(e17, inv) : e17;
                 e18 = (rv == pd.r18) ? fmaxf(e18, inv) : e18;
                 e53 = (rv == pd.r53) ? fmaxf(e53, inv) : e53;
@@ -389,18 +332,16 @@ lne3d_q_kernel(const SrcT *__restrict__ vol, int Xs, int Ys, int Zs, int src_off
             }
         });
         const float lq = quartile_pair<float, 1>(pd.r17, pd.r18), uq = quartile_pair<float, 3>(pd.r53, pd.r54);
-        float A, B, factor;
+        float A, B;
         bool unit;
-        l3q_factor<FLAVOUR>(lq, uq, A, B, unit, factor);
+        q_factor<FLAVOUR>(lq, uq, A, B, unit);
         const float d_mean = d_sum * (1.0f / L3_T);
         // |d lq| <= 0.25 (1 + r17) e17 + 0.75 (1 + r18) e18, |d uq| <= 0.75 (1 + r53) e53 + 0.25 (1 + r54) e54
-        const float d_lq = 0.25f * ((pd.r17 > 0.f) ? fmaf(pd.r17, e17, e17) : 0.f) + 0.75f * ((pd.r18 > 0.f) ? fmaf(pd.r18, e18, e18) : 0.f);
-        const float d_uq = 0.75f * ((pd.r53 > 0.f) ? fmaf(pd.r53, e53, e53) : 0.f) + 0.25f * ((pd.r54 > 0.f) ? fmaf(pd.r54, e54, e54) : 0.f);
-        bool mark;
-        if (unit) mark = d_mean > L3Q_REFINE_THR * pd.mean;
-        else mark = fmaf(pd.mean, 2.f * d_lq * B + (d_lq + d_uq) * A, d_mean * A * B) > L3Q_REFINE_THR * A * B * pd.mean;
+        const float d_lq = 0.25f * q_err(pd.r17, e17) + 0.75f * q_err(pd.r18, e18);
+        const float d_uq = 0.75f * q_err(pd.r53, e53) + 0.25f * q_err(pd.r54, e54);
+        const bool mark = q_mark<false>(unit, pd.mean, d_lq, d_uq, d_mean, A, B);
         const int64_t v = ((int64_t)(x0 + plx) * Y + (y0 + pty)) * Z + (z0 + ptz);
-        out[v] = mark ? L3Q_SENTINEL : pd.score;
+        out[v] = mark ? Q_SENTINEL : pd.score;
     }
 }
 
@@ -434,9 +375,7 @@ __device__ __forceinline__ double l3_line_value_f64(const SrcT *__restrict__ vol
         mn = fmin(mn, v[li]);
         mx = fmax(mx, v[li]);
     }
-    double den = mx - mn;
-    if (FLAVOUR == HIPR_FLAVOUR_F3) den += eps;
-    else if (FLAVOUR != HIPR_FLAVOUR_F2) den = fmax(den, eps);
+    const double den = q_den<FLAVOUR>(mx - mn, eps);
     return (v[L3_HALF] - mn) / den;
 }
 
@@ -462,7 +401,7 @@ lne3d_refine_kernel(const SrcT *__restrict__ vol, int Xs, int Ys, int Zs, int sr
     if (threadIdx.x == 0) n_marked = 0;
     __syncthreads();
     for (int i = threadIdx.x; i < RF3_SPAN; i += RF3_THREADS)
-        if (v0 + i < nvox && out[v0 + i] == L3Q_SENTINEL) marked[atomicAdd(&n_marked, 1u)] = (unsigned short)i;
+        if (v0 + i < nvox && out[v0 + i] == Q_SENTINEL) marked[atomicAdd(&n_marked, 1u)] = (unsigned short)i;
     __syncthreads();
     const int n = (int)n_marked;
     if (n == 0) return;
@@ -530,7 +469,7 @@ lne3d_refine_dirs_kernel(const SrcT *__restrict__ vol, int Xs, int Ys, int Zs, i
     const int64_t n = (int64_t)X * Y * Z * L3_T;
     const double eps = 1e-8 * (maxkey ? fabs(double_of_key(*maxkey)) : 1.0);
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-        if (out[i] != L3Q_SENTINEL) continue;
+        if (out[i] != Q_SENTINEL) continue;
         const int t = (int)(i % L3_T);
         const int64_t v = i / L3_T;
         const int z = (int)(v % Z);
@@ -663,23 +602,14 @@ static int lne3d_dispatch(const T *vol, int Xs, int Ys, int Zs, int padded, int 
     return after_launch();
 }
 
-// strict relative parity is on unless HIPR_LNE3D_REFINE=0 (2 = diagnostic: mark only)
-static int refine3d_mode() {
-    static const int mode = [] {
-        const char *e = getenv("HIPR_LNE3D_REFINE");
-        return (e && e[0] >= '0' && e[0] <= '2') ? e[0] - '0' : 1;
-    }();
-    return mode;
-}
-
+// refine: refine_mode("HIPR_LNE3D_REFINE")
 template <typename SrcT, int FLAVOUR, int MODE>
 static int launch_q3d(const SrcT *vol, int Xs, int Ys, int Zs, int src_off, int X, int Y, int Z,
-                      const unsigned long long *maxkey, float *out, cudaStream_t st) {
+                      const unsigned long long *maxkey, float *out, int refine, cudaStream_t st) {
     constexpr int TX = 8;
     constexpr int SX = TX + L3_P - 1;
     const size_t smem = (size_t)SX * L3_SY * L3_SZ * sizeof(float);
-    const int mode = refine3d_mode();
-    auto kern = mode ? lne3d_q_kernel<SrcT, FLAVOUR, MODE, TX, true> : lne3d_q_kernel<SrcT, FLAVOUR, MODE, TX, false>;
+    auto kern = refine ? lne3d_q_kernel<SrcT, FLAVOUR, MODE, TX, true> : lne3d_q_kernel<SrcT, FLAVOUR, MODE, TX, false>;
     static std::atomic<uint64_t> attr_done{0};
     if (first_use_on_device(attr_done)) {
         HIPR_CUDA(cudaFuncSetAttribute(lne3d_q_kernel<SrcT, FLAVOUR, MODE, TX, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -690,7 +620,7 @@ static int launch_q3d(const SrcT *vol, int Xs, int Ys, int Zs, int src_off, int 
     dim3 grid((unsigned)(nzb * nyb), (unsigned)nxb);
     kern<<<grid, 256, smem, st>>>(vol, Xs, Ys, Zs, src_off, X, Y, Z, maxkey, out);
     int e = after_launch();
-    if (e || mode != 1) return e;
+    if (e || refine != 1) return e;
     const int64_t nvox = (int64_t)X * Y * Z;
     if (MODE == 0) {
         lne3d_refine_dirs_kernel<SrcT><<<sm_count() * 8, 256, 0, st>>>(vol, Xs, Ys, Zs, src_off, X, Y, Z, maxkey, out);
@@ -704,16 +634,16 @@ static int launch_q3d(const SrcT *vol, int Xs, int Ys, int Zs, int src_off, int 
 
 template <typename SrcT>
 static int lne3d_q_dispatch(const SrcT *vol, int Xs, int Ys, int Zs, int padded, int flavour, int mode,
-                            const unsigned long long *maxkey, float *out, cudaStream_t st) {
+                            const unsigned long long *maxkey, float *out, int refine, cudaStream_t st) {
     const int P = L3_P;
     const int X = padded ? Xs - (P - 1) : Xs, Y = padded ? Ys - (P - 1) : Ys, Z = padded ? Zs - (P - 1) : Zs;
     const int src_off = padded ? L3_HALF : 0;
     if (X < 1 || Y < 1 || Z < 1) return HIPR_E_PATCH;
-    if (mode == 0) return launch_q3d<SrcT, HIPR_FLAVOUR_ME2, 0>(vol, Xs, Ys, Zs, src_off, X, Y, Z, maxkey, out, st);
+    if (mode == 0) return launch_q3d<SrcT, HIPR_FLAVOUR_ME2, 0>(vol, Xs, Ys, Zs, src_off, X, Y, Z, maxkey, out, refine, st);
     switch (flavour) {
-        case HIPR_FLAVOUR_F2: return launch_q3d<SrcT, HIPR_FLAVOUR_F2, 1>(vol, Xs, Ys, Zs, src_off, X, Y, Z, maxkey, out, st);
-        case HIPR_FLAVOUR_F3: return launch_q3d<SrcT, HIPR_FLAVOUR_F3, 1>(vol, Xs, Ys, Zs, src_off, X, Y, Z, maxkey, out, st);
-        case HIPR_FLAVOUR_ME2: return launch_q3d<SrcT, HIPR_FLAVOUR_ME2, 1>(vol, Xs, Ys, Zs, src_off, X, Y, Z, maxkey, out, st);
+        case HIPR_FLAVOUR_F2: return launch_q3d<SrcT, HIPR_FLAVOUR_F2, 1>(vol, Xs, Ys, Zs, src_off, X, Y, Z, maxkey, out, refine, st);
+        case HIPR_FLAVOUR_F3: return launch_q3d<SrcT, HIPR_FLAVOUR_F3, 1>(vol, Xs, Ys, Zs, src_off, X, Y, Z, maxkey, out, refine, st);
+        case HIPR_FLAVOUR_ME2: return launch_q3d<SrcT, HIPR_FLAVOUR_ME2, 1>(vol, Xs, Ys, Zs, src_off, X, Y, Z, maxkey, out, refine, st);
         default: return HIPR_E_FLAVOUR;
     }
 }
@@ -733,11 +663,12 @@ extern "C" int hipr_lne3d_q(const void *volume_dev, int Xs, int Ys, int Zs, int 
         if (table_host[i] != kBaked3D[i]) return HIPR_E_UNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
     const unsigned long long *mk = reinterpret_cast<const unsigned long long *>(maxkey_dev);
+    static const int refine = refine_mode("HIPR_LNE3D_REFINE");
     if (dtype == HIPR_F64)
         return lne3d_q_dispatch<double>((const double *)volume_dev, Xs, Ys, Zs, padded, flavour, dirs_only ? 0 : 1, mk,
-                                        out_dev, st);
+                                        out_dev, refine, st);
     return lne3d_q_dispatch<float>((const float *)volume_dev, Xs, Ys, Zs, padded, flavour, dirs_only ? 0 : 1, mk,
-                                   out_dev, st);
+                                   out_dev, refine, st);
 }
 
 extern "C" int hipr_line_profile_3d(const void *volume_padded_dev, int Xp, int Yp, int Zp, int dtype, int patch_size,
