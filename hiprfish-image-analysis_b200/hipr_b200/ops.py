@@ -673,8 +673,10 @@ def cell_spectra_accumulate(cube, labels, max_label, sums=None, counts=None):
     labels = _dev(labels, "labels", (torch.int32, torch.int64))
     Cn = cube.shape[-1]
     npix = labels.numel()
-    if cube.numel() != npix * Cn:
-        raise ValueError("cube %s and labels %s do not match" % (tuple(cube.shape), tuple(labels.shape)))
+    # pixel p of the label image pairs with cube row p: a transposed label image has the right size, the wrong pairing
+    if tuple(cube.shape[:-1]) != tuple(labels.shape):
+        raise ValueError("cube %s and labels %s do not match: the cube must be labels.shape + (C,)"
+                         % (tuple(cube.shape), tuple(labels.shape)))
     max_label = int(max_label)
     if (sums is None) != (counts is None):
         raise ValueError("pass both sums and counts (to keep accumulating) or neither")
@@ -1212,8 +1214,9 @@ def cell_spectra_host(cube, labels):
         raise TypeError("labels must be int32 or int64, got %s" % labels.dtype)
     Cn = cube.shape[-1]
     npix = labels.size
-    if cube.size != npix * Cn:
-        raise ValueError("cube and labels do not match")
+    if cube.shape[:-1] != labels.shape:
+        raise ValueError("cube %s and labels %s do not match: the cube must be labels.shape + (C,)"
+                         % (cube.shape, labels.shape))
     cap = 4096
 
     def alloc(k):
