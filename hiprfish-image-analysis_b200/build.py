@@ -7,7 +7,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 LIB = os.path.join(HERE, "libhipr_b200.so")
-SOURCES = ["chansum.cu", "register.cu", "nlm2d.cu", "nlm3d.cu", "lne2d.cu", "lne2d_q.cu", "fused2d.cu", "pipeline2d.cu", "mosaic_p2p.cu", "lne3d.cu", "cell_spectra.cu", "cell_geometry.cu", "kmeans1d.cu", "xcorr2d.cu", "label.cu", "watershed.cu", "host_api.cu"]
+SOURCES = ["chansum.cu", "register.cu", "nlm2d.cu", "nlm3d.cu", "lne2d.cu", "lne2d_q.cu", "fused2d.cu", "pipeline2d.cu", "mosaic_p2p.cu", "lne3d.cu", "cell_spectra.cu", "cell_geometry.cu", "kmeans1d.cu", "xcorr2d.cu", "label.cu", "watershed.cu", "morphology.cu", "host_api.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-O2", "--expt-relaxed-constexpr"]
 

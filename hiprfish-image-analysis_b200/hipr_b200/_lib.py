@@ -50,6 +50,9 @@ _SIGNATURES = {
     "hipr_label": (_i, [_vp, _i, _i, _i, _i, _i, _i, _i, _vp, _i64, _vp, _i, _vp, _vp]),
     "hipr_label_counts": (_i, [_vp, _i, _i, _i, _i, _i, _i, _i64, _vp, _vp, _vp]),
     "hipr_label_clear": (_i, [_vp, _i, _vp, _i64, _vp, _i64, _vp, _vp]),
+    "hipr_morphology_workspace_bytes": (_i64, [_i, _i, _i, _i, _i]),
+    "hipr_binary_morphology": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _i, _i, _i, _i, _i, _vp, _i64, _vp, _vp]),
+    "hipr_morphology_runs": (_i, [_vp, _i, _i, _i, _vp, _i]),
     "hipr_watershed_workspace_bytes": (_i64, [_i, _i, _i, _i, _i, _i]),
     "hipr_watershed": (_i, [_vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _i, _vp, _i64, _vp, _vp, _vp]),
     "hipr_kmeans1d_workspace_bytes": (_i64, []),

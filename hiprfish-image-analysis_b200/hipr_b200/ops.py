@@ -13,7 +13,8 @@ Reference blocks replaced (paths relative to the reference repository):
   lne3d_dirs        bio/neighbor.pyx:186-263
   lne3d             bio/neighbor.pyx + bio/hiprfish_imaging_biofilm_analysis.py:812-817, 905-917, 1114-1125
   cell_spectra      syn/...measurement.py:167-172
-  label, remove_small_objects, binary_fill_holes, clear_border, relabel_sequential, watershed
+  label, remove_small_objects, binary_fill_holes, clear_border, relabel_sequential, watershed,
+  binary_erosion, binary_dilation, binary_opening, binary_closing
                     the segmentation back end, syn/...measurement.py:125-158, eco/...measurement.py:44-127,
                     bio/...analysis.py:367-419, 463-501
 """
@@ -1029,6 +1030,110 @@ def watershed(image, markers, connectivity=1, mask=None):
     if st:
         raise HiprError("watershed: phase %d did not converge within its round cap" % st)
     return out
+
+
+# ---------------------------------------------------------------------------------------------
+# binary morphology (K12, csrc/morphology.cu)
+# ---------------------------------------------------------------------------------------------
+
+MORPHOLOGY_MAX_EXTENT = 31     # HIPR_MORPH_MAX_EXTENT: disk(15), ball(15)
+MORPHOLOGY_MAX_RUNS = 1000     # HIPR_MORPH_MAX_RUNS
+
+
+def _structure(structure, ndim):
+    """-> the structure as a C-contiguous uint8 numpy array of `ndim` axes (1 = member), checked as scipy checks it
+    plus this kernel's limits.  None: generate_binary_structure(ndim, 1), built here (the product imports no scipy)."""
+    if structure is None:
+        idx = np.indices((3,) * ndim)
+        return np.ascontiguousarray((np.abs(idx - 1).sum(axis=0) <= 1).astype(np.uint8))
+    s = np.asarray(structure) != 0
+    if s.ndim != ndim:
+        raise RuntimeError("structure and input must have same dimensionality")
+    if any(n % 2 == 0 for n in s.shape):
+        raise ValueError("structure extents must be odd, got shape %s (an even extent needs scipy's origin shift, "
+                         "which is not offered)" % (s.shape,))
+    if max(s.shape) > MORPHOLOGY_MAX_EXTENT:
+        raise ValueError("structure extents must be at most %d, got shape %s" % (MORPHOLOGY_MAX_EXTENT, s.shape))
+    s = np.ascontiguousarray(s.astype(np.uint8))
+    if _structure_runs(s).shape[0] > MORPHOLOGY_MAX_RUNS:
+        raise ValueError("structure has more than %d runs of members along its last axis (the kernel's limit)"
+                         % MORPHOLOGY_MAX_RUNS)
+    return s
+
+
+def _structure_runs(s):
+    """The kernel's run table of a checked structure: (n, 4) int32 rows (d0, d1, first d2, last d2) of offsets from the
+    centre, one per maximal run of members along the last axis; a 2-D structure has d0 = 0."""
+    s3 = s.reshape((1,) * (3 - s.ndim) + s.shape)
+    ptr = s3.ctypes.data_as(C.c_void_p)
+    n = lib().hipr_morphology_runs(ptr, *s3.shape, None, 0)
+    check(min(n, 0), "structure")
+    runs = np.empty((n, 4), dtype=np.int32)
+    check(min(lib().hipr_morphology_runs(ptr, *s3.shape, runs.ctypes.data_as(C.c_void_p), n), 0), "structure")
+    return runs
+
+
+def _iterations(iterations):
+    if isinstance(iterations, bool) or not isinstance(iterations, (int, np.integer)):
+        raise TypeError("iterations must be an integer")
+    if iterations < 1:
+        raise ValueError("iterations must be >= 1 (scipy's iterations < 1, repeat until nothing changes, is not "
+                         "offered), got %d" % iterations)
+    return int(iterations)
+
+
+def _morphology(mask, structure, iterations, border_value, dilate):
+    raw, _, dims = _label_input(mask, "mask", (torch.bool, torch.uint8))
+    s = _structure(structure, dims[0])
+    iterations = _iterations(iterations)
+    ws = lib().hipr_morphology_workspace_bytes(*dims, iterations)
+    if ws < 0:
+        check(int(ws), "binary morphology (an image of 2^31 pixels or more)")
+    dev = raw.device
+    work = torch.empty(int(ws), dtype=torch.uint8, device=dev)
+    out = torch.empty(raw.shape, dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        check(lib().hipr_binary_morphology(C.c_void_p(raw.data_ptr()), *dims, s.ctypes.data_as(C.c_void_p),
+                                           *(s.shape + (1,) * (3 - s.ndim)), int(dilate), 1 if border_value else 0,
+                                           iterations, C.c_void_p(work.data_ptr()), int(ws),
+                                           C.c_void_p(out.data_ptr()), _stream()),
+              "binary_dilation" if dilate else "binary_erosion")
+    return out.view(torch.bool)
+
+
+def binary_erosion(mask, structure=None, iterations=1, border_value=0):
+    """scipy.ndimage.binary_erosion(mask, structure, iterations, border_value=border_value) on the device, bit for bit.
+
+    mask: bool / uint8 CUDA tensor, 2-D (H, W) or 3-D (X, Y, Z), non-zero is True.  structure: None (the cross,
+    generate_binary_structure(ndim, 1)) or a host array-like (numpy, CPU tensor) of ndim axes, non-zero is a member;
+    every extent odd and at most 31.  out[p] = AND over members o of mask[p + o], with every pixel outside the image
+    equal to border_value (non-zero counts as 1), repeated `iterations` (>= 1) times.  -> a new bool tensor.  One launch
+    per pass; no host synchronisation and no device-to-host copy."""
+    return _morphology(mask, structure, iterations, border_value, False)
+
+
+def binary_dilation(mask, structure=None, iterations=1, border_value=0):
+    """scipy.ndimage.binary_dilation(mask, structure, iterations, border_value=border_value) on the device, bit for
+    bit: out[p] = OR over members o of mask[p - o] (the structure reflected), repeated `iterations` times.  Arguments,
+    result and cost as binary_erosion; no host synchronisation and no device-to-host copy."""
+    return _morphology(mask, structure, iterations, border_value, True)
+
+
+def binary_opening(mask, structure=None, iterations=1, border_value=0):
+    """scipy.ndimage.binary_opening(mask, structure, iterations, border_value=border_value) on the device, bit for bit:
+    binary_erosion `iterations` times, then binary_dilation `iterations` times, both with border_value.  2 x iterations
+    launches; no host synchronisation and no device-to-host copy."""
+    return binary_dilation(binary_erosion(mask, structure, iterations, border_value), structure, iterations,
+                           border_value)
+
+
+def binary_closing(mask, structure=None, iterations=1, border_value=0):
+    """scipy.ndimage.binary_closing(mask, structure, iterations, border_value=border_value) on the device, bit for bit:
+    binary_dilation `iterations` times, then binary_erosion `iterations` times, both with border_value (so with the
+    default 0 the closing erodes from the image edge, as scipy's does).  2 x iterations launches; no host
+    synchronisation and no device-to-host copy."""
+    return binary_erosion(binary_dilation(mask, structure, iterations, border_value), structure, iterations,
+                          border_value)
 
 
 # ---------------------------------------------------------------------------------------------

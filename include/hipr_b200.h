@@ -378,6 +378,37 @@ int hipr_label_counts(const void *labels_dev, int label_bytes, int ndim, int d0,
 int hipr_label_clear(const void *image_dev, int dtype, const int32_t *labels_dev, int64_t npix,
                      const int32_t *flagged_dev, int64_t fill, void *out_dev, void *stream);
 
+/* ---- binary morphology (csrc/morphology.cu) ---------------------------------------------------------------------
+ * The opening of the k-means mask before remove_small_objects / binary_fill_holes (syn/..._measurement.py:125-158,
+ * bio/..._analysis.py:367-419, 463-501) and the erosion that makes the watershed seeds (eco/..._measurement.py:44-127).
+ * hipr_binary_morphology: scipy.ndimage.binary_erosion(mask, structure, iterations, border_value=border_value)
+ *   (dilate == 0) or scipy.ndimage.binary_dilation(...) (dilate != 0), origin 0, bit for bit.  Erosion:
+ *   out[p] = AND over members o of in[p + o]; dilation: out[p] = OR over members o of in[p - o]; every pixel outside
+ *   the image is border_value (non-zero = 1) in every pass.  An empty structure erodes to all 1 and dilates to all 0.
+ *   mask_dev       C-order (d0, d1) (ndim 2) or (d0, d1, d2) (ndim 3) uint8, non-zero = 1
+ *   structure_host C-order (s0, s1) (ndim 2) or (s0, s1, s2) (ndim 3) uint8 in HOST memory, non-zero = member; every
+ *                  extent odd and <= HIPR_MORPH_MAX_EXTENT, at most HIPR_MORPH_MAX_RUNS runs (hipr_morphology_runs);
+ *                  read during the call and passed to the kernel by value
+ *   iterations     >= 1 passes, each a launch; the passes alternate between out_dev and the workspace, the last
+ *                  writes out_dev
+ *   out_dev        same shape, uint8 0 / 1; must not overlap mask_dev
+ *   workspace      hipr_morphology_workspace_bytes(ndim, d0, d1, d2, iterations) bytes (0 for one pass; negative:
+ *                  HIPR_E_RANGE when the image has 2^31 pixels or more); what it holds before the call does not matter
+ *   No host synchronisation, no copy.  binary_opening is erosion then dilation, binary_closing dilation then erosion,
+ *   each with the same iterations and border_value: two calls.
+ * hipr_morphology_runs: the run table behind the kernel, host only.  Writes up to `capacity` runs of a (s0, s1, s2)
+ *   structure (pass s0 = 1 for a 2-D one) into runs_out (capacity, 4) int32: (d0, d1, first d2, last d2), offsets from
+ *   the centre, one per maximal run of members along the last axis, in C order; returns the number of runs (which may
+ *   exceed capacity), HIPR_E_ARG for an even or non-positive extent, HIPR_E_RANGE for an extent above the limit.
+ */
+#define HIPR_MORPH_MAX_EXTENT 31
+#define HIPR_MORPH_MAX_RUNS   1000  /* the run table travels in the 4 KB kernel parameter space; a full 31^3 cube has 961 */
+int64_t hipr_morphology_workspace_bytes(int ndim, int d0, int d1, int d2, int iterations);
+int hipr_binary_morphology(const uint8_t *mask_dev, int ndim, int d0, int d1, int d2, const uint8_t *structure_host,
+                           int s0, int s1, int s2, int dilate, int border_value, int iterations, void *workspace_dev,
+                           int64_t workspace_bytes, uint8_t *out_dev, void *stream);
+int hipr_morphology_runs(const uint8_t *structure_host, int s0, int s1, int s2, int32_t *runs_out, int capacity);
+
 /* ---- marker watershed (csrc/watershed.cu) -----------------------------------------------------------------------
  * skimage.segmentation.watershed(image, markers, connectivity=connectivity, mask=mask) (no compactness, no watershed
  * line), the last step of the segmentation back end: syn/..._measurement.py:125-158, eco/..._measurement.py:44-127,
