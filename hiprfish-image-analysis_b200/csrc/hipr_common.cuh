@@ -49,6 +49,25 @@ inline int after_launch() {
         if (_e != cudaSuccess) return (int)_e;            \
     } while (0)
 
+// The segmentation entry points take (ndim, d0, d1, d2): a 2-D image (H, W) is the volume (1, H, W).  HIPR_E_ARG for
+// another ndim or an empty axis, HIPR_E_RANGE at 2^31 pixels or more (their kernels index pixels with int32).
+inline int volume_xyz(int ndim, int d0, int d1, int d2, int &X, int &Y, int &Z) {
+    if (ndim == 2) { X = 1; Y = d0; Z = d1; }
+    else if (ndim == 3) { X = d0; Y = d1; Z = d2; }
+    else return HIPR_E_ARG;
+    if (X < 1 || Y < 1 || Z < 1) return HIPR_E_ARG;
+    return (int64_t)X * Y * Z > 0x7fffffffLL ? HIPR_E_RANGE : HIPR_OK;
+}
+
+// The smallest power of two >= n, capped at cap (a tile edge).
+inline int pow2_at_least(int n, int cap) {
+    int p = 1;
+    while (p < n && p < cap) p <<= 1;
+    return p;
+}
+
+inline int64_t align256(int64_t b) { return (b + 255) / 256 * 256; }
+
 // ---------------------------------------------------------------------------------------
 // Order-preserving 64-bit key of a double, so a global max is one atomicMax on uint64.
 // key(a) < key(b)  <=>  a < b for all non-NaN doubles; key 0 is below every real number.

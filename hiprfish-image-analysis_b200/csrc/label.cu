@@ -302,19 +302,6 @@ label_clear_kernel(const T *__restrict__ img, const int *__restrict__ labels, in
         out[p] = flagged[labels[p]] ? fill : img[p];
 }
 
-static bool dims_of(int ndim, int d0, int d1, int d2, Dims &d) {
-    if (ndim == 2) { d.X = 1; d.Y = d0; d.Z = d1; }
-    else if (ndim == 3) { d.X = d0; d.Y = d1; d.Z = d2; }
-    else return false;
-    return d.X >= 1 && d.Y >= 1 && d.Z >= 1;
-}
-
-static int pow2_at_least(int n, int cap) {
-    int p = 1;
-    while (p < n && p < cap) p <<= 1;
-    return p;
-}
-
 // Tiles of up to 512 pixels, 32 along Z where the image allows it (coalesced rows); a volume splits the rest
 // evenly between X and Y (4 x 4 x 32), an image takes 16 rows.
 static void choose_tile(Dims &d) {
@@ -326,17 +313,15 @@ static void choose_tile(Dims &d) {
     d.NTZ = (d.Z + d.TZ - 1) / d.TZ;
 }
 
-static int64_t align256(int64_t b) { return (b + 255) / 256 * 256; }
-
 }  // namespace hipr
 
 using namespace hipr;
 
 extern "C" int64_t hipr_label_workspace_bytes(int ndim, int d0, int d1, int d2) {
     Dims d;
-    if (!dims_of(ndim, d0, d1, d2, d)) return HIPR_E_ARG;
+    const int e = volume_xyz(ndim, d0, d1, d2, d.X, d.Y, d.Z);
+    if (e) return e;
     const int64_t npix = (int64_t)d.X * d.Y * d.Z;
-    if (npix > 0x7fffffffLL) return HIPR_E_RANGE;
     return align256(npix * 4) + align256((npix + LB_CHUNK - 1) / LB_CHUNK * 4);
 }
 
@@ -344,7 +329,8 @@ extern "C" int hipr_label(const void *image_dev, int dtype, int invert, int ndim
                           int connectivity, void *workspace_dev, int64_t workspace_bytes, void *labels_out,
                           int label_bytes, int64_t *n_dev, void *stream) {
     Dims d;
-    if (!image_dev || !workspace_dev || !labels_out || !dims_of(ndim, d0, d1, d2, d)) return HIPR_E_ARG;
+    if (!image_dev || !workspace_dev || !labels_out || volume_xyz(ndim, d0, d1, d2, d.X, d.Y, d.Z) == HIPR_E_ARG)
+        return HIPR_E_ARG;
     if (connectivity < 1 || connectivity > ndim) return HIPR_E_ARG;
     if (dtype != HIPR_U8 && dtype != HIPR_I32 && dtype != HIPR_I64) return HIPR_E_DTYPE;
     if (label_bytes != 4 && label_bytes != 8) return HIPR_E_DTYPE;
@@ -389,10 +375,11 @@ extern "C" int hipr_label_counts(const void *labels_dev, int label_bytes, int nd
                                  int border, int64_t max_label, int32_t *counts_dev, int32_t *overflow_dev,
                                  void *stream) {
     Dims d;
-    if (!labels_dev || !counts_dev || max_label < 0 || !dims_of(ndim, d0, d1, d2, d)) return HIPR_E_ARG;
+    const int vol = volume_xyz(ndim, d0, d1, d2, d.X, d.Y, d.Z);
+    if (!labels_dev || !counts_dev || max_label < 0 || vol == HIPR_E_ARG) return HIPR_E_ARG;
     if (label_bytes != 4 && label_bytes != 8) return HIPR_E_DTYPE;
+    if (vol) return vol;
     const int64_t npix = (int64_t)d.X * d.Y * d.Z;
-    if (npix > 0x7fffffffLL) return HIPR_E_RANGE;
     cudaStream_t st = (cudaStream_t)stream;
     HIPR_CUDA(cudaMemsetAsync(counts_dev, 0, (size_t)(max_label + 1) * sizeof(int32_t), st));
     if (overflow_dev) HIPR_CUDA(cudaMemsetAsync(overflow_dev, 0, sizeof(int32_t), st));

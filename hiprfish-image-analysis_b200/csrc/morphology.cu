@@ -107,19 +107,6 @@ morphology_kernel(const uint8_t *__restrict__ in, uint8_t *__restrict__ out, con
     }
 }
 
-static bool morph_dims(int ndim, int d0, int d1, int d2, int &X, int &Y, int &Z) {
-    if (ndim == 2) { X = 1; Y = d0; Z = d1; }
-    else if (ndim == 3) { X = d0; Y = d1; Z = d2; }
-    else return false;
-    return X >= 1 && Y >= 1 && Z >= 1;
-}
-
-static int pow2_at_least(int n, int cap) {
-    int p = 1;
-    while (p < n && p < cap) p <<= 1;
-    return p;
-}
-
 static int stage_words(const MorphArgs &a) {
     return (a.TX + 2 * a.rx) * (a.TY + 2 * a.ry) * (a.TW + 2) + 1 + a.TX * a.TY * a.TW;
 }
@@ -169,10 +156,10 @@ extern "C" int hipr_morphology_runs(const uint8_t *structure_host, int s0, int s
 
 extern "C" int64_t hipr_morphology_workspace_bytes(int ndim, int d0, int d1, int d2, int iterations) {
     int X, Y, Z;
-    if (!morph_dims(ndim, d0, d1, d2, X, Y, Z) || iterations < 1) return HIPR_E_ARG;
-    const int64_t npix = (int64_t)X * Y * Z;
-    if (npix > 0x7fffffffLL) return HIPR_E_RANGE;
-    return iterations > 1 ? (npix + 255) / 256 * 256 : 0;
+    const int e = volume_xyz(ndim, d0, d1, d2, X, Y, Z);
+    if (e == HIPR_E_ARG || iterations < 1) return HIPR_E_ARG;
+    if (e) return e;
+    return iterations > 1 ? align256((int64_t)X * Y * Z) : 0;
 }
 
 extern "C" int hipr_binary_morphology(const uint8_t *mask_dev, int ndim, int d0, int d1, int d2,
@@ -180,7 +167,7 @@ extern "C" int hipr_binary_morphology(const uint8_t *mask_dev, int ndim, int d0,
                                       int border_value, int iterations, void *workspace_dev, int64_t workspace_bytes,
                                       uint8_t *out_dev, void *stream) {
     MorphArgs a;
-    if (!mask_dev || !out_dev || !morph_dims(ndim, d0, d1, d2, a.X, a.Y, a.Z)) return HIPR_E_ARG;
+    if (!mask_dev || !out_dev || volume_xyz(ndim, d0, d1, d2, a.X, a.Y, a.Z) == HIPR_E_ARG) return HIPR_E_ARG;
     if (ndim == 2) { s2 = s1; s1 = s0; s0 = 1; }
     const int64_t need = hipr_morphology_workspace_bytes(ndim, d0, d1, d2, iterations);
     if (need < 0) return (int)need;

@@ -280,16 +280,14 @@ watershed_kernel(const V *__restrict__ img, const MT *__restrict__ markers, cons
     }
 }
 
-static bool ws_geom(int ndim, int d0, int d1, int d2, int connectivity, WsGeom &g) {
-    if (ndim == 2) { g.X = 1; g.Y = d0; g.Z = d1; }
-    else if (ndim == 3) { g.X = d0; g.Y = d1; g.Z = d2; }
-    else return false;
-    if (g.X < 1 || g.Y < 1 || g.Z < 1 || connectivity < 1 || connectivity > ndim) return false;
-    auto edge = [](int n, int cap) { int p = 1; while (p < n && p < cap) p <<= 1; return p; };
+// HIPR_E_ARG for a bad shape or connectivity, else volume_xyz's HIPR_E_RANGE / HIPR_OK with g filled in.
+static int ws_geom(int ndim, int d0, int d1, int d2, int connectivity, WsGeom &g) {
+    const int vol = volume_xyz(ndim, d0, d1, d2, g.X, g.Y, g.Z);
+    if (vol == HIPR_E_ARG || connectivity < 1 || connectivity > ndim) return HIPR_E_ARG;
     const int e = ndim == 2 ? WS_EDGE2 : WS_EDGE3;
-    g.TX = ndim == 2 ? 1 : edge(g.X, e);
-    g.TY = edge(g.Y, e);
-    g.TZ = edge(g.Z, e);
+    g.TX = ndim == 2 ? 1 : pow2_at_least(g.X, e);
+    g.TY = pow2_at_least(g.Y, e);
+    g.TZ = pow2_at_least(g.Z, e);
     g.NTX = (g.X + g.TX - 1) / g.TX;
     g.NTY = (g.Y + g.TY - 1) / g.TY;
     g.NTZ = (g.Z + g.TZ - 1) / g.TZ;
@@ -308,10 +306,8 @@ static bool ws_geom(int ndim, int d0, int d1, int d2, int connectivity, WsGeom &
             }
     g.npix = (int64_t)g.X * g.Y * g.Z;
     g.cap = g.npix + 1;
-    return true;
+    return vol;
 }
-
-static int64_t ws_align(int64_t b) { return (b + 255) / 256 * 256; }
 
 }  // namespace hipr
 
@@ -321,10 +317,10 @@ extern "C" int64_t hipr_watershed_workspace_bytes(int ndim, int d0, int d1, int 
     if (image_dtype != HIPR_F32 && image_dtype != HIPR_F64) return HIPR_E_DTYPE;
     if (label_bytes != 4 && label_bytes != 8) return HIPR_E_DTYPE;
     WsGeom g;
-    if (!ws_geom(ndim, d0, d1, d2, 1, g)) return HIPR_E_ARG;
-    if (g.npix > 0x7fffffffLL) return HIPR_E_RANGE;
+    const int e = ws_geom(ndim, d0, d1, d2, 1, g);
+    if (e) return e;
     const int64_t ntiles = (int64_t)g.NTX * g.NTY * g.NTZ;
-    return WS_CTRL_BYTES + ws_align(6 * ntiles * 4) + ws_align(g.npix * 8) + 2 * ws_align(g.npix * 4);
+    return WS_CTRL_BYTES + align256(6 * ntiles * 4) + align256(g.npix * 8) + 2 * align256(g.npix * 4);
 }
 
 template <typename V, typename MT, typename OutT>
@@ -343,10 +339,10 @@ static int ws_launch(const void *image, const void *markers, const uint8_t *mask
     if (grid > ntiles) grid = ntiles;
     WsCtrl *ctrl = (WsCtrl *)ws;
     unsigned int *dirty = (unsigned int *)(ws + WS_CTRL_BYTES);
-    char *p = ws + WS_CTRL_BYTES + ws_align(6 * ntiles * 4);
+    char *p = ws + WS_CTRL_BYTES + align256(6 * ntiles * 4);
     uint64_t *lw = (uint64_t *)p;
-    uint32_t *dw = (uint32_t *)(p + ws_align(g.npix * 8));
-    uint32_t *iw = (uint32_t *)(p + ws_align(g.npix * 8) + ws_align(g.npix * 4));
+    uint32_t *dw = (uint32_t *)(p + align256(g.npix * 8));
+    uint32_t *iw = (uint32_t *)(p + align256(g.npix * 8) + align256(g.npix * 4));
     HIPR_CUDA(cudaMemsetAsync(ws, 0, WS_CTRL_BYTES + 6 * ntiles * 4, st));
     const V *img = (const V *)image;
     const MT *mk = (const MT *)markers;
@@ -362,7 +358,7 @@ extern "C" int hipr_watershed(const void *image_dev, int image_dtype, const void
                               void *stream) {
     WsGeom g;
     if (!image_dev || !markers_dev || !workspace_dev || !labels_out || !status_dev) return HIPR_E_ARG;
-    if (!ws_geom(ndim, d0, d1, d2, connectivity, g)) return HIPR_E_ARG;
+    if (ws_geom(ndim, d0, d1, d2, connectivity, g) == HIPR_E_ARG) return HIPR_E_ARG;
     const int64_t need = hipr_watershed_workspace_bytes(ndim, d0, d1, d2, image_dtype, label_bytes);
     if (need < 0) return (int)need;
     if (workspace_bytes < need) return HIPR_E_RANGE;

@@ -26,12 +26,62 @@ import torch
 from . import tables
 from ._lib import F32, F64, FLAVOURS, I32, I64, U8, HiprError, check, lib
 
-_DT = {torch.float32: F32, torch.float64: F64}
-_VT = {torch.float32: F32, torch.float64: F64, torch.int32: I32, torch.int64: I64, torch.uint8: U8, torch.bool: U8}
+# the ABI's dtype code of each torch dtype an entry point may take (bool is stored as one byte, like uint8)
+_ABI = {torch.float32: F32, torch.float64: F64, torch.int32: I32, torch.int64: I64, torch.uint8: U8, torch.bool: U8}
+_LABEL_DTYPES = (torch.bool, torch.uint8, torch.int32, torch.int64)
+UNSUPPORTED = -9
+HIPR_E_RANGE = -7
 
 
 def _stream():
-    return C.c_void_p(torch.cuda.current_stream().cuda_stream)
+    return torch.cuda.current_stream().cuda_stream
+
+
+_PLAIN = {int, float, bool, type(None)}
+
+
+def _arg(a):
+    """One argument of a libhipr_b200 call: tensors and numpy arrays by their data pointer, a MaxKey by its keys, a
+    list or tuple of them as an array of pointers; anything else (numbers, None, C.byref(...)) as it is."""
+    # isinstance(a, torch.Tensor) is slow when false: it comes last, after the exact type and the other classes
+    if type(a) is torch.Tensor:
+        return a.data_ptr()
+    if isinstance(a, np.ndarray):
+        return a.ctypes.data
+    if isinstance(a, MaxKey):
+        return a.key.data_ptr()
+    if isinstance(a, (list, tuple)):
+        return (C.c_void_p * len(a))(*[_arg(x) for x in a])
+    if isinstance(a, torch.Tensor):
+        return a.data_ptr()
+    return a
+
+
+def _call(name, *args, what=None, ok=()):
+    """lib().hipr_<name>(*args), its return code checked under the prefix `what` (default: name); the codes in `ok`
+    are returned instead of raised."""
+    # numbers and None, most of the arguments, pass without a call of _arg
+    code = getattr(lib(), "hipr_" + name)(*[a if type(a) in _PLAIN else _arg(a) for a in args])
+    if code not in ok:
+        check(code, what or name)
+    return code
+
+
+def _launch(name, device, *args, what=None, ok=()):
+    """_call of a device entry point on `device`, stream-ordered on torch's current stream."""
+    with torch.cuda.device(device):
+        return _call(name, *args, _stream(), what=what, ok=ok)
+
+
+def _workspace(name, device, *size_args, what=None, errors=None):
+    """The uint8 device workspace hipr_<name>(*size_args) asks for.  A negative answer raises ValueError(errors[code])
+    where the caller names the code, and goes through check (prefix `what`, default: name) otherwise."""
+    need = int(getattr(lib(), "hipr_" + name)(*size_args))
+    if need < 0:
+        if errors and need in errors:
+            raise ValueError(errors[need])
+        check(need, what or name)
+    return torch.empty(need, dtype=torch.uint8, device=device)
 
 
 def _dev(t, name, dtypes=(torch.float32, torch.float64)):
@@ -44,8 +94,45 @@ def _dev(t, name, dtypes=(torch.float32, torch.float64)):
     return t.contiguous()
 
 
-def _tab_ptr(tab):
-    return tab.ctypes.data_as(C.c_void_p)
+def _dims(t, name):
+    """(ndim, d0, d1, d2) of a 2-D image or a 3-D volume (d2 = 1 for an image), as the segmentation entry points take
+    it; ValueError for another rank or an empty tensor."""
+    if t.dim() not in (2, 3):
+        raise ValueError("%s must be a 2-D image or a 3-D volume, got shape %s" % (name, tuple(t.shape)))
+    if t.numel() == 0:
+        raise ValueError("%s is empty" % name)
+    return (t.dim(),) + tuple(t.shape) + (1,) * (3 - t.dim())
+
+
+def _same(a, b, names):
+    """ValueError unless tensor a (called names[0]) has the shape and device of b (names[1])."""
+    if a.shape != b.shape:
+        raise ValueError("%s %s and %s %s differ in shape" % (names[0], tuple(a.shape), names[1], tuple(b.shape)))
+    if a.device != b.device:
+        raise ValueError("%s and %s are on different devices" % (names[1], names[0]))
+
+
+def _out_dims(shape, P, padded, what):
+    """Output shape of a stencil with P-sample lines: the input's shape, or with padded=True the shape of the image
+    inside its (P - 1) / 2 border.  ValueError when that is empty."""
+    dims = tuple(d - P + 1 for d in shape) if padded else tuple(shape)
+    if min(dims) < 1:
+        raise ValueError("%s smaller than the patch" % what)
+    return dims
+
+
+_CUBE_AXES = {3: "(H, W, C)", 4: "(X, Y, Z, C)"}
+
+
+def _host_cube(a, ndim=None, dtypes=(np.float32,), name="cube"):
+    """A numpy entry point's input as a C-contiguous array: TypeError for another dtype, ValueError (ndim given) for
+    another rank."""
+    a = np.ascontiguousarray(a)
+    if a.dtype not in dtypes:
+        raise TypeError("%s must be %s, got %s" % (name, " or ".join(np.dtype(d).name for d in dtypes), a.dtype))
+    if ndim is not None and a.ndim != ndim:
+        raise ValueError("cube must be %s" % _CUBE_AXES[ndim])
+    return a
 
 
 def _flavour(f):
@@ -62,28 +149,22 @@ class MaxKey:
         # filled (and reset) by hipr_chansum / hipr_image_range; no torch kernel on the hot path
         self.key = torch.empty(2, dtype=torch.int64, device=device)
 
-    def ptr(self):
-        return C.c_void_p(self.key.data_ptr())
-
     def value(self):
         out = torch.empty(1, dtype=torch.float64, device=self.key.device)
-        with torch.cuda.device(self.key.device):
-            check(lib().hipr_maxkey_decode(self.ptr(), C.c_void_p(out.data_ptr()), _stream()), "maxkey_decode")
+        _launch("maxkey_decode", self.key.device, self, out)
         return out
 
     def values(self):
         """(max, min) as 1-element float64 device tensors."""
         out = torch.empty(2, dtype=torch.float64, device=self.key.device)
-        with torch.cuda.device(self.key.device):
-            check(lib().hipr_range_decode(self.ptr(), C.c_void_p(out.data_ptr()), _stream()), "range_decode")
+        _launch("range_decode", self.key.device, self, out)
         return out[0:1], out[1:2]
 
     @classmethod
     def from_values(cls, vmax, vmin):
         mm = torch.cat([vmax.reshape(1), vmin.reshape(1)]).to(torch.float64).contiguous()
         mk = cls(mm.device)
-        with torch.cuda.device(mm.device):
-            check(lib().hipr_range_encode(C.c_void_p(mm.data_ptr()), mk.ptr(), _stream()), "range_encode")
+        _launch("range_encode", mm.device, mm, mk)
         return mk
 
 
@@ -101,14 +182,9 @@ def channel_sum(cube, calibration=None, normalize=True, dtype=torch.float32, ret
             calibration = calibration.expand_as(cube).contiguous()
     out = torch.empty(cube.shape[:-1], dtype=dtype, device=cube.device)
     mk = MaxKey(cube.device) if (normalize or return_max) else None
-    with torch.cuda.device(cube.device):
-        check(lib().hipr_chansum(C.c_void_p(cube.data_ptr()),
-                                 C.c_void_p(calibration.data_ptr()) if calibration is not None else None,
-                                 npix, Cn, C.c_void_p(out.data_ptr()), _DT[dtype],
-                                 mk.ptr() if mk else None, _stream()), "channel_sum")
-        if normalize:
-            check(lib().hipr_normalize(C.c_void_p(out.data_ptr()), _DT[dtype], npix, mk.ptr(), _stream()),
-                  "normalize")
+    _launch("chansum", cube.device, cube, calibration, npix, Cn, out, _ABI[dtype], mk, what="channel_sum")
+    if normalize:
+        _launch("normalize", cube.device, out, _ABI[dtype], npix, mk)
     return (out, mk) if return_max else out
 
 
@@ -124,9 +200,8 @@ def channel_sum_raw(cube, scale, return_max=False):
     npix = cube.numel() // Cn
     out = torch.empty(cube.shape[:-1], dtype=torch.float64, device=cube.device)
     mk = MaxKey(cube.device)
-    with torch.cuda.device(cube.device):
-        check(lib().hipr_chansum_raw(C.c_void_p(cube.data_ptr()), cube.element_size(), float(scale), npix, Cn,
-                                     C.c_void_p(out.data_ptr()), mk.ptr(), _stream()), "channel_sum_raw")
+    _launch("chansum_raw", cube.device, cube, cube.element_size(), float(scale), npix, Cn, out, mk,
+            what="channel_sum_raw")
     return (out, mk) if return_max else out
 
 
@@ -165,13 +240,7 @@ def register_stacks(stacks, shifts=None, calibration=None, return_cube=True):
     cube = torch.empty((H, W, Cn), dtype=torch.float32, device=dev) if return_cube else None
     s64 = torch.empty((H, W), dtype=torch.float64, device=dev)
     mk = MaxKey(dev)
-    ptrs = (C.c_void_p * n)(*[s.data_ptr() for s in stacks])
-    with torch.cuda.device(dev):
-        check(lib().hipr_register_stacks(ptrs, chans.ctypes.data_as(C.c_void_p), srow.ctypes.data_as(C.c_void_p),
-                                         scol.ctypes.data_as(C.c_void_p), n, H, W,
-                                         C.c_void_p(calibration.data_ptr()) if calibration is not None else None,
-                                         C.c_void_p(cube.data_ptr()) if cube is not None else None,
-                                         C.c_void_p(s64.data_ptr()), mk.ptr(), _stream()), "register_stacks")
+    _launch("register_stacks", dev, stacks, chans, srow, scol, n, H, W, calibration, cube, s64, mk)
     return cube, s64, mk
 
 
@@ -185,12 +254,8 @@ def neighbor2d_score_from_stacks(stacks, shifts=None, calibration=None, flavour=
 
 
 def _xcorr_workspace(H, W, n, device):
-    need = int(lib().hipr_xcorr2d_workspace_bytes(int(H), int(W), int(n)))
-    if need < 0:
-        if need == -9:
-            raise ValueError("image height and width must each be a power of two in [2, 8192], got (%d, %d)" % (H, W))
-        check(need, "xcorr2d_workspace_bytes")
-    return torch.empty(need, dtype=torch.uint8, device=device)
+    return _workspace("xcorr2d_workspace_bytes", device, int(H), int(W), int(n), errors={
+        UNSUPPORTED: "image height and width must each be a power of two in [2, 8192], got (%d, %d)" % (H, W)})
 
 
 def register_translation(src, target, return_correlation=False):
@@ -213,12 +278,8 @@ def register_translation(src, target, return_correlation=False):
     work = _xcorr_workspace(H, W, 2, dev)
     shift = torch.empty(2, dtype=torch.float64, device=dev)
     corr = torch.empty((H, W), dtype=torch.float64, device=dev) if return_correlation else None
-    with torch.cuda.device(dev):
-        check(lib().hipr_register_translation_2d(C.c_void_p(src.data_ptr()), C.c_void_p(target.data_ptr()),
-                                                 _DT[src.dtype], H, W, C.c_void_p(work.data_ptr()), work.numel(),
-                                                 C.c_void_p(shift.data_ptr()),
-                                                 C.c_void_p(corr.data_ptr()) if corr is not None else None,
-                                                 _stream()), "register_translation")
+    _launch("register_translation_2d", dev, src, target, _ABI[src.dtype], H, W, work, work.numel(), shift, corr,
+            what="register_translation")
     out = shift.cpu().numpy()
     return (out, corr) if return_correlation else out
 
@@ -249,11 +310,8 @@ def excitation_shifts(stacks, transform="log", eps=0.0):
     work = _xcorr_workspace(H, W, n, dev)
     shifts = torch.empty((n, 2), dtype=torch.float64, device=dev)
     chans = np.asarray([s.shape[2] for s in stacks], dtype=np.int32)
-    ptrs = (C.c_void_p * n)(*[s.data_ptr() for s in stacks])
-    with torch.cuda.device(dev):
-        check(lib().hipr_excitation_shifts(ptrs, chans.ctypes.data_as(C.c_void_p), n, H, W,
-                                           SHIFT_TRANSFORMS[transform], float(eps), C.c_void_p(work.data_ptr()),
-                                           work.numel(), C.c_void_p(shifts.data_ptr()), _stream()), "excitation_shifts")
+    _launch("excitation_shifts", dev, stacks, chans, n, H, W, SHIFT_TRANSFORMS[transform], float(eps), work,
+            work.numel(), shifts)
     return shifts.cpu().numpy()
 
 
@@ -266,24 +324,18 @@ def denoise_nl_means(image, patch_size=7, patch_distance=11, h=0.1):
     if image.dim() == 3:
         # a z-stack volume (bio/...analysis.py:454, h = 0.03): csrc/nlm3d.cu
         X, Y, Z = image.shape
-        need = int(lib().hipr_denoise_nl_means_3d_workspace(X, Y, Z, int(patch_distance)))
-        if need < 0:
-            raise ValueError("patch_distance must be in [0, 15]")
-        work = torch.empty(need, dtype=torch.uint8, device=image.device)
+        work = _workspace("denoise_nl_means_3d_workspace", image.device, X, Y, Z, int(patch_distance),
+                          errors={-1: "patch_distance must be in [0, 15]"})
         out = torch.empty_like(image)
-        with torch.cuda.device(image.device):
-            check(lib().hipr_denoise_nl_means_3d(C.c_void_p(image.data_ptr()), X, Y, Z, _DT[image.dtype], int(patch_size),
-                                                 int(patch_distance), float(h), C.c_void_p(out.data_ptr()),
-                                                 C.c_void_p(work.data_ptr()), need, _stream()), "denoise_nl_means_3d")
+        _launch("denoise_nl_means_3d", image.device, image, X, Y, Z, _ABI[image.dtype], int(patch_size),
+                int(patch_distance), float(h), out, work, work.numel())
         return out
     if image.dim() != 2:
         raise ValueError("image must be 2-D or 3-D, got %d-D" % image.dim())
     Hh, Ww = image.shape
     out = torch.empty_like(image)
-    with torch.cuda.device(image.device):
-        check(lib().hipr_denoise_nl_means_2d(C.c_void_p(image.data_ptr()), Hh, Ww, _DT[image.dtype], int(patch_size),
-                                             int(patch_distance), float(h), C.c_void_p(out.data_ptr()), _stream()),
-              "denoise_nl_means")
+    _launch("denoise_nl_means_2d", image.device, image, Hh, Ww, _ABI[image.dtype], int(patch_size), int(patch_distance),
+            float(h), out, what="denoise_nl_means")
     return out
 
 
@@ -299,15 +351,9 @@ def lne2d(image, flavour="F1", patch_size=11, phi_range=9, padded=False, maxkey=
     tab = tables.line_table_2d(patch_size, phi_range)
     P = tab.shape[1]
     Hs, Ws = image.shape
-    H, W = (Hs - P + 1, Ws - P + 1) if padded else (Hs, Ws)
-    if H < 1 or W < 1:
-        raise ValueError("image smaller than the patch")
-    out = torch.empty((H, W), dtype=image.dtype, device=image.device)
-    with torch.cuda.device(image.device):
-        check(lib().hipr_lne2d(C.c_void_p(image.data_ptr()), Hs, Ws, Ws, int(bool(padded)), _DT[image.dtype], P,
-                               tab.shape[0], _tab_ptr(tab), _flavour(flavour),
-                               maxkey.ptr() if maxkey is not None else None, C.c_void_p(out.data_ptr()),
-                               _stream()), "lne2d")
+    out = torch.empty(_out_dims(image.shape, P, padded, "image"), dtype=image.dtype, device=image.device)
+    _launch("lne2d", image.device, image, Hs, Ws, Ws, int(bool(padded)), _ABI[image.dtype], P, tab.shape[0], tab,
+            _flavour(flavour), maxkey, out)
     return out
 
 
@@ -315,9 +361,7 @@ def image_range(image):
     """MaxKey (max and min keys) of any float image, for lne2d_fixed."""
     image = _dev(image, "image")
     mk = MaxKey(image.device)
-    with torch.cuda.device(image.device):
-        check(lib().hipr_image_range(C.c_void_p(image.data_ptr()), _DT[image.dtype], image.numel(), mk.ptr(),
-                                     _stream()), "image_range")
+    _launch("image_range", image.device, image, _ABI[image.dtype], image.numel(), mk)
     return mk
 
 
@@ -335,18 +379,12 @@ def lne2d_fixed(image, flavour="F1", patch_size=11, phi_range=9, padded=False, r
         range_keys = image_range(image)      # F3 scales its epsilon by the global range
     # F1 / F2 with no keys: every 32x32 tile is quantised with its own min / max (finest resolution)
     Hs, Ws = image.shape
-    H, W = (Hs - 10, Ws - 10) if padded else (Hs, Ws)
-    if H < 1 or W < 1:
-        raise ValueError("image smaller than the patch")
-    out = torch.empty((H, W), dtype=torch.float32, device=image.device)
-    with torch.cuda.device(image.device):
-        check(lib().hipr_lne2d_q(C.c_void_p(image.data_ptr()), Hs, Ws, Ws, int(bool(padded)), _DT[image.dtype], 11, 9,
-                                 _tab_ptr(tab), _flavour(flavour), range_keys.ptr() if range_keys is not None else None,
-                                 C.c_void_p(out.data_ptr()), _stream()), "lne2d_fixed")
+    out = torch.empty(_out_dims(image.shape, 11, padded, "image"), dtype=torch.float32, device=image.device)
+    _launch("lne2d_q", image.device, image, Hs, Ws, Ws, int(bool(padded)), _ABI[image.dtype], 11, 9, tab,
+            _flavour(flavour), range_keys, out, what="lne2d_fixed")
     return out
 
 
-UNSUPPORTED = -9
 _SIDE = {}
 
 
@@ -355,6 +393,28 @@ def _side_streams(device, n=2):
     if key not in _SIDE:
         _SIDE[key] = [torch.cuda.Stream(device=device) for _ in range(n)]
     return _SIDE[key]
+
+
+def _over_side_streams(batch, fn):
+    """fn(item) for each item of a batch, alternating between two side streams (so that one item's HBM-bound channel
+    sum runs beside the previous item's stencil) and joined on the caller's stream; -> the results stacked (each
+    part of a tuple result stacked on its own)."""
+    cur = torch.cuda.current_stream(batch.device)
+    side = _side_streams(batch.device)
+    for st in side:
+        st.wait_stream(cur)
+    res = []
+    for i, item in enumerate(batch):
+        with torch.cuda.stream(side[i % len(side)]):
+            res.append(fn(item))
+    for st in side:
+        cur.wait_stream(st)
+    for r in res:
+        for t in (r if isinstance(r, tuple) else (r,)):
+            t.record_stream(cur)
+    if res and isinstance(res[0], tuple):
+        return tuple(torch.stack(part) for part in zip(*res))
+    return torch.stack(res)
 
 
 def neighbor2d_fused(cube, flavour="F1", patch_size=11, phi_range=9, return_sum=False):
@@ -369,14 +429,9 @@ def neighbor2d_fused(cube, flavour="F1", patch_size=11, phi_range=9, return_sum=
     score = torch.empty((H, W), dtype=torch.float32, device=cube.device)
     s = torch.empty((H, W), dtype=torch.float64, device=cube.device) if return_sum else None
     mk = MaxKey(cube.device) if return_sum else None
-    with torch.cuda.device(cube.device):
-        code = lib().hipr_neighbor2d_fused(C.c_void_p(cube.data_ptr()), H, W, Cn, tab.shape[1], tab.shape[0],
-                                           _tab_ptr(tab), _flavour(flavour), C.c_void_p(score.data_ptr()),
-                                           C.c_void_p(s.data_ptr()) if return_sum else None,
-                                           mk.ptr() if return_sum else None, _stream())
-    if code == UNSUPPORTED:
+    if _launch("neighbor2d_fused", cube.device, cube, H, W, Cn, tab.shape[1], tab.shape[0], tab, _flavour(flavour),
+               score, s, mk, ok=(UNSUPPORTED,)) == UNSUPPORTED:
         return None
-    check(code, "neighbor2d_fused")
     return (score, s, mk) if return_sum else score
 
 
@@ -392,13 +447,9 @@ def neighbor2d_pipeline(cube, flavour="F1", patch_size=11, phi_range=9, bands=0)
     score = torch.empty((H, W), dtype=torch.float32, device=cube.device)
     s = torch.empty((H, W), dtype=torch.float64, device=cube.device)
     mk = MaxKey(cube.device)
-    with torch.cuda.device(cube.device):
-        code = lib().hipr_neighbor2d(C.c_void_p(cube.data_ptr()), H, W, Cn, tab.shape[1], tab.shape[0], _tab_ptr(tab),
-                                     _flavour(flavour), C.c_void_p(score.data_ptr()), C.c_void_p(s.data_ptr()),
-                                     mk.ptr(), int(bands), _stream())
-    if code == UNSUPPORTED:
+    if _launch("neighbor2d", cube.device, cube, H, W, Cn, tab.shape[1], tab.shape[0], tab, _flavour(flavour), score, s,
+               mk, int(bands), ok=(UNSUPPORTED,)) == UNSUPPORTED:
         return None
-    check(code, "neighbor2d")
     return score, s, mk
 
 
@@ -422,25 +473,9 @@ def neighbor2d_score(cube, flavour="F1", calibration=None, patch_size=11, phi_ra
         score = lne2d(den if dtype in (None, torch.float64) else den.to(dtype), flavour, patch_size, phi_range)
         return (score, den) if return_sum else score
     if cube.dim() == 4:
-        # independent FOVs alternate between two streams: FOV i+1's channel sum (HBM-bound) runs
-        # under FOV i's stencil (SM-bound); joined on the caller's stream before returning
-        cur = torch.cuda.current_stream(cube.device)
-        side = _side_streams(cube.device)
-        for st in side:
-            st.wait_stream(cur)
-        res = []
-        for i, c in enumerate(cube):
-            with torch.cuda.stream(side[i % len(side)]):
-                res.append(neighbor2d_score(c, flavour, None if calibration is None else calibration, patch_size,
-                                            phi_range, dtype, return_sum, denoise_h))
-        for st in side:
-            cur.wait_stream(st)
-        for r in res:
-            for t in (r if return_sum else (r,)):
-                t.record_stream(cur)
-        if return_sum:
-            return torch.stack([r[0] for r in res]), torch.stack([r[1] for r in res])
-        return torch.stack(res)
+        # independent FOVs, each with its own max
+        return _over_side_streams(cube, lambda c: neighbor2d_score(c, flavour, calibration, patch_size, phi_range,
+                                                                   dtype, return_sum, denoise_h))
     if cube.dim() != 3:
         raise ValueError("cube must be (H, W, C) or (N, H, W, C)")
     if dtype is None and calibration is None:
@@ -450,9 +485,7 @@ def neighbor2d_score(cube, flavour="F1", calibration=None, patch_size=11, phi_ra
             if not return_sum:
                 return score
             sn = torch.empty(s.shape, dtype=torch.float32, device=s.device)
-            with torch.cuda.device(cube.device):
-                check(lib().hipr_normalize_cast(C.c_void_p(s.data_ptr()), s.numel(), mk.ptr(),
-                                                C.c_void_p(sn.data_ptr()), _stream()), "normalize_cast")
+            _launch("normalize_cast", cube.device, s, s.numel(), mk, sn)
             return score, sn
     fixed = dtype is None and tables.line_table_2d(patch_size, phi_range).shape[:2] == (9, 11)
     if dtype is None:
@@ -463,9 +496,7 @@ def neighbor2d_score(cube, flavour="F1", calibration=None, patch_size=11, phi_ra
     else:
         score = lne2d(s, flavour, patch_size, phi_range, padded=False, maxkey=mk)
     if return_sum:
-        with torch.cuda.device(cube.device):
-            check(lib().hipr_normalize(C.c_void_p(s.data_ptr()), _DT[dtype], s.numel(), mk.ptr(), _stream()),
-                  "normalize")
+        _launch("normalize", cube.device, s, _ABI[dtype], s.numel(), mk)
         return score, s
     return score
 
@@ -478,12 +509,9 @@ def line_profile_2d(image_padded, patch_size, phi_range):
     tab = tables.line_table_2d(patch_size, phi_range)
     R, P = tab.shape[0], tab.shape[1]
     Hp, Wp = image_padded.shape
-    if Hp < P or Wp < P:
-        raise ValueError("image smaller than the patch")
-    out = torch.empty((Hp - P + 1, Wp - P + 1, R, P), dtype=image_padded.dtype, device=image_padded.device)
-    with torch.cuda.device(image_padded.device):
-        check(lib().hipr_line_profile_2d(C.c_void_p(image_padded.data_ptr()), Hp, Wp, _DT[image_padded.dtype], P, R,
-                                         _tab_ptr(tab), C.c_void_p(out.data_ptr()), _stream()), "line_profile_2d")
+    out = torch.empty(_out_dims(image_padded.shape, P, True, "image") + (R, P), dtype=image_padded.dtype,
+                      device=image_padded.device)
+    _launch("line_profile_2d", image_padded.device, image_padded, Hp, Wp, _ABI[image_padded.dtype], P, R, tab, out)
     return out
 
 
@@ -498,15 +526,12 @@ def _host_gather(name, image_padded, ndim, table_args, what, per_sample, out, pi
         raise ValueError("Buffer has wrong number of dimensions (expected %d, got %d)" % (ndim, a.ndim))
     tab = (tables.line_table_2d if ndim == 2 else tables.line_table_3d)(*table_args)
     R, P = tab.shape[0], tab.shape[1]
-    if min(a.shape) < P:
-        raise ValueError("%s smaller than the patch" % what)
-    shape = tuple(d - P + 1 for d in a.shape) + ((R, P) if per_sample else (R,))
+    shape = _out_dims(a.shape, P, True, what) + ((R, P) if per_sample else (R,))
     if out is None:
         out = torch.empty(shape, dtype=torch.float64, pin_memory=True).numpy() if pinned else np.empty(shape, dtype=np.float64)
     elif out.shape != shape or out.dtype != np.float64 or not out.flags.c_contiguous:
         raise ValueError("out must be a C-contiguous float64 array of shape %s" % (shape,))
-    check(getattr(lib(), "hipr_" + name)(a.ctypes.data_as(C.c_void_p), *a.shape, P, R, _tab_ptr(tab),
-                                         out.ctypes.data_as(C.c_void_p)), name)
+    _call(name, a, *a.shape, P, R, tab, out)
     return out
 
 
@@ -530,13 +555,8 @@ def line_profile_3d(volume_padded, patch_size, theta_range, phi_range):
     v = _vol(volume_padded, "image_padded")
     tab = tables.line_table_3d(patch_size, theta_range, phi_range)
     T, P = tab.shape[0], tab.shape[1]
-    Xp, Yp, Zp = v.shape
-    if min(Xp, Yp, Zp) < P:
-        raise ValueError("volume smaller than the patch")
-    out = torch.empty((Xp - P + 1, Yp - P + 1, Zp - P + 1, T, P), dtype=v.dtype, device=v.device)
-    with torch.cuda.device(v.device):
-        check(lib().hipr_line_profile_3d(C.c_void_p(v.data_ptr()), Xp, Yp, Zp, _DT[v.dtype], P, T, _tab_ptr(tab),
-                                         C.c_void_p(out.data_ptr()), _stream()), "line_profile_3d")
+    out = torch.empty(_out_dims(v.shape, P, True, "volume") + (T, P), dtype=v.dtype, device=v.device)
+    _launch("line_profile_3d", v.device, v, *v.shape, _ABI[v.dtype], P, T, tab, out)
     return out
 
 
@@ -545,15 +565,8 @@ def lne3d_dirs(volume, patch_size=11, theta_range=9, phi_range=9, padded=True, m
     v = _vol(volume, "image_padded")
     tab = tables.line_table_3d(patch_size, theta_range, phi_range)
     T, P = tab.shape[0], tab.shape[1]
-    Xs, Ys, Zs = v.shape
-    dims = [d - P + 1 for d in v.shape] if padded else list(v.shape)
-    if min(dims) < 1:
-        raise ValueError("volume smaller than the patch")
-    out = torch.empty(dims + [T], dtype=v.dtype, device=v.device)
-    with torch.cuda.device(v.device):
-        check(lib().hipr_lne3d_dirs(C.c_void_p(v.data_ptr()), Xs, Ys, Zs, int(bool(padded)), _DT[v.dtype], P, T,
-                                    _tab_ptr(tab), maxkey.ptr() if maxkey is not None else None,
-                                    C.c_void_p(out.data_ptr()), _stream()), "lne3d_dirs")
+    out = torch.empty(_out_dims(v.shape, P, padded, "volume") + (T,), dtype=v.dtype, device=v.device)
+    _launch("lne3d_dirs", v.device, v, *v.shape, int(bool(padded)), _ABI[v.dtype], P, T, tab, maxkey, out)
     return out
 
 
@@ -579,15 +592,8 @@ def lne3d(volume, flavour="F2", patch_size=11, theta_range=9, phi_range=9, padde
     else:
         tab = tables.line_table_3d(patch_size, theta_range, phi_range)
     T, P = tab.shape[0], tab.shape[1]
-    Xs, Ys, Zs = v.shape
-    dims = [d - P + 1 for d in v.shape] if padded else list(v.shape)
-    if min(dims) < 1:
-        raise ValueError("volume smaller than the patch")
-    out = torch.empty(dims, dtype=v.dtype, device=v.device)
-    with torch.cuda.device(v.device):
-        check(lib().hipr_lne3d(C.c_void_p(v.data_ptr()), Xs, Ys, Zs, int(bool(padded)), _DT[v.dtype], P, T,
-                               _tab_ptr(tab), _flavour(flavour), maxkey.ptr() if maxkey is not None else None,
-                               C.c_void_p(out.data_ptr()), _stream()), "lne3d")
+    out = torch.empty(_out_dims(v.shape, P, padded, "volume"), dtype=v.dtype, device=v.device)
+    _launch("lne3d", v.device, v, *v.shape, int(bool(padded)), _ABI[v.dtype], P, T, tab, _flavour(flavour), maxkey, out)
     return out
 
 
@@ -599,18 +605,11 @@ def lne3d_fixed(volume, flavour="ME2", patch_size=11, theta_range=9, phi_range=9
     v = _vol(volume, "volume")
     tab = tables.line_table_3d(patch_size, theta_range, phi_range)
     T, P = tab.shape[0], tab.shape[1]
-    Xs, Ys, Zs = v.shape
-    dims = [d - P + 1 for d in v.shape] if padded else list(v.shape)
-    if min(dims) < 1:
-        raise ValueError("volume smaller than the patch")
-    out = torch.empty(dims + ([T] if dirs_only else []), dtype=torch.float32, device=v.device)
-    with torch.cuda.device(v.device):
-        code = lib().hipr_lne3d_q(C.c_void_p(v.data_ptr()), Xs, Ys, Zs, int(bool(padded)), _DT[v.dtype], P, T,
-                                  _tab_ptr(tab), _flavour(flavour), int(bool(dirs_only)),
-                                  maxkey.ptr() if maxkey is not None else None, C.c_void_p(out.data_ptr()), _stream())
-    if code == UNSUPPORTED:
+    out = torch.empty(_out_dims(v.shape, P, padded, "volume") + ((T,) if dirs_only else ()), dtype=torch.float32,
+                      device=v.device)
+    if _launch("lne3d_q", v.device, v, *v.shape, int(bool(padded)), _ABI[v.dtype], P, T, tab, _flavour(flavour),
+               int(bool(dirs_only)), maxkey, out, what="lne3d_fixed", ok=(UNSUPPORTED,)) == UNSUPPORTED:
         return None
-    check(code, "lne3d_fixed")
     return out
 
 
@@ -625,19 +624,8 @@ def neighbor3d_score(cube, flavour="ME2", patch_size=11, theta_range=9, phi_rang
     stencil (csrc/nlm3d.cu, float64 stencil after it)."""
     cube = _dev(cube, "cube", (torch.float32,))
     if cube.dim() == 5:
-        cur = torch.cuda.current_stream(cube.device)
-        side = _side_streams(cube.device)
-        for st in side:
-            st.wait_stream(cur)
-        res = []
-        for i, c in enumerate(cube):
-            with torch.cuda.stream(side[i % len(side)]):
-                res.append(neighbor3d_score(c, flavour, patch_size, theta_range, phi_range, dtype, denoise_h, denoise_distance))
-        for st in side:
-            cur.wait_stream(st)
-        for r in res:
-            r.record_stream(cur)
-        return torch.stack(res)
+        return _over_side_streams(cube, lambda c: neighbor3d_score(c, flavour, patch_size, theta_range, phi_range,
+                                                                   dtype, denoise_h, denoise_distance))
     if cube.dim() != 4:
         raise ValueError("cube must be (X, Y, Z, C) or (N, X, Y, Z, C)")
     if denoise_h is not None:
@@ -661,10 +649,20 @@ def neighbor3d_score(cube, flavour="ME2", patch_size=11, theta_range=9, phi_rang
 def label_max(labels):
     labels = _dev(labels, "labels", (torch.int32, torch.int64))
     out = torch.empty(1, dtype=torch.int64, device=labels.device)
-    with torch.cuda.device(labels.device):
-        check(lib().hipr_label_max(C.c_void_p(labels.data_ptr()), labels.element_size(), labels.numel(),
-                                   C.c_void_p(out.data_ptr()), _stream()), "label_max")
+    _launch("label_max", labels.device, labels, labels.element_size(), labels.numel(), out)
     return out
+
+
+def _cell_sums(device, cube, labels, Cn, max_label, sums=None, counts=None):
+    """hipr_cell_spectra_accumulate of a cube (a tensor, or the device pointer of a resident one) over a contiguous
+    label image into sums / counts; None: a new zeroed table (hipr_cell_spectra_reset) on `device`."""
+    if sums is None:
+        sums = torch.empty((max_label + 1, Cn), dtype=torch.float64, device=device)
+        counts = torch.empty(max_label + 1, dtype=torch.int32, device=device)
+        _launch("cell_spectra_reset", device, sums, counts, max_label, Cn)
+    _launch("cell_spectra_accumulate", device, cube, labels, labels.element_size(), labels.numel(),
+            labels.shape[-1] if labels.dim() > 1 else 0, Cn, max_label, sums, counts, None)
+    return sums, counts
 
 
 def cell_spectra_accumulate(cube, labels, max_label, sums=None, counts=None):
@@ -673,7 +671,6 @@ def cell_spectra_accumulate(cube, labels, max_label, sums=None, counts=None):
     cube = _dev(cube, "cube", (torch.float32,))
     labels = _dev(labels, "labels", (torch.int32, torch.int64))
     Cn = cube.shape[-1]
-    npix = labels.numel()
     # pixel p of the label image pairs with cube row p: a transposed label image has the right size, the wrong pairing
     if tuple(cube.shape[:-1]) != tuple(labels.shape):
         raise ValueError("cube %s and labels %s do not match: the cube must be labels.shape + (C,)"
@@ -681,21 +678,7 @@ def cell_spectra_accumulate(cube, labels, max_label, sums=None, counts=None):
     max_label = int(max_label)
     if (sums is None) != (counts is None):
         raise ValueError("pass both sums and counts (to keep accumulating) or neither")
-    fresh = sums is None
-    if sums is None:
-        sums = torch.empty((max_label + 1, Cn), dtype=torch.float64, device=cube.device)
-    if counts is None:
-        counts = torch.empty(max_label + 1, dtype=torch.int32, device=cube.device)
-    with torch.cuda.device(cube.device):
-        if fresh:
-            check(lib().hipr_cell_spectra_reset(C.c_void_p(sums.data_ptr()), C.c_void_p(counts.data_ptr()), max_label,
-                                                Cn, _stream()), "cell_spectra_reset")
-        check(lib().hipr_cell_spectra_accumulate(C.c_void_p(cube.data_ptr()), C.c_void_p(labels.data_ptr()),
-                                                 labels.element_size(), npix,
-                                                 labels.shape[-1] if labels.dim() > 1 else 0, Cn, max_label,
-                                                 C.c_void_p(sums.data_ptr()), C.c_void_p(counts.data_ptr()), None,
-                                                 _stream()), "cell_spectra_accumulate")
-    return sums, counts
+    return _cell_sums(cube.device, cube, labels, Cn, max_label, sums, counts)
 
 
 def cell_spectra_finalize(sums, counts):
@@ -709,11 +692,7 @@ def cell_spectra_finalize(sums, counts):
     area = torch.empty(cap, dtype=torch.int64, device=dev)
     avg = torch.empty((cap, Cn), dtype=torch.float64, device=dev)
     norm = torch.empty((cap, Cn), dtype=torch.float64, device=dev)
-    with torch.cuda.device(dev):
-        check(lib().hipr_cell_spectra_finalize(C.c_void_p(sums.data_ptr()), C.c_void_p(counts.data_ptr()), max_label,
-                                               Cn, C.c_void_p(n_cells.data_ptr()), C.c_void_p(labels.data_ptr()),
-                                               C.c_void_p(area.data_ptr()), C.c_void_p(avg.data_ptr()),
-                                               C.c_void_p(norm.data_ptr()), _stream()), "cell_spectra_finalize")
+    _launch("cell_spectra_finalize", dev, sums, counts, max_label, Cn, n_cells, labels, area, avg, norm)
     n = int(n_cells.item())
     return labels[:n], area[:n], avg[:n], norm[:n]
 
@@ -749,13 +728,8 @@ def cell_geometry(labels, max_label=None):
     lab = torch.empty(cap, dtype=torch.int64, device=dev)
     area = torch.empty(cap, dtype=torch.int64, device=dev)
     geom = torch.empty((cap, 9), dtype=torch.float64, device=dev)
-    with torch.cuda.device(dev):
-        check(lib().hipr_cell_moments(C.c_void_p(labels.data_ptr()), labels.element_size(), Hh, Ww, max_label,
-                                      C.c_void_p(mom.data_ptr()), _stream()), "cell_moments")
-        check(lib().hipr_cell_geometry_finalize(C.c_void_p(mom.data_ptr()), max_label, C.c_void_p(scratch.data_ptr()),
-                                                C.c_void_p(n_cells.data_ptr()), C.c_void_p(lab.data_ptr()),
-                                                C.c_void_p(area.data_ptr()), C.c_void_p(geom.data_ptr()), _stream()),
-              "cell_geometry_finalize")
+    _launch("cell_moments", dev, labels, labels.element_size(), Hh, Ww, max_label, mom)
+    _launch("cell_geometry_finalize", dev, mom, max_label, scratch, n_cells, lab, area, geom)
     n = int(n_cells.item())
     return lab[:n], area[:n], geom[:n]
 
@@ -780,7 +754,7 @@ def paint_labels(labels, values, max_label=None):
     values: (max_label + 1,) or (max_label + 1, K) float32 / float64 (or int32 / int64 / uint8 / bool lookup
     tables), row 0 = background."""
     labels = _dev(labels, "labels", (torch.int32, torch.int64))
-    values = _dev(values, "values", tuple(_VT))
+    values = _dev(values, "values", (torch.float32, torch.float64, torch.int32, torch.int64, torch.uint8, torch.bool))
     squeeze = values.dim() == 1
     v2 = values.reshape(values.shape[0], -1)
     if max_label is None:
@@ -789,10 +763,8 @@ def paint_labels(labels, values, max_label=None):
         raise ValueError("values needs max_label + 1 rows")
     K = v2.shape[1]
     out = torch.empty(tuple(labels.shape) + (() if squeeze else (K,)), dtype=values.dtype, device=labels.device)
-    with torch.cuda.device(labels.device):
-        check(lib().hipr_paint_labels(C.c_void_p(labels.data_ptr()), labels.element_size(), labels.numel(),
-                                      C.c_void_p(v2.data_ptr()), K, int(max_label), _VT[values.dtype],
-                                      C.c_void_p(out.data_ptr()), _stream()), "paint_labels")
+    _launch("paint_labels", labels.device, labels, labels.element_size(), labels.numel(), v2, K, int(max_label),
+            _ABI[values.dtype], out)
     return out
 
 
@@ -802,19 +774,12 @@ def paint_labels(labels, values, max_label=None):
 # entries: which components to keep, the new numbering) are built with torch on the device.
 # ---------------------------------------------------------------------------------------------
 
-_LABEL_DT = {torch.bool: U8, torch.uint8: U8, torch.int32: I32, torch.int64: I64}
-
-
-def _label_input(image, name, dtypes=tuple(_LABEL_DT)):
+def _label_input(image, name, dtypes=_LABEL_DTYPES):
     """-> (contiguous tensor, with bool viewed as uint8; dtype code; (ndim, d0, d1, d2))."""
     image = _dev(image, name, dtypes)
-    if image.dim() not in (2, 3):
-        raise ValueError("%s must be a 2-D image or a 3-D volume, got shape %s" % (name, tuple(image.shape)))
-    if image.numel() == 0:
-        raise ValueError("%s is empty" % name)
+    dims = _dims(image, name)
     raw = image.view(torch.uint8) if image.dtype == torch.bool else image
-    shape = tuple(image.shape) + (1,) * (3 - image.dim())
-    return raw, _LABEL_DT[image.dtype], (image.dim(),) + shape
+    return raw, _ABI[image.dtype], dims
 
 
 def _connectivity(connectivity, ndim):
@@ -829,17 +794,11 @@ def _connectivity(connectivity, ndim):
 
 def _label(raw, code, dims, connectivity, invert=False, dtype=torch.int32):
     """Labels and the component count n (a 1-element int64 device tensor); no synchronisation."""
-    ws = lib().hipr_label_workspace_bytes(*dims)
-    if ws < 0:
-        check(int(ws), "label (an image of 2^31 pixels or more)")
     dev = raw.device
-    work = torch.empty(int(ws), dtype=torch.uint8, device=dev)
+    work = _workspace("label_workspace_bytes", dev, *dims, what="label (an image of 2^31 pixels or more)")
     out = torch.empty(raw.shape, dtype=dtype, device=dev)
     n = torch.empty(1, dtype=torch.int64, device=dev)
-    with torch.cuda.device(dev):
-        check(lib().hipr_label(C.c_void_p(raw.data_ptr()), code, int(invert), *dims, connectivity,
-                               C.c_void_p(work.data_ptr()), int(ws), C.c_void_p(out.data_ptr()), out.element_size(),
-                               C.c_void_p(n.data_ptr()), _stream()), "label")
+    _launch("label", dev, raw, code, int(invert), *dims, connectivity, work, work.numel(), out, out.element_size(), n)
     return out, n
 
 
@@ -849,10 +808,7 @@ def _label_counts(labels, dims, max_label, border=-1):
     dev = labels.device
     counts = torch.empty(max_label + 1, dtype=torch.int32, device=dev)
     over = torch.empty(1, dtype=torch.int32, device=dev)
-    with torch.cuda.device(dev):
-        check(lib().hipr_label_counts(C.c_void_p(labels.data_ptr()), labels.element_size(), *dims, int(border),
-                                      int(max_label), C.c_void_p(counts.data_ptr()), C.c_void_p(over.data_ptr()),
-                                      _stream()), "label_counts")
+    _launch("label_counts", dev, labels, labels.element_size(), *dims, int(border), int(max_label), counts, over)
     return counts, over
 
 
@@ -930,10 +886,7 @@ def clear_border(labels, buffer_size=0, bgval=0):
     lab, n = _label(raw, code, dims, dims[0])
     on_edge, _ = _label_counts(lab, dims, int(n.item()), border=buffer_size)
     out = torch.empty_like(raw)
-    with torch.cuda.device(raw.device):
-        check(lib().hipr_label_clear(C.c_void_p(raw.data_ptr()), code, C.c_void_p(lab.data_ptr()), raw.numel(),
-                                     C.c_void_p(on_edge.data_ptr()), bgval, C.c_void_p(out.data_ptr()), _stream()),
-              "clear_border")
+    _launch("label_clear", raw.device, raw, code, lab, raw.numel(), on_edge, bgval, out, what="clear_border")
     return out.view(torch.bool) if labels.dtype == torch.bool else out
 
 
@@ -974,20 +927,11 @@ def _watershed(image, markers, connectivity=1, mask=None):
     (hipr_b200.h: status, rounds and tile visits per phase, CTAs).  Synchronises once, for the NaN check."""
     image = _dev(image, "image", (torch.float32, torch.float64) + tuple(_WS_EXACT))
     markers = _dev(markers, "markers", (torch.int32, torch.int64))
-    if image.dim() not in (2, 3):
-        raise ValueError("image must be a 2-D image or a 3-D volume, got shape %s" % (tuple(image.shape),))
-    if image.numel() == 0:
-        raise ValueError("image is empty")
-    if markers.shape != image.shape:
-        raise ValueError("markers %s and image %s differ in shape" % (tuple(markers.shape), tuple(image.shape)))
-    if image.device != markers.device:
-        raise ValueError("image and markers are on different devices")
+    dims = _dims(image, "image")          # markers and mask: the image's shape
+    _same(markers, image, ("markers", "image"))
     if mask is not None:
         mask = _dev(mask, "mask", (torch.bool, torch.uint8))
-        if mask.shape != image.shape:
-            raise ValueError("mask %s and image %s differ in shape" % (tuple(mask.shape), tuple(image.shape)))
-        if mask.device != image.device:
-            raise ValueError("image and mask are on different devices")
+        _same(mask, image, ("mask", "image"))
         mask = mask.view(torch.uint8) if mask.dtype == torch.bool else mask
     conn = _connectivity(connectivity, image.dim())
     if image.dtype in _WS_EXACT:
@@ -996,20 +940,13 @@ def _watershed(image, markers, connectivity=1, mask=None):
         nan = torch.isnan(image) if mask is None else torch.isnan(image) & (mask != 0)
         if bool(nan.any()):
             raise ValueError("image has NaN inside the mask: the flooding order is undefined there")
-    dims = (image.dim(),) + tuple(image.shape) + (1,) * (3 - image.dim())
-    code, lb = _DT[image.dtype], markers.element_size()
-    ws = lib().hipr_watershed_workspace_bytes(*dims, code, lb)
-    if ws < 0:
-        check(int(ws), "watershed (an image of 2^31 pixels or more)")
+    code, lb = _ABI[image.dtype], markers.element_size()
     dev = image.device
-    work = torch.empty(int(ws), dtype=torch.uint8, device=dev)
+    work = _workspace("watershed_workspace_bytes", dev, *dims, code, lb,
+                      what="watershed (an image of 2^31 pixels or more)")
     out = torch.empty_like(markers)
     status = torch.empty(8, dtype=torch.int64, device=dev)
-    with torch.cuda.device(dev):
-        check(lib().hipr_watershed(C.c_void_p(image.data_ptr()), code, C.c_void_p(markers.data_ptr()), lb,
-                                   C.c_void_p(mask.data_ptr()) if mask is not None else None, *dims, conn,
-                                   C.c_void_p(work.data_ptr()), int(ws), C.c_void_p(out.data_ptr()),
-                                   C.c_void_p(status.data_ptr()), _stream()), "watershed")
+    _launch("watershed", dev, image, code, markers, lb, mask, *dims, conn, work, work.numel(), out, status)
     return out, status
 
 
@@ -1086,18 +1023,13 @@ def _morphology(mask, structure, iterations, border_value, dilate):
     raw, _, dims = _label_input(mask, "mask", (torch.bool, torch.uint8))
     s = _structure(structure, dims[0])
     iterations = _iterations(iterations)
-    ws = lib().hipr_morphology_workspace_bytes(*dims, iterations)
-    if ws < 0:
-        check(int(ws), "binary morphology (an image of 2^31 pixels or more)")
     dev = raw.device
-    work = torch.empty(int(ws), dtype=torch.uint8, device=dev)
+    work = _workspace("morphology_workspace_bytes", dev, *dims, iterations,
+                      what="binary morphology (an image of 2^31 pixels or more)")
     out = torch.empty(raw.shape, dtype=torch.uint8, device=dev)
-    with torch.cuda.device(dev):
-        check(lib().hipr_binary_morphology(C.c_void_p(raw.data_ptr()), *dims, s.ctypes.data_as(C.c_void_p),
-                                           *(s.shape + (1,) * (3 - s.ndim)), int(dilate), 1 if border_value else 0,
-                                           iterations, C.c_void_p(work.data_ptr()), int(ws),
-                                           C.c_void_p(out.data_ptr()), _stream()),
-              "binary_dilation" if dilate else "binary_erosion")
+    _launch("binary_morphology", dev, raw, *dims, s, *(s.shape + (1,) * (3 - s.ndim)), int(dilate),
+            1 if border_value else 0, iterations, work, work.numel(), out,
+            what="binary_dilation" if dilate else "binary_erosion")
     return out.view(torch.bool)
 
 
@@ -1175,17 +1107,13 @@ def kmeans_threshold(image, n_clusters=2, random_state=0, n_init=1, transform=No
     except KeyError:
         raise ValueError("transform must be None, 'log10' or 'log'")
     dev = image.device
-    work = torch.empty(int(lib().hipr_kmeans1d_workspace_bytes()), dtype=torch.uint8, device=dev)
+    work = _workspace("kmeans1d_workspace_bytes", dev)
     labels = torch.empty(image.shape, dtype=torch.int32, device=dev) if return_labels else None
     mask = torch.empty(image.shape, dtype=torch.uint8, device=dev) if return_mask else None
     res = torch.empty(32, dtype=torch.float64, device=dev)
-    with torch.cuda.device(dev):
-        check(lib().hipr_kmeans1d(C.c_void_p(image.data_ptr()), _DT[image.dtype], image.numel(), tcode, float(eps),
-                                  int(bool(positive_only)), k, int(n_init), u.ctypes.data_as(C.c_void_p), int(max_iter),
-                                  float(tol), C.c_void_p(work.data_ptr()),
-                                  C.c_void_p(labels.data_ptr()) if labels is not None else None, int(fill_label),
-                                  C.c_void_p(mask.data_ptr()) if mask is not None else None,
-                                  C.c_void_p(res.data_ptr()), _stream()), "kmeans_threshold")
+    _launch("kmeans1d", dev, image, _ABI[image.dtype], image.numel(), tcode, float(eps), int(bool(positive_only)), k,
+            int(n_init), u, int(max_iter), float(tol), work, labels, int(fill_label), mask, res,
+            what="kmeans_threshold")
     r = res.cpu().numpy()
     status = int(r[0])
     if status == 2:
@@ -1208,7 +1136,7 @@ def pinned_empty(shape, dtype=np.float32):
     dtype = np.dtype(dtype)
     nbytes = int(np.prod(shape)) * dtype.itemsize
     p = C.c_void_p()
-    check(lib().hipr_host_alloc(C.byref(p), max(nbytes, 1)), "host_alloc")
+    _call("host_alloc", C.byref(p), max(nbytes, 1))
 
     class _Owner:
         def __init__(self, ptr):
@@ -1228,32 +1156,24 @@ def pinned_empty(shape, dtype=np.float32):
 def neighbor2d_score_host(cube, flavour="F1", patch_size=11, phi_range=9, return_sum=False, out=None, denoise_h=None):
     """numpy (H, W, C) float32 -> numpy (H, W) float32 score map, through hipr_neighbor2d_host (denoise_h: with the
     NL-means denoise of syn/...measurement.py:108 in the chain, hipr_neighbor2d_host_denoise)."""
-    cube = np.ascontiguousarray(cube)
-    if cube.dtype != np.float32:
-        raise TypeError("cube must be float32, got %s" % cube.dtype)
-    if cube.ndim != 3:
-        raise ValueError("cube must be (H, W, C)")
+    cube = _host_cube(cube, 3)
     H, W, Cn = cube.shape
     tab = tables.line_table_2d(patch_size, phi_range)
     score = out if out is not None else np.empty((H, W), dtype=np.float32)
     s = np.empty((H, W), dtype=np.float32) if return_sum else None
     name, denoise = ("neighbor2d_host", ()) if denoise_h is None else ("neighbor2d_host_denoise", (float(denoise_h),))
-    check(getattr(lib(), "hipr_" + name)(cube.ctypes.data_as(C.c_void_p), H, W, Cn, tab.shape[1], tab.shape[0],
-                                         _tab_ptr(tab), _flavour(flavour), *denoise, score.ctypes.data_as(C.c_void_p),
-                                         s.ctypes.data_as(C.c_void_p) if return_sum else None), name)
+    _call(name, cube, H, W, Cn, tab.shape[1], tab.shape[0], tab, _flavour(flavour), *denoise, score, s)
     return (score, s) if return_sum else score
 
 
 def neighbor2d_score_host_batch(cubes, flavour="F1", patch_size=11, phi_range=9, denoise_h=None, out=None):
     """A list of numpy (H, W, C) float32 cubes -> list of numpy (H, W) float32 score maps through
     hipr_neighbor2d_host_batch: FOV i + 1 crosses PCIe while FOV i is denoised (denoise_h), scored and read back."""
-    cubes = [np.ascontiguousarray(c) for c in cubes]
+    cubes = [_host_cube(c) for c in cubes]
     if not cubes:
         raise ValueError("empty batch")
     H, W, Cn = cubes[0].shape
     for c in cubes:
-        if c.dtype != np.float32:
-            raise TypeError("cube must be float32, got %s" % c.dtype)
         if c.shape != (H, W, Cn):
             raise ValueError("every cube of a batch must have the same (H, W, C)")
     n = len(cubes)
@@ -1261,10 +1181,8 @@ def neighbor2d_score_host_batch(cubes, flavour="F1", patch_size=11, phi_range=9,
     scores = out if out is not None else [np.empty((H, W), dtype=np.float32) for _ in range(n)]
     if len(scores) != n:
         raise ValueError("one output array per cube")
-    cp = (C.c_void_p * n)(*[c.ctypes.data for c in cubes])
-    sp = (C.c_void_p * n)(*[s.ctypes.data for s in scores])
-    check(lib().hipr_neighbor2d_host_batch(cp, n, H, W, Cn, tab.shape[1], tab.shape[0], _tab_ptr(tab), _flavour(flavour),
-                                           float(denoise_h) if denoise_h else 0.0, sp), "neighbor2d_host_batch")
+    _call("neighbor2d_host_batch", cubes, n, H, W, Cn, tab.shape[1], tab.shape[0], tab, _flavour(flavour),
+          float(denoise_h) if denoise_h else 0.0, scores)
     return scores
 
 
@@ -1273,76 +1191,68 @@ def neighbor3d_score_host(cube, flavour="ME2", patch_size=11, theta_range=9, phi
     """numpy (X, Y, Z, C) float32 -> numpy (X, Y, Z) float32 score volume, through hipr_neighbor3d_host
     (bio/...analysis.py:807-817 for 'ME2'); denoise_h: with the 3-D NL-means of bio/...analysis.py:454 in the chain
     (hipr_neighbor3d_host_denoise)."""
-    cube = np.ascontiguousarray(cube)
-    if cube.dtype != np.float32:
-        raise TypeError("cube must be float32, got %s" % cube.dtype)
-    if cube.ndim != 4:
-        raise ValueError("cube must be (X, Y, Z, C)")
+    cube = _host_cube(cube, 4)
     X, Y, Z, Cn = cube.shape
     tab = tables.line_table_3d(patch_size, theta_range, phi_range)
     score = out if out is not None else np.empty((X, Y, Z), dtype=np.float32)
-    if denoise_h is not None:
-        check(lib().hipr_neighbor3d_host_denoise(cube.ctypes.data_as(C.c_void_p), X, Y, Z, Cn, tab.shape[1], tab.shape[0],
-                                                 _tab_ptr(tab), _flavour(flavour), float(denoise_h), int(denoise_distance),
-                                                 score.ctypes.data_as(C.c_void_p)), "neighbor3d_host_denoise")
-        return score
-    check(lib().hipr_neighbor3d_host(cube.ctypes.data_as(C.c_void_p), X, Y, Z, Cn, tab.shape[1], tab.shape[0],
-                                     _tab_ptr(tab), _flavour(flavour), score.ctypes.data_as(C.c_void_p)),
-          "neighbor3d_host")
+    name, denoise = (("neighbor3d_host", ()) if denoise_h is None else
+                     ("neighbor3d_host_denoise", (float(denoise_h), int(denoise_distance))))
+    _call(name, cube, X, Y, Z, Cn, tab.shape[1], tab.shape[0], tab, _flavour(flavour), *denoise, score)
     return score
 
 
 def neighbor2d_score_host_raw(cube, scale, flavour="F1", patch_size=11, phi_range=9, out=None):
     """numpy (H, W, C) uint16 / uint8 raw counts -> numpy (H, W) float32 score map, the score of the cube
     bioformats' rescale would produce (count / scale in float32), through hipr_neighbor2d_host_raw."""
-    cube = np.ascontiguousarray(cube)
-    if cube.dtype not in (np.uint8, np.uint16):
-        raise TypeError("raw cube must be uint8 or uint16, got %s" % cube.dtype)
-    if cube.ndim != 3:
-        raise ValueError("cube must be (H, W, C)")
+    cube = _host_cube(cube, 3, (np.uint8, np.uint16), "raw cube")
     H, W, Cn = cube.shape
     tab = tables.line_table_2d(patch_size, phi_range)
     score = out if out is not None else np.empty((H, W), dtype=np.float32)
-    check(lib().hipr_neighbor2d_host_raw(cube.ctypes.data_as(C.c_void_p), cube.itemsize, float(scale), H, W, Cn,
-                                         tab.shape[1], tab.shape[0], _tab_ptr(tab), _flavour(flavour),
-                                         score.ctypes.data_as(C.c_void_p), None), "neighbor2d_host_raw")
+    _call("neighbor2d_host_raw", cube, cube.itemsize, float(scale), H, W, Cn, tab.shape[1], tab.shape[0], tab,
+          _flavour(flavour), score, None)
     return score
 
 
 def cell_spectra_host(cube, labels):
     """numpy cube (..., C) float32 + integer label image -> (labels, area, avgint, avgint_norm)."""
-    cube = np.ascontiguousarray(cube)
-    labels = np.ascontiguousarray(labels)
-    if cube.dtype != np.float32:
-        raise TypeError("cube must be float32, got %s" % cube.dtype)
-    if labels.dtype not in (np.int32, np.int64):
-        raise TypeError("labels must be int32 or int64, got %s" % labels.dtype)
+    cube = _host_cube(cube)
+    labels = _host_cube(labels, None, (np.int32, np.int64), "labels")
     Cn = cube.shape[-1]
-    npix = labels.size
     if cube.shape[:-1] != labels.shape:
         raise ValueError("cube %s and labels %s do not match: the cube must be labels.shape + (C,)"
                          % (cube.shape, labels.shape))
-    cap = 4096
+    cols = labels.shape[-1] if labels.ndim > 1 else 0
 
-    def alloc(k):
-        return np.empty(k, np.int64), np.empty(k, np.int64), np.empty((k, Cn), np.float64), np.empty((k, Cn), np.float64)
+    def fill(cap, n, *table):
+        return _call("cell_spectra_host", cube, labels, labels.itemsize, labels.size, cols, Cn, cap, n, *table,
+                     ok=(HIPR_E_RANGE,))
 
-    n = C.c_int64(0)
-    lab, area, avg, norm = alloc(cap)
-    code = lib().hipr_cell_spectra_host(cube.ctypes.data_as(C.c_void_p), labels.ctypes.data_as(C.c_void_p),
-                                        labels.itemsize, npix, labels.shape[-1] if labels.ndim > 1 else 0, Cn, cap,
-                                        C.byref(n),
-                                        lab.ctypes.data_as(C.c_void_p), area.ctypes.data_as(C.c_void_p),
-                                        avg.ctypes.data_as(C.c_void_p), norm.ctypes.data_as(C.c_void_p))
-    if code == -7 and n.value > cap:
-        # more cells than the first guess: the table is still on the device, fetch it (no second pass over the cube)
+    def fetch(cap, n, *table):
+        # the table is still on the device: fetch it (no second pass over the cube)
+        return _call("cell_spectra_host_fetch", cap, *table, what="cell_spectra_host")
+
+    return _cell_table(Cn, "cell_spectra_host", fill, fetch)
+
+
+def _cell_rows(k, Cn):
+    """A host cell table of k rows: labels, area, avgint, avgint_norm."""
+    return np.empty(k, np.int64), np.empty(k, np.int64), np.empty((k, Cn), np.float64), np.empty((k, Cn), np.float64)
+
+
+def _cell_table(Cn, what, fill, refill):
+    """(labels, area, avgint, avgint_norm) from a host entry point: fill(cap, n, *table) writes up to cap rows and the
+    number of cells to n; when they do not fit (HIPR_E_RANGE with n > cap), refill(cap, n, *table) writes them again
+    to a table of cap = n rows."""
+    n, cap = C.c_int64(0), 4096
+    table = _cell_rows(cap, Cn)
+    code = fill(cap, C.byref(n), *table)
+    if code == HIPR_E_RANGE and n.value > cap:
         cap = int(n.value)
-        lab, area, avg, norm = alloc(cap)
-        code = lib().hipr_cell_spectra_host_fetch(cap, lab.ctypes.data_as(C.c_void_p), area.ctypes.data_as(C.c_void_p),
-                                                  avg.ctypes.data_as(C.c_void_p), norm.ctypes.data_as(C.c_void_p))
-    check(code, "cell_spectra_host")
+        table = _cell_rows(cap, Cn)
+        code = refill(cap, C.byref(n), *table)
+    check(code, what)
     k = int(n.value)
-    return lab[:k], area[:k], avg[:k], norm[:k]
+    return tuple(a[:k] for a in table)
 
 
 class Fov:
@@ -1357,17 +1267,12 @@ class Fov:
     """
 
     def __init__(self, cube):
-        cube = np.ascontiguousarray(cube)
-        if cube.dtype != np.float32:
-            raise TypeError("cube must be float32, got %s" % cube.dtype)
-        if cube.ndim != 3:
-            raise ValueError("cube must be (H, W, C)")
+        cube = _host_cube(cube, 3)
         self.shape = cube.shape
         # hipr_fov_upload uses the current device (needed only to check device labels against it)
         self._device = torch.cuda.current_device() if torch.cuda.is_available() else None
         h = C.c_void_p()
-        check(lib().hipr_fov_upload(cube.ctypes.data_as(C.c_void_p), cube.shape[0], cube.shape[1], cube.shape[2],
-                                    C.byref(h)), "fov_upload")
+        _call("fov_upload", cube, *cube.shape, C.byref(h))
         self._h = h
 
     def _handle(self):
@@ -1380,9 +1285,7 @@ class Fov:
         tab = tables.line_table_2d(patch_size, phi_range)
         score = out if out is not None else np.empty((H, W), dtype=np.float32)
         s = np.empty((H, W), dtype=np.float32) if return_sum else None
-        check(lib().hipr_fov_score(self._handle(), tab.shape[1], tab.shape[0], _tab_ptr(tab), _flavour(flavour),
-                                   score.ctypes.data_as(C.c_void_p), s.ctypes.data_as(C.c_void_p) if return_sum else None),
-              "fov_score")
+        _call("fov_score", self._handle(), tab.shape[1], tab.shape[0], tab, _flavour(flavour), score, s)
         return (score, s) if return_sum else score
 
     def cell_spectra(self, labels):
@@ -1391,26 +1294,17 @@ class Fov:
         place, stream-ordered on torch's current stream: a label image from `watershed` never leaves the device)."""
         if isinstance(labels, torch.Tensor):
             return self._cell_spectra_device(labels)
-        labels = np.ascontiguousarray(labels)
-        if labels.dtype not in (np.int32, np.int64):
-            raise TypeError("labels must be int32 or int64, got %s" % labels.dtype)
+        labels = _host_cube(labels, None, (np.int32, np.int64), "labels")
         H, W, Cn = self.shape
         if labels.shape != (H, W):
             raise ValueError("labels must be (%d, %d)" % (H, W))
-        cap = 4096
-        while True:
-            lab, area = np.empty(cap, np.int64), np.empty(cap, np.int64)
-            avg, norm = np.empty((cap, Cn), np.float64), np.empty((cap, Cn), np.float64)
-            n = C.c_int64(0)
-            code = lib().hipr_fov_cell_spectra(self._handle(), labels.ctypes.data_as(C.c_void_p), labels.itemsize, cap,
-                                               C.byref(n), lab.ctypes.data_as(C.c_void_p), area.ctypes.data_as(C.c_void_p),
-                                               avg.ctypes.data_as(C.c_void_p), norm.ctypes.data_as(C.c_void_p))
-            if code == -7 and n.value > cap:
-                cap = int(n.value)           # the cube is resident: the second call is one pass over it, no upload
-                continue
-            check(code, "fov_cell_spectra")
-            k = int(n.value)
-            return lab[:k], area[:k], avg[:k], norm[:k]
+
+        def fill(cap, n, *table):
+            return _call("fov_cell_spectra", self._handle(), labels, labels.itemsize, cap, n, *table,
+                         ok=(HIPR_E_RANGE,))
+
+        # the cube is resident: the second call is one pass over it, no upload
+        return _cell_table(Cn, "fov_cell_spectra", fill, fill)
 
     def _cell_spectra_device(self, labels):
         labels = _dev(labels, "labels", (torch.int32, torch.int64))
@@ -1420,26 +1314,17 @@ class Fov:
         if labels.device.index != self._device:
             raise ValueError("labels live on cuda:%d, this field of view on cuda:%d" % (labels.device.index,
                                                                                        self._device))
-        cube = C.c_void_p(self.device_arrays()[0])
+        cube = self.device_arrays()[0]
         max_label = int(label_max(labels).item())
         if max_label <= 0:
-            return (np.empty(0, np.int64), np.empty(0, np.int64), np.empty((0, Cn), np.float64),
-                    np.empty((0, Cn), np.float64))
-        sums = torch.empty((max_label + 1, Cn), dtype=torch.float64, device=labels.device)
-        counts = torch.empty(max_label + 1, dtype=torch.int32, device=labels.device)
-        with torch.cuda.device(labels.device):
-            check(lib().hipr_cell_spectra_reset(C.c_void_p(sums.data_ptr()), C.c_void_p(counts.data_ptr()), max_label,
-                                                Cn, _stream()), "cell_spectra_reset")
-            check(lib().hipr_cell_spectra_accumulate(cube, C.c_void_p(labels.data_ptr()), labels.element_size(),
-                                                     H * W, W, Cn, max_label, C.c_void_p(sums.data_ptr()),
-                                                     C.c_void_p(counts.data_ptr()), None, _stream()),
-                  "cell_spectra_accumulate")
+            return _cell_rows(0, Cn)
+        sums, counts = _cell_sums(labels.device, cube, labels, Cn, max_label)
         return tuple(t.cpu().numpy() for t in cell_spectra_finalize(sums, counts))
 
     def device_arrays(self):
         """(cube, channel sums, range keys) device pointers as ints, for callers that continue on the device."""
         a, b, c = C.c_void_p(), C.c_void_p(), C.c_void_p()
-        check(lib().hipr_fov_device_arrays(self._handle(), C.byref(a), C.byref(b), C.byref(c)), "fov_device_arrays")
+        _call("fov_device_arrays", self._handle(), C.byref(a), C.byref(b), C.byref(c))
         return a.value, b.value, c.value
 
     def close(self):

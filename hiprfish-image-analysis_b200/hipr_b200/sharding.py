@@ -12,8 +12,14 @@
 The compute steps are the CUDA operators in hipr_b200.ops; `MosaicSlab` takes them as hooks so
 the communication logic can be exercised on CPU tensors with the gloo backend in tests.
 """
+import ctypes as C
+
 import torch
 import torch.distributed as dist
+
+from . import tables
+from ._lib import FLAVOURS, lib
+from .ops import _call, _launch
 
 HALO = 5   # (patch_size - 1) / 2 for the 11-sample lines every pipeline uses
 
@@ -129,9 +135,6 @@ class P2PMosaicSlab:
     torch.distributed), which also lets two ranks share one GPU (cudaIpc mappings work within a device)."""
 
     def __init__(self, rows, width, group=None, timeout_ms=None):
-        import ctypes as C
-        from ._lib import check, lib
-        self._C, self._check, self._lib = C, check, lib()
         self.group = group
         self.world = dist.get_world_size(group)
         self.rank = dist.get_rank(group)
@@ -140,16 +143,16 @@ class P2PMosaicSlab:
         dist.all_gather_object(all_rows, self.rows, group=group)
         self.all_rows = [int(r) for r in all_rows]
         self.rows_max = max(self.all_rows)
-        nbytes = self._lib.hipr_mosaic_p2p_bytes(self.rows_max, self.width, self.world)
+        nbytes = lib().hipr_mosaic_p2p_bytes(self.rows_max, self.width, self.world)
         if nbytes <= 0:
             raise ValueError("mosaic geometry not supported by the peer-memory exchange")
         if timeout_ms is not None:
-            check(self._lib.hipr_mosaic_p2p_set_timeout_ms(float(timeout_ms)), "p2p_set_timeout_ms")
+            _call("mosaic_p2p_set_timeout_ms", float(timeout_ms), what="p2p_set_timeout_ms")
         base = C.c_void_p()
-        check(self._lib.hipr_p2p_alloc(C.byref(base), nbytes), "p2p_alloc")
+        _call("p2p_alloc", C.byref(base), nbytes)
         self._own = base
         handle = (C.c_ubyte * 64)()
-        check(self._lib.hipr_p2p_get_handle(base, handle), "p2p_get_handle")
+        _call("p2p_get_handle", base, handle)
         handles = [None] * self.world
         dist.all_gather_object(handles, bytes(handle), group=group)
         self._opened = []
@@ -160,7 +163,7 @@ class P2PMosaicSlab:
                 continue
             peer = C.c_void_p()
             buf = (C.c_ubyte * 64).from_buffer_copy(h)
-            check(self._lib.hipr_p2p_open_handle(buf, C.byref(peer)), "p2p_open_handle (rank %d)" % r)
+            _call("p2p_open_handle", buf, C.byref(peer), what="p2p_open_handle (rank %d)" % r)
             self._opened.append(peer)
             bases.append(peer.value)
         self._bases = (C.c_void_p * self.world)(*bases)
@@ -172,10 +175,9 @@ class P2PMosaicSlab:
         dist.barrier(group=group)        # every rank has opened every buffer before the first push
 
     def _rows_ptr(self, parity, with_top_halo):
-        C = self._C
         p = C.c_void_p()
-        self._check(self._lib.hipr_mosaic_p2p_rows_ptr(self._own, self.rows_max, self.width, self.world, parity,
-                                                       int(with_top_halo), C.byref(p)), "p2p_rows_ptr")
+        _call("mosaic_p2p_rows_ptr", self._own, self.rows_max, self.width, self.world, parity, int(with_top_halo),
+              C.byref(p), what="p2p_rows_ptr")
         return p
 
     def score(self, cube_slab, flavour="F1", bands=0, check=False):
@@ -183,49 +185,36 @@ class P2PMosaicSlab:
         bands >= 3 (F1 / F2): one call that also hides the stencil under the channel sum, band by band
         (hipr_mosaic_p2p_score; every tile quantised with its own range).  bands = 0: channel sum, exchange,
         stencil in order (bit-identical to MosaicSlab.score); F3 uses the exchanged global range."""
-        from . import tables
-        from ._lib import FLAVOURS
-        C = self._C
         if tuple(cube_slab.shape[:2]) != (self.rows, self.width) or cube_slab.dtype != torch.float32:
             raise ValueError("cube_slab must be (%d, %d, C) float32" % (self.rows, self.width))
         cube_slab = cube_slab.contiguous()
         Cn = cube_slab.shape[2]
+        dev = cube_slab.device
         self.epoch += 1
         parity = self.epoch & 1
-        st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
-        keys = C.c_void_p(self._keys.data_ptr())
+        rows_up = self.all_rows[self.rank - 1] if self.rank > 0 else 0
         if bands >= 3:
             tab = tables.line_table_2d(11, 9)
-            out = torch.empty((self.rows, self.width), dtype=torch.float32, device=cube_slab.device)
-            rows_up = self.all_rows[self.rank - 1] if self.rank > 0 else 0
-            self._check(self._lib.hipr_mosaic_p2p_score(C.c_void_p(cube_slab.data_ptr()), Cn, self._bases, self.rank,
-                                                        self.world, self.rows, rows_up, self.rows_max, self.width, parity,
-                                                        self.epoch, tab.ctypes.data_as(C.c_void_p), FLAVOURS[flavour],
-                                                        int(bands), keys, C.c_void_p(self._range.data_ptr()),
-                                                        C.c_void_p(self._error.data_ptr()), C.c_void_p(out.data_ptr()), st),
-                        "mosaic_p2p_score")
+            out = torch.empty((self.rows, self.width), dtype=torch.float32, device=dev)
+            _launch("mosaic_p2p_score", dev, cube_slab, Cn, self._bases, self.rank, self.world, self.rows, rows_up,
+                    self.rows_max, self.width, parity, self.epoch, tab, FLAVOURS[flavour], int(bands), self._keys,
+                    self._range, self._error, out)
             if check:
                 self.check_peers()
             return out
         # channel sums straight into this rank's peer-mapped buffer (rows 5 .. 5 + rows of ext[parity])
-        self._check(self._lib.hipr_chansum(C.c_void_p(cube_slab.data_ptr()), None, self.rows * self.width, Cn,
-                                           self._rows_ptr(parity, False), 1, keys, st), "channel_sum")
-        rows_up = self.all_rows[self.rank - 1] if self.rank > 0 else 0
-        self._check(self._lib.hipr_mosaic_p2p_exchange(self._bases, self.rank, self.world, self.rows, rows_up, self.rows_max,
-                                                       self.width, parity, keys, self.epoch,
-                                                       C.c_void_p(self._range.data_ptr()), C.c_void_p(self._error.data_ptr()),
-                                                       st), "mosaic_p2p_exchange")
+        _launch("chansum", dev, cube_slab, None, self.rows * self.width, Cn, self._rows_ptr(parity, False), 1,
+                self._keys, what="channel_sum")
+        _launch("mosaic_p2p_exchange", dev, self._bases, self.rank, self.world, self.rows, rows_up, self.rows_max,
+                self.width, parity, self._keys, self.epoch, self._range, self._error)
         n_top = HALO if self.rank > 0 else 0
         n_bottom = HALO if self.rank + 1 < self.world else 0
         Hs = self.rows + n_top + n_bottom
         tab = tables.line_table_2d(11, 9)
-        out = torch.empty((Hs, self.width), dtype=torch.float32, device=cube_slab.device)
-        self._check(self._lib.hipr_lne2d_q(self._rows_ptr(parity, n_top > 0), Hs, self.width, self.width, 0, 1, 11, 9,
-                                           tab.ctypes.data_as(C.c_void_p), FLAVOURS[flavour],
-                                           C.c_void_p(self._range.data_ptr()) if flavour not in ("F1", "F2") else None,
-                                           C.c_void_p(out.data_ptr()), st), "lne2d_q")
-        self._check(self._lib.hipr_mosaic_p2p_guard(C.c_void_p(self._error.data_ptr()), C.c_void_p(out.data_ptr()),
-                                                    out.numel(), st), "mosaic_p2p_guard")
+        out = torch.empty((Hs, self.width), dtype=torch.float32, device=dev)
+        _launch("lne2d_q", dev, self._rows_ptr(parity, n_top > 0), Hs, self.width, self.width, 0, 1, 11, 9, tab,
+                FLAVOURS[flavour], self._range if flavour not in ("F1", "F2") else None, out)
+        _launch("mosaic_p2p_guard", dev, self._error, out, out.numel())
         if check:
             self.check_peers()
         return out[n_top: Hs - n_bottom]
@@ -239,10 +228,10 @@ class P2PMosaicSlab:
         torch.cuda.synchronize()
         dist.barrier(group=self.group)   # nobody still pushes into a buffer that is about to be freed
         for p in self._opened:
-            self._lib.hipr_p2p_close_handle(p)
+            lib().hipr_p2p_close_handle(p)
         self._opened = []
         if self._own is not None:
-            self._lib.hipr_p2p_free(self._own)
+            lib().hipr_p2p_free(self._own)
             self._own = None
 
 

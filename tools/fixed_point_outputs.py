@@ -7,7 +7,6 @@ Dump once per library, each in its own process, then compare:
     python tools/fixed_point_outputs.py compare A.npz B.npz
 """
 import argparse
-import ctypes as C
 import os
 import sys
 
@@ -52,10 +51,8 @@ def dump(path, lib_path):
                     continue
                 for tname, tab in (("baked", pinned), ("table", other)):
                     o = torch.empty((2048, 2048), dtype=torch.float32, device=dev)
-                    ops.check(_lib.lib().hipr_lne2d_q(
-                        C.c_void_p(img.data_ptr()), 2048, 2048, 2048, 0, ops._DT[dt], 11, 9,
-                        tab.ctypes.data_as(C.c_void_p), _lib.FLAVOURS[fl], keys.ptr() if rng == "global" else None,
-                        C.c_void_p(o.data_ptr()), None), "hipr_lne2d_q")
+                    ops._launch("lne2d_q", dev, img, 2048, 2048, 2048, 0, ops._ABI[dt], 11, 9, tab, _lib.FLAVOURS[fl],
+                                keys if rng == "global" else None, o, what="hipr_lne2d_q")
                     put("lne2d_%s_%s_%s_%s" % (str(dt)[6:], fl, rng, tname), o)
     # 3-D: a seeded smooth volume at the z-stack benchmark's size, and a smaller one for the per-direction output
     g = torch.Generator(device=dev).manual_seed(11)
